@@ -1,13 +1,18 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: train sequences/sec (fwd + MPJPE + bwd + Adam), BASELINE.json's metric.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload k2|k4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload k2|k4] [--dump-outputs DIR]
 
 N=1 workload = BASELINE.json configs[1]: MotionMixer MlpMixer with squeeze-excitation, H36M xyz
 10 -> 10 frames, batch 4096 per GPU (SURVEY.md §8d "K2": hidden 50, tokens 20, channels 50, 4 blocks,
 mish, dropout 0.1, r_se 8).  N>1: the driver launches this file under torchrun; each rank trains on
 its own shard of the global batch (weak scaling: 4096 sequences per GPU) with one flat-bucket NCCL
 all-reduce per step.  One JSON line is printed by rank 0.
+
+``--dump-outputs DIR`` writes what the timed path computed in its last timed step as ``DIR/<name>.npy`` (see ``step_outputs``).  The
+inputs and the initial weights are seeded, so two builds run with the same arguments can be compared output for output.  Compare
+with a tolerance: the step is not bit-reproducible from run to run, and two runs of the default command on one B200 (1000 W power
+limit) differed by up to 4e-4 of an array's largest magnitude after the 55 training steps, the loss by 6e-7 relative.
 
 ``--impl reference`` times the reference's own CPU implementation of the same step on the host cores: the UNMODIFIED
 reference modules staged under oracle/_ref by oracle/make_ref.py (h36m.mlp_mixer.MlpMixer / h36m.conv_mixer_model.ConvMixer +
@@ -248,6 +253,36 @@ def cpu_baseline(w, budget_s=15.0):
             "sample": "%d steps of the full %d-sequence batch (%s, fp32, %d threads)" % (n, w["B"], what, cores)}
 
 
+DUMP_LIMIT = 64 * 2 ** 20
+
+
+def step_outputs(ts, loss):
+    """Host copies of what the last TrainStep.step call computed: the loss it returned, the prediction of its forward pass, the
+    parameter gradients and the model's state_dict after its Adam update."""
+    import numpy as np
+    out = {"loss": np.asarray(loss, dtype=np.float32), "pred": ts.plan.pred.cpu().numpy()}
+    for name, off, n, shape in ts._named_flat():
+        out["grad." + name] = ts.flat.g[off:off + n].view(shape).cpu().numpy()
+    for name, v in ts.model.state_dict().items():
+        out["state." + name] = v.cpu().numpy()
+    return out
+
+
+def dump_outputs(path, outputs):
+    """DIR/<name>.npy per output, float32 as computed (integer buffers as float64).  If the whole would pass DUMP_LIMIT, the
+    prediction is cut to every k-th sequence, the same rows in every run."""
+    import numpy as np
+    outputs = {k: (v if v.dtype in (np.float32, np.float64) else v.astype(np.float64)) for k, v in outputs.items()}
+    rest = sum(v.nbytes for k, v in outputs.items() if k != "pred")
+    stride = -(-outputs["pred"].nbytes // max(DUMP_LIMIT - rest, 1))
+    outputs["pred"] = outputs["pred"][::stride]
+    os.makedirs(path, exist_ok=True)
+    for k, v in outputs.items():
+        np.save(os.path.join(path, k + ".npy"), v)
+    print("bench: %d outputs of the last timed step written to %s (prediction row stride %d)" % (len(outputs), path, stride),
+          file=sys.stderr)
+
+
 # ---------------------------------------------------------------------------------------------------
 def run_ours(args, w):
     import torch
@@ -333,6 +368,8 @@ def run_ours(args, w):
     t_ms, last_loss = timed(args.steps, devd, False)
     median_ms = timed.median_ms
     barrier()
+    # copied now: the arms below train the same model further
+    outputs = step_outputs(ts, last_loss) if args.dump_outputs and rank == 0 else None
     # ---- data parallel: every rank must hold bit-identical parameters after the timed steps
     dp_identical = None
     if world > 1:
@@ -525,6 +562,8 @@ def run_ours(args, w):
                                   "ms_per_step": t_alt_ms / args.steps}
     if world == 1 and not args.no_cpu_baseline:
         out["cpu_baseline"] = cpu_baseline(w)
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     emit(out)
     shutdown()
 
@@ -541,7 +580,13 @@ def main():
                     help="arithmetic of the MixerBlock contractions: tf32 = the north star's reduced-precision (2e-3) mode, served by the "
                          "tcgen05 kernel family (default, the headline); fp32 = the 1e-5 mode on fp32 SIMT kernels")
     ap.add_argument("--no-alt-precision", action="store_true", help="skip the extra timing of the other precision mode")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed (loss, prediction, gradients, "
+                    "state_dict after the update) as DIR/<name>.npy, at most 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     claim_stdout()
     args.warmup = max(args.warmup, 3)
     w = WORKLOADS[args.workload]

@@ -43,7 +43,7 @@ def rel_err(a, b):
     return float(np.abs(a - b).max()) / denom
 
 
-REPORT = []          # one record per check_close call; tests/conftest.py writes it to profiles/parity_report.json after a GPU run
+REPORT = []          # one record per check_close call; tests/conftest.py writes it to $MMX_PARITY_REPORT after a GPU run
 
 
 def _record(name, rel, rtol, clause, scale):

@@ -1,28 +1,15 @@
 """Checkpoint / wire format (SURVEY §8 f4): ``torch.save(model.state_dict())`` files are interchangeable with the REAL reference
 modules in both directions (strict), incl. the aliased ``se2.*`` keys, BatchNorm buffers and ``encoder.frequencies``; and a
 TrainStep run resumes bit-compatibly from (model.state_dict(), TrainStep.state_dict()).
-The reference modules come from oracle/_ref (unmodified copies staged by oracle/make_ref.py)."""
+The reference side is the state_dict the reference modules themselves wrote into the golden fixtures (tests/golden/make_golden.py:
+the unmodified reference module built after ``torch.manual_seed(0)``, its ``state_dict()`` stored entry by entry, in order)."""
 import io
 
 import numpy as np
 import pytest
 import torch
 
-from oracle import make_ref
-from tests.golden_util import Golden
-
-needs_ref = pytest.mark.skipif(not make_ref.available(), reason="oracle/_ref not staged (python oracle/make_ref.py)")
-
-MLP = dict(num_classes=66, num_blocks=3, hidden_dim=50, tokens_mlp_dim=20, channels_mlp_dim=50, seq_len=10, pred_len=10, activation="mish",
-           regularization=0.1, input_size=66, r_se=8, use_se=True)
-CONVS = {
-    "twice_se_harmonic": dict(num_blocks=2, dimPosIn=66, dimPosEmb=50, dimPosOut=66, in_nTP=10, out_nTP=25, conv_nChan=1, conv1_kernel_shape=(1, 3),
-                              conv1_stride=(1, 1), conv1_padding=(0, 1), mode_conv="twice", activation="mish", regularization=0.1, use_se=True, r_se=8),
-    "once_bn_c4": dict(num_blocks=2, dimPosIn=33, dimPosEmb=64, dimPosOut=33, in_nTP=10, out_nTP=5, conv_nChan=4, conv1_kernel_shape=(5, 9),
-                       mode_conv="once", activation="mish", regularization=-1.0, use_se=True, r_se=8, encoder_n_harmonic_functions=0, encoder_omega0=0),
-    "twice_bn_nose": dict(num_blocks=1, dimPosIn=33, dimPosEmb=32, dimPosOut=33, in_nTP=10, out_nTP=5, conv_nChan=2, conv1_kernel_shape=(3, 3),
-                          mode_conv="twice", activation="gelu", regularization=-1.0, use_se=False, encoder_n_harmonic_functions=4, encoder_omega0=0.1),
-}
+from tests.golden_util import Golden, golden_cases
 
 
 def _roundtrip(sd):
@@ -32,58 +19,61 @@ def _roundtrip(sd):
     return torch.load(buf)
 
 
-def _check_both_ways(ours, ref):
-    sd_o, sd_r = ours.state_dict(), ref.state_dict()
+def _ours(g):
+    from motionmixerconv_b200.conv_mixer_model import ConvMixer
+    from motionmixerconv_b200.mlp_mixer import MlpMixer
+    return (MlpMixer if g.family == "mlp" else ConvMixer)(**g.cfg)
+
+
+def _reference_state_dict(g):
+    """What the reference module's ``state_dict()`` held: keys in its order, shapes, dtypes and values."""
+    return {k: torch.from_numpy(np.array(v)) for k, v in g.params.items()}
+
+
+def _check_both_ways(ours, sd_r):
+    sd_o = ours.state_dict()
     assert list(sd_o.keys()) == list(sd_r.keys())
     assert [tuple(v.shape) for v in sd_o.values()] == [tuple(v.shape) for v in sd_r.values()]
     assert [v.dtype for v in sd_o.values()] == [v.dtype for v in sd_r.values()]
-    # product checkpoint -> reference module (strict), and the values really arrive
-    ref.load_state_dict(_roundtrip(sd_o), strict=True)
-    for k, v in ref.state_dict().items():
-        assert torch.equal(v, sd_o[k]), k
-    # reference checkpoint -> product module (strict)
-    for p in ref.parameters():
-        p.data.add_(1.0)
-    ours.load_state_dict(_roundtrip(ref.state_dict()), strict=True)
+    # product checkpoint -> reference module: its strict load_state_dict needs exactly these keys and shapes, and the values arrive
+    ck = _roundtrip(sd_o)
+    assert list(ck.keys()) == list(sd_r.keys())
+    for k, v in ck.items():
+        assert tuple(v.shape) == tuple(sd_r[k].shape) and v.dtype == sd_r[k].dtype and torch.equal(v, sd_o[k]), k
+    # reference checkpoint -> product module (strict); parameters moved so that the load is visible (aliases move together)
+    params = {n for n, _ in ours.named_parameters(remove_duplicate=False)}
+    sd_r = {k: v + 1.0 if k in params else v for k, v in sd_r.items()}
+    ours.load_state_dict(_roundtrip(sd_r), strict=True)
     for k, v in ours.state_dict().items():
-        assert torch.equal(v, ref.state_dict()[k]), k
+        assert torch.equal(v, sd_r[k]), k
 
 
-@needs_ref
 def test_mlpmixer_checkpoints_interchange_with_the_reference_module():
-    from motionmixerconv_b200.mlp_mixer import MlpMixer
-    Ref, _, _ = make_ref.import_reference()
-    torch.manual_seed(1)
-    ours = MlpMixer(**MLP)
-    torch.manual_seed(2)
-    ref = Ref(**MLP)
-    _check_both_ways(ours, ref)
+    for case in golden_cases("mlp"):
+        g = Golden(case)
+        torch.manual_seed(1)
+        _check_both_ways(_ours(g), _reference_state_dict(g))
 
 
-@needs_ref
-@pytest.mark.parametrize("name", sorted(CONVS))
-def test_convmixer_checkpoints_interchange_with_the_reference_module(name):
-    from motionmixerconv_b200.conv_mixer_model import ConvMixer
-    _, Ref, _ = make_ref.import_reference()
+@pytest.mark.parametrize("case", golden_cases("conv"))
+def test_convmixer_checkpoints_interchange_with_the_reference_module(case):
+    g = Golden(case)
     torch.manual_seed(1)
-    ours = ConvMixer(**CONVS[name])
-    torch.manual_seed(2)
-    ref = Ref(**CONVS[name])
-    _check_both_ways(ours, ref)
-    if CONVS[name]["use_se"] and CONVS[name]["mode_conv"] == "twice":
+    ours = _ours(g)
+    _check_both_ways(ours, _reference_state_dict(g))
+    if g.cfg["use_se"] and g.cfg["mode_conv"] == "twice":
         sd = ours.state_dict()
         assert sd["Mixer_Block.0.se2.excitationBlock.0.weight"].data_ptr() == sd["Mixer_Block.0.se.excitationBlock.0.weight"].data_ptr()
 
 
-@needs_ref
 def test_same_seed_gives_the_reference_modules_initial_weights():
-    from motionmixerconv_b200.mlp_mixer import MlpMixer
-    Ref, _, _ = make_ref.import_reference()
-    torch.manual_seed(7)
-    a = MlpMixer(**MLP).state_dict()
-    torch.manual_seed(7)
-    b = Ref(**MLP).state_dict()
-    assert all(torch.equal(a[k], b[k]) for k in b)
+    for case in golden_cases():
+        g = Golden(case)
+        torch.manual_seed(0)            # the seed the fixture's reference module was built with
+        a = _ours(g).state_dict()
+        b = _reference_state_dict(g)
+        assert list(a.keys()) == list(b.keys()), case
+        assert all(torch.equal(a[k], b[k]) for k in b), case
 
 
 @pytest.mark.gpu

@@ -1,5 +1,5 @@
-"""CPU: the checkpoint validator (motionmixerconv_b200/checkpoint.py) on state_dicts written by the REFERENCE modules (oracle/_ref)
-and on the golden fixtures' parameters; detects missing / reordered keys, wrong shapes, broken se2 aliases."""
+"""CPU: the checkpoint validator (motionmixerconv_b200/checkpoint.py) on state_dicts written by the REFERENCE modules (the golden
+fixtures' parameters, tests/golden/make_golden.py); detects missing / reordered keys, wrong shapes, broken se2 aliases."""
 import json
 
 import numpy as np
@@ -7,7 +7,6 @@ import pytest
 import torch
 
 from motionmixerconv_b200 import checkpoint as CK
-from oracle import make_ref
 from tests.golden_util import Golden, golden_cases
 
 
@@ -18,24 +17,21 @@ def test_fixture_parameters_validate(case):
     assert CK.validate_state_dict(sd, g.family, g.cfg) == []
 
 
-@pytest.mark.skipif(not make_ref.available(), reason="oracle/_ref not staged")
 def test_reference_checkpoint_file_through_the_cli(tmp_path, capsys):
-    _, RefConv, _ = make_ref.import_reference()
-    cfg = dict(num_blocks=2, dimPosIn=33, dimPosEmb=48, dimPosOut=33, in_nTP=10, out_nTP=10, conv_nChan=4, conv1_kernel_shape=[5, 5],
-               mode_conv="twice", activation="mish", regularization=-1.0, use_se=True, r_se=8, encoder_n_harmonic_functions=8, encoder_omega0=0.1)
-    torch.manual_seed(0)
-    ref = RefConv(**{k: (tuple(v) if isinstance(v, list) else v) for k, v in cfg.items()})
-    path = tmp_path / "model.pt"
-    torch.save(ref.state_dict(), path)
-    assert CK.main([str(path), "--family", "conv", "--cfg", json.dumps(cfg)]) == 0
-    assert "OK" in capsys.readouterr().out
-    sd = ref.state_dict()
-    bad = dict(sd)
-    bad["Mixer_Block.0.se2.excitationBlock.0.weight"] = sd["Mixer_Block.0.se2.excitationBlock.0.weight"] + 1.0      # alias broken
-    bad["LN.weight"] = torch.zeros(7)                                                                                # wrong shape
-    del bad["fc_out.bias"]                                                                                           # missing
-    problems = CK.validate_state_dict(bad, "conv", cfg)
-    text = "\n".join(problems)
-    assert "missing keys" in text and "LN.weight: shape" in text and "se2" in text
-    reordered = dict(reversed(list(sd.items())))
-    assert any("key order" in p for p in CK.validate_state_dict(reordered, "conv", cfg))
+    for case in ("conv_k1", "conv_k3_bn"):      # harmonic encoder + se2 aliases; BatchNorm buffers + se2 aliases
+        g = Golden(case)
+        cfg = json.loads(json.dumps(g.cfg))
+        sd = {k: torch.from_numpy(np.array(v)) for k, v in g.params.items()}
+        path = tmp_path / (case + ".pt")
+        torch.save(sd, path)
+        assert CK.main([str(path), "--family", "conv", "--cfg", json.dumps(cfg)]) == 0
+        assert "OK" in capsys.readouterr().out
+        bad = dict(sd)
+        bad["Mixer_Block.0.se2.excitationBlock.0.weight"] = sd["Mixer_Block.0.se2.excitationBlock.0.weight"] + 1.0      # alias broken
+        bad["LN.weight"] = torch.zeros(7)                                                                                # wrong shape
+        del bad["fc_out.bias"]                                                                                           # missing
+        problems = CK.validate_state_dict(bad, "conv", cfg)
+        text = "\n".join(problems)
+        assert "missing keys" in text and "LN.weight: shape" in text and "se2" in text
+        reordered = dict(reversed(list(sd.items())))
+        assert any("key order" in p for p in CK.validate_state_dict(reordered, "conv", cfg))

@@ -1,6 +1,6 @@
 import ctypes as C, os, sys, json
 import torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from motionmixerconv_b200 import _lib as L
 from motionmixerconv_b200 import functional as F_
 lib = L.load()
