@@ -120,17 +120,27 @@ VARIANTS = {
     "no_se": dict(use_se=False),
     "se_hidden_2": dict(r_se=4),
     "h48_ch24": dict(hidden_dim=48, channels_mlp_dim=24),
-    "h64_ch64_gelu": dict(hidden_dim=64, channels_mlp_dim=64, activation="gelu"),      # KP = 80, per-row bulk copies
+    "h64_ch64_gelu": dict(hidden_dim=64, channels_mlp_dim=64, activation="gelu"),      # streamed weights at operand width 64
     "h78_ch30": dict(hidden_dim=78, channels_mlp_dim=30),
+    "h72_ch72": dict(hidden_dim=72, channels_mlp_dim=72),                              # resident KP = 80, 4-float row loads
+    "h50_ch49": dict(hidden_dim=50, channels_mlp_dim=49),                              # odd ch: resident KP = 64 only
+    "h64_ch63": dict(hidden_dim=64, channels_mlp_dim=63),                              # odd ch: resident KP = 80 only
     "tok7_T8": dict(tokens_mlp_dim=7, seq_len=8, pred_len=8),                          # generic-T instantiation (T != 10)
     "T16_to25": dict(seq_len=16, pred_len=25, tokens_mlp_dim=32, r_se=8),              # two sequences per warp, SE hidden 2
+    "T13_h52": dict(seq_len=13, hidden_dim=52, channels_mlp_dim=52, r_se=4),           # two sequences per warp, 6 idle lanes
+    "T6_h40": dict(seq_len=6, hidden_dim=40, channels_mlp_dim=40, r_se=2),             # five sequences per warp, SE hidden 3
 }
 
 
 @pytest.mark.parametrize("name", sorted(VARIANTS))
 def test_shape_variants_vs_oracle(name):
+    from motionmixerconv_b200 import _lib as L
+    from motionmixerconv_b200 import functional as F_
     cfg = dict(Golden("mlp_k2").cfg, num_blocks=2, regularization=0, **VARIANTS[name])
     model = _model(cfg, None, seed=3).train()
+    mb = model.Mixer_Block[0]
+    desc = F_.mlp_block_desc(515, mb.seq_len, mb.hidden_dim, *mb.meta())
+    assert L.load().mmx_mlp_block_saves(C.byref(desc)) == 1         # the tcgen05 family serves it (no FP32 fall-back)
     params = {k: v.detach().cpu().numpy() for k, v in model.state_dict().items()}
     x, gt = synthetic_pose_windows(515, cfg["seq_len"], cfg["pred_len"], 66, scale="amass", seed=9)
     _compare(*_run(model, x, gt), _oracle(cfg, params, x, gt))
