@@ -179,7 +179,8 @@ int mmx_mlp_head_fwd(const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, const f
 int mmx_mlp_head_bwd(const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, const MmxMlpHeadParams* grads,
                      const float* x, const float* dout, float* dx, void* stream);
 /* The same with a precision mode: MMX_PREC_TF32 runs the whole head as one tcgen05 kernel per direction (H < 64, D <= 80,
- * T, To <= 128), see csrc/mmx_head_tc5.cuh; other shapes fall back to the fp32 kernels. */
+ * H and D even and >= 8, T, To <= 128, T*H and To*D multiples of 4, 16-byte aligned tensors), see csrc/mmx_head_tc5.cuh;
+ * other shapes fall back to the fp32 kernels, which serve T <= 32 (MMX_E_UNSUPPORTED above). */
 int mmx_mlp_head_fwd_prec(const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, const float* x, float* out, int precision, void* stream);
 int mmx_mlp_head_bwd_prec(const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, const MmxMlpHeadParams* grads,
                           const float* x, const float* dout, float* dx, int precision, void* stream);

@@ -56,9 +56,14 @@ int plan_linear(int rows, int K, int N, bool bwd, LinearDims* out, size_t* smem,
     return fail(MMX_E_UNSUPPORTED, "linear layer K=%d N=%d does not fit shared memory", K, N);
 }
 
-int plan_head(const MmxMlpHeadDesc* d, bool bwd, MlpHeadDims* out, size_t* smem, int* grid) {
+int check_head_desc(const MmxMlpHeadDesc* d) {
     if (!d) return fail(MMX_E_INVALID, "null descriptor");
     if (d->B <= 0 || d->T <= 0 || d->To <= 0 || d->H <= 0 || d->D <= 0) return fail(MMX_E_INVALID, "non-positive dimension");
+    return MMX_OK;
+}
+
+int plan_head(const MmxMlpHeadDesc* d, bool bwd, MlpHeadDims* out, size_t* smem, int* grid) {
+    if (int rc = check_head_desc(d)) return rc;
     if (d->T > 32) return fail(MMX_E_UNSUPPORTED, "seq_len %d > 32", d->T);
     if (((d->To + 3) / 4) * ((d->T + 3) / 4) > kThreads) return fail(MMX_E_UNSUPPORTED, "pred_len %d too large", d->To);
     const DevInfo di = dev_info();
@@ -156,11 +161,13 @@ int mmx_mlp_head_bwd(const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, const M
 
 int mmx_mlp_head_fwd_prec(const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, const float* x, float* out, int precision, void* stream) {
     if (!x || !out) return fail(MMX_E_INVALID, "mmx_mlp_head_fwd: null tensor");
-    MlpHeadFwdArgs a; size_t smem; int grid;
-    int rc = plan_head(d, false, &a.d, &smem, &grid);
+    int rc = check_head_desc(d);
     if (rc) return rc;
     if ((rc = check_head_params(w, "mmx_mlp_head_fwd"))) return rc;
+    // the tcgen05 head serves T, To <= 128; the fp32 planner below stops at T = 32, so it is asked only when tcgen05 declines
     if (precision == MMX_PREC_TF32 && mmx_head_tc5_ok(d) && !((((uintptr_t)x) | ((uintptr_t)out)) & 15)) return mmx_head_tc5_fwd(d, w, x, out, stream);
+    MlpHeadFwdArgs a; size_t smem; int grid;
+    if ((rc = plan_head(d, false, &a.d, &smem, &grid))) return rc;
     a.w = to_hw(w); a.x = x; a.out = out;
     if (d->T == 10) return launch<HeadFwdBody<10>>(a, grid, kThreads, smem, stream, 1);
     return launch<HeadFwdBody<0>>(a, grid, kThreads, smem, stream, 1);
@@ -169,13 +176,14 @@ int mmx_mlp_head_fwd_prec(const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, co
 int mmx_mlp_head_bwd_prec(const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, const MmxMlpHeadParams* grads,
                           const float* x, const float* dout, float* dx, int precision, void* stream) {
     if (!x || !dout || !dx) return fail(MMX_E_INVALID, "mmx_mlp_head_bwd: null tensor");
-    MlpHeadBwdArgs a; size_t smem; int grid;
-    int rc = plan_head(d, true, &a.d, &smem, &grid);
+    int rc = check_head_desc(d);
     if (rc) return rc;
     if ((rc = check_head_params(w, "mmx_mlp_head_bwd"))) return rc;
     if ((rc = check_head_params(grads, "mmx_mlp_head_bwd(grads)"))) return rc;
     if (precision == MMX_PREC_TF32 && mmx_head_tc5_ok(d) && !((((uintptr_t)x) | ((uintptr_t)dout) | ((uintptr_t)dx)) & 15))
         return mmx_head_tc5_bwd(d, w, grads, x, dout, dx, stream);
+    MlpHeadBwdArgs a; size_t smem; int grid;
+    if ((rc = plan_head(d, true, &a.d, &smem, &grid))) return rc;
     a.w = to_hw(w); a.g = to_hw(grads); a.x = x; a.dout = dout; a.dx = dx;
     const int tiles = ((d->D + 3) / 4) * ((d->H + 3) / 4);
     if (d->T == 10) {
