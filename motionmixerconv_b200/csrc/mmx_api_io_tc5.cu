@@ -5,11 +5,11 @@
 
 #if defined(MMX_HOST_EMU)
 bool mmx_lin_tc5_ok(long long, int, int, const void*, const void*, const void*) { return false; }
-int mmx_lin_tc5_fwd(long long, int, int, const float*, const float*, const float*, float*, void*) { return fail(MMX_E_UNSUPPORTED, "no tensor cores in the emulator"); }
-int mmx_lin_tc5_bwd(long long, int, int, const float*, const float*, const float*, float*, float*, float*, void*) { return fail(MMX_E_UNSUPPORTED, "no tensor cores in the emulator"); }
+int mmx_lin_tc5(bool, long long, int, int, const float*, const float*, const float*, const float*, float*, float*, float*, void*) {
+    return fail(MMX_E_UNSUPPORTED, "no tensor cores in the emulator");
+}
 bool mmx_head_tc5_ok(const MmxMlpHeadDesc*) { return false; }
-int mmx_head_tc5_fwd(const MmxMlpHeadDesc*, const MmxMlpHeadParams*, const float*, float*, void*) { return fail(MMX_E_UNSUPPORTED, "no tensor cores in the emulator"); }
-int mmx_head_tc5_bwd(const MmxMlpHeadDesc*, const MmxMlpHeadParams*, const MmxMlpHeadParams*, const float*, const float*, float*, void*) {
+int mmx_head_tc5(bool, const MmxMlpHeadDesc*, const MmxMlpHeadParams*, const MmxMlpHeadParams*, const float*, const float*, float*, void*) {
     return fail(MMX_E_UNSUPPORTED, "no tensor cores in the emulator");
 }
 #else
@@ -29,39 +29,24 @@ bool mmx_lin_tc5_ok(long long rows, int K, int N, const void* x, const void* y, 
     return true;
 }
 
-static void fill_lin(lin::LinArgs& a, long long rows, int K, int N) {
+// forward: out = y = x W^T + b (dy, dw, db unused); backward: dw += dY^T x, db += column sums of dY, out = dx (nullable)
+int mmx_lin_tc5(bool bwd, long long rows, int K, int N, const float* x, const float* w, const float* b, const float* dy, float* dw,
+                float* db, float* out, void* stream) {
+    lin::LinArgs a;
+    a.x = x; a.w = w; a.b = b; a.dy = dy; a.out = out; a.g_w = dw; a.g_b = db;
     a.R = rows; a.K = K; a.N = N;
     a.abort_count = mmx_tc5_abort_ptr();
-    a.dy = nullptr; a.g_w = a.g_b = nullptr;
-}
-
-int mmx_lin_tc5_fwd(long long rows, int K, int N, const float* x, const float* w, const float* b, float* y, void* stream) {
-    lin::LinArgs a;
-    fill_lin(a, rows, K, N);
-    a.x = x; a.w = w; a.b = b; a.out = y;
     const DevInfo di = dev_info();
     const long long ntiles = (rows + 127) / 128;
     const bool small = (K + 1 > N ? K + 1 : N) <= 64;
-    const size_t smem = small ? lin::lin_smem_bytes<64>(K, N, false) : lin::lin_smem_bytes<80>(K, N, false);
+    const size_t smem = small ? lin::lin_smem<64>(K, N, bwd).total : lin::lin_smem<80>(K, N, bwd).total;
     const int per_sm = imax(1, imin(2, (int)((di.max_smem + 1024) / (smem + 1024))));
     const int grid = (int)(ntiles < (long long)di.sms * per_sm ? ntiles : (long long)di.sms * per_sm);
-    return small ? launch_tc5(lin::lin_fwd_kernel<64, 2>, a, grid, chan::kThreadsChan, smem, stream)
-                 : launch_tc5(lin::lin_fwd_kernel<80, 2>, a, grid, chan::kThreadsChan, smem, stream);
-}
-
-int mmx_lin_tc5_bwd(long long rows, int K, int N, const float* x, const float* w, const float* dy, float* dw, float* db, float* dx,
-                    void* stream) {
-    lin::LinArgs a;
-    fill_lin(a, rows, K, N);
-    a.x = x; a.w = w; a.b = nullptr; a.dy = dy; a.out = dx; a.g_w = dw; a.g_b = db;
-    const DevInfo di = dev_info();
-    const long long ntiles = (rows + 127) / 128;
-    const bool small = (K + 1 > N ? K + 1 : N) <= 64;
-    const size_t smem = small ? lin::lin_smem_bytes<64>(K, N, true) : lin::lin_smem_bytes<80>(K, N, true);
-    const int per_sm = imax(1, imin(2, (int)((di.max_smem + 1024) / (smem + 1024))));
-    const int grid = (int)(ntiles < (long long)di.sms * per_sm ? ntiles : (long long)di.sms * per_sm);
-    return small ? launch_tc5(lin::lin_bwd_kernel<64, 2>, a, grid, chan::kThreadsChan, smem, stream)
-                 : launch_tc5(lin::lin_bwd_kernel<80, 2>, a, grid, chan::kThreadsChan, smem, stream);
+    if (bwd)
+        return small ? launch_tc5(lin::lin_bwd_kernel<64, 2>, a, grid, tc5::kCtaThreads, smem, stream)
+                     : launch_tc5(lin::lin_bwd_kernel<80, 2>, a, grid, tc5::kCtaThreads, smem, stream);
+    return small ? launch_tc5(lin::lin_fwd_kernel<64, 2>, a, grid, tc5::kCtaThreads, smem, stream)
+                 : launch_tc5(lin::lin_fwd_kernel<80, 2>, a, grid, tc5::kCtaThreads, smem, stream);
 }
 
 // ------------------------------------------------------------------------------------------ output head
@@ -73,34 +58,21 @@ bool mmx_head_tc5_ok(const MmxMlpHeadDesc* d) {
     return true;
 }
 
-static void fill_head(head::HeadArgs& a, const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, const MmxMlpHeadParams* g) {
+// forward: out = head(x) (grads, dout unused); backward: grads += parameter gradients, out = dx
+int mmx_head_tc5(bool bwd, const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, const MmxMlpHeadParams* grads, const float* x,
+                 const float* dout, float* out, void* stream) {
+    head::HeadArgs a;
     a.ln_g = w->ln_w; a.ln_b = w->ln_b; a.wt = w->wt; a.bt = w->bt; a.wf = w->wf; a.bf = w->bf;
-    if (g) { a.g_ln_g = g->ln_w; a.g_ln_b = g->ln_b; a.g_wt = g->wt; a.g_bt = g->bt; a.g_wf = g->wf; a.g_bf = g->bf; }
+    if (bwd) { a.g_ln_g = grads->ln_w; a.g_ln_b = grads->ln_b; a.g_wt = grads->wt; a.g_bt = grads->bt; a.g_wf = grads->wf; a.g_bf = grads->bf; }
     else a.g_ln_g = a.g_ln_b = a.g_wt = a.g_bt = a.g_wf = a.g_bf = nullptr;
     a.B = d->B; a.T = d->T; a.To = d->To; a.H = d->H; a.D = d->D;
     a.S = 128 / imax(d->T, d->To);
-    a.dout = nullptr;
+    a.x = x; a.dout = bwd ? dout : nullptr; a.out = out;
     a.abort_count = mmx_tc5_abort_ptr();
-}
-
-int mmx_head_tc5_fwd(const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, const float* x, float* out, void* stream) {
-    head::HeadArgs a;
-    fill_head(a, d, w, nullptr);
-    a.x = x; a.out = out;
-    const DevInfo di = dev_info();
     const int ntiles = (d->B + a.S - 1) / a.S;
-    const size_t smem = head::head_smem(d->H, d->D, false).total;
-    return launch_tc5(head::head_fwd_kernel, a, imin(ntiles, di.sms), chan::kThreadsChan, smem, stream);
-}
-
-int mmx_head_tc5_bwd(const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, const MmxMlpHeadParams* grads, const float* x, const float* dout,
-                     float* dx, void* stream) {
-    head::HeadArgs a;
-    fill_head(a, d, w, grads);
-    a.x = x; a.dout = dout; a.out = dx;
-    const DevInfo di = dev_info();
-    const int ntiles = (d->B + a.S - 1) / a.S;
-    const size_t smem = head::head_smem(d->H, d->D, true).total;
-    return launch_tc5(head::head_bwd_kernel, a, imin(ntiles, di.sms), chan::kThreadsChan, smem, stream);
+    const int grid = imin(ntiles, dev_info().sms);
+    const size_t smem = head::head_smem(d->H, d->D, bwd).total;
+    return bwd ? launch_tc5(head::head_bwd_kernel, a, grid, tc5::kCtaThreads, smem, stream)
+               : launch_tc5(head::head_fwd_kernel, a, grid, tc5::kCtaThreads, smem, stream);
 }
 #endif

@@ -100,12 +100,11 @@ using namespace mmx_tu_misc;
 
 // tcgen05 kernels of the embedding / output head (mmx_api_io_tc5.cu)
 bool mmx_lin_tc5_ok(long long rows, int K, int N, const void* x, const void* y, const void* dx);
-int mmx_lin_tc5_fwd(long long rows, int K, int N, const float* x, const float* w, const float* b, float* y, void* stream);
-int mmx_lin_tc5_bwd(long long rows, int K, int N, const float* x, const float* w, const float* dy, float* dw, float* db, float* dx, void* stream);
+int mmx_lin_tc5(bool bwd, long long rows, int K, int N, const float* x, const float* w, const float* b, const float* dy, float* dw,
+                float* db, float* out, void* stream);
 bool mmx_head_tc5_ok(const MmxMlpHeadDesc* d);
-int mmx_head_tc5_fwd(const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, const float* x, float* out, void* stream);
-int mmx_head_tc5_bwd(const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, const MmxMlpHeadParams* grads, const float* x, const float* dout,
-                     float* dx, void* stream);
+int mmx_head_tc5(bool bwd, const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, const MmxMlpHeadParams* grads, const float* x,
+                 const float* dout, float* out, void* stream);
 
 // ====================================================================================== C ABI
 extern "C" {
@@ -122,7 +121,7 @@ int mmx_linear_bwd(int rows, int K, int N, const float* x, const float* w, const
 
 int mmx_linear_fwd_prec(int rows, int K, int N, const float* x, const float* w, const float* b, float* y, int precision, void* stream) {
     if (!x || !w || !b || !y) return fail(MMX_E_INVALID, "mmx_linear_fwd: null tensor");
-    if (precision == MMX_PREC_TF32 && mmx_lin_tc5_ok(rows, K, N, x, y, nullptr)) return mmx_lin_tc5_fwd(rows, K, N, x, w, b, y, stream);
+    if (precision == MMX_PREC_TF32 && mmx_lin_tc5_ok(rows, K, N, x, y, nullptr)) return mmx_lin_tc5(false, rows, K, N, x, w, b, nullptr, nullptr, nullptr, y, stream);
     LinearFwdArgs a; size_t smem; int grid;
     int rc = plan_linear(rows, K, N, false, &a.d, &smem, &grid);
     if (rc) return rc;
@@ -133,7 +132,7 @@ int mmx_linear_fwd_prec(int rows, int K, int N, const float* x, const float* w, 
 int mmx_linear_bwd_prec(int rows, int K, int N, const float* x, const float* w, const float* dy, float* dw, float* db,
                         float* dx, int precision, void* stream) {
     if (!x || !w || !dy || !dw || !db) return fail(MMX_E_INVALID, "mmx_linear_bwd: null tensor");
-    if (precision == MMX_PREC_TF32 && mmx_lin_tc5_ok(rows, K, N, x, dy, dx)) return mmx_lin_tc5_bwd(rows, K, N, x, w, dy, dw, db, dx, stream);
+    if (precision == MMX_PREC_TF32 && mmx_lin_tc5_ok(rows, K, N, x, dy, dx)) return mmx_lin_tc5(true, rows, K, N, x, w, nullptr, dy, dw, db, dx, stream);
     LinearBwdArgs a; size_t smem; int grid;
     int rc = plan_linear(rows, K, N, true, &a.d, &smem, &grid);
     if (rc) return rc;
@@ -165,7 +164,7 @@ int mmx_mlp_head_fwd_prec(const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, co
     if (rc) return rc;
     if ((rc = check_head_params(w, "mmx_mlp_head_fwd"))) return rc;
     // the tcgen05 head serves T, To <= 128; the fp32 planner below stops at T = 32, so it is asked only when tcgen05 declines
-    if (precision == MMX_PREC_TF32 && mmx_head_tc5_ok(d) && !((((uintptr_t)x) | ((uintptr_t)out)) & 15)) return mmx_head_tc5_fwd(d, w, x, out, stream);
+    if (precision == MMX_PREC_TF32 && mmx_head_tc5_ok(d) && !((((uintptr_t)x) | ((uintptr_t)out)) & 15)) return mmx_head_tc5(false, d, w, nullptr, x, nullptr, out, stream);
     MlpHeadFwdArgs a; size_t smem; int grid;
     if ((rc = plan_head(d, false, &a.d, &smem, &grid))) return rc;
     a.w = to_hw(w); a.x = x; a.out = out;
@@ -181,7 +180,7 @@ int mmx_mlp_head_bwd_prec(const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, co
     if ((rc = check_head_params(w, "mmx_mlp_head_bwd"))) return rc;
     if ((rc = check_head_params(grads, "mmx_mlp_head_bwd(grads)"))) return rc;
     if (precision == MMX_PREC_TF32 && mmx_head_tc5_ok(d) && !((((uintptr_t)x) | ((uintptr_t)dout) | ((uintptr_t)dx)) & 15))
-        return mmx_head_tc5_bwd(d, w, grads, x, dout, dx, stream);
+        return mmx_head_tc5(true, d, w, grads, x, dout, dx, stream);
     MlpHeadBwdArgs a; size_t smem; int grid;
     if ((rc = plan_head(d, true, &a.d, &smem, &grid))) return rc;
     a.w = to_hw(w); a.g = to_hw(grads); a.x = x; a.dout = dout; a.dx = dx;

@@ -50,10 +50,10 @@ extern "C" int mmx_tc5_abort_count(void) {
 
 // keep-scales of one dropout site of this kernel family, as the kernels draw them (debug / test entry point)
 static __global__ void tc5_mask_kernel(Dropout dr, uint32_t site, long long rows, int W, float* out) {
-    const uint32_t key = chan::drop_key(dr.seed_lo, dr.seed_hi, site, dr.step), W8 = (uint32_t)(W + 7) >> 3;
+    const uint32_t key = tc5::drop_key(dr.seed_lo, dr.seed_hi, site, dr.step), W8 = (uint32_t)(W + 7) >> 3;
     for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < rows * W; i += (long long)gridDim.x * blockDim.x) {
         const uint32_t row = (uint32_t)(i / W), w = (uint32_t)(i - (long long)row * W);
-        const uint32_t kb = dr.thresh >> 16 ? chan::keep8(key, dr.thresh >> 16, row, W8, w >> 3) : 0xffu;
+        const uint32_t kb = dr.thresh >> 16 ? tc5::keep8(key, dr.thresh >> 16, row, W8, w >> 3) : 0xffu;
         out[i] = (kb >> (w & 7)) & 1u ? dr.scale : 0.0f;
     }
 }
@@ -74,12 +74,12 @@ static int kp_of(const MmxMlpBlockDesc* d) {
     const int need = (d->H > d->ch ? d->H : d->ch) + 1;      // + the ones column that carries the bias gradients
     if (need <= 64) return 64;
     if (need <= 80) return 80;
-    if (need - 1 <= 128 && !(d->ch & 1) && !env_int("MMX_MLP_NO_WIDE", 0)) return 128;
+    if (need - 1 <= 128 && !(d->ch & 1)) return 128;
     return 0;
 }
 
 bool mmx_mlp_tc5_ok(const MmxMlpBlockDesc* d) {
-    if (d->precision != MMX_PREC_TF32 || env_int("MMX_MLP_NO_TC5", 0)) return false;
+    if (d->precision != MMX_PREC_TF32) return false;
     if (d->T < 2 || d->T > tok::kMaxT || d->tok < 1 || d->tok > tok::kMaxTok) return false;
     if (d->H < 8 || d->ch < 8 || (d->H & 1) || kp_of(d) == 0) return false;
     if ((d->T * d->H) & 3) return false;                      // bulk copies: every tile is a multiple of 16 bytes
@@ -120,7 +120,7 @@ static int run_tok(bool bwd, const tok::TokArgs& t, void* stream) {
     if (smem > (size_t)di.max_smem) return fail(MMX_E_UNSUPPORTED, "token half: tile does not fit shared memory (H=%d)", t.H);
     const int threads = tok::kTokThreads;
     int per_sm = (int)((di.max_smem + 1024) / (smem + 1024));
-    per_sm = imax(1, imin(per_sm, env_int("MMX_TOK_CTAS", bwd ? 2 : 4)));
+    per_sm = imax(1, imin(per_sm, bwd ? 2 : 4));
     const int ntiles = (t.B + t.S - 1) / t.S;
     const int grid = balanced_grid(ntiles, di.sms * per_sm);
     return bwd ? launch_tc5(tok::tok_bwd_kernel<ACT, TT>, t, grid, threads, smem, stream)
@@ -152,17 +152,17 @@ static void fill_chan(chan::ChanArgs& c, const MmxMlpBlockDesc* d, const MmxMlpB
 template <int ACT, int KP, int VEC>
 static int run_chan(bool bwd, const chan::ChanArgs& c, void* stream) {
     const DevInfo di = dev_info();
-    const size_t smem = chan::chan_smem_bytes<KP>(c.T, c.H, VEC, bwd);
-    if (smem > (size_t)di.max_smem) return fail(MMX_E_UNSUPPORTED, "channel half: tile does not fit shared memory (H=%d ch=%d)", c.H, c.ch);
     const chan::Geo g = chan::make_geo(c.T, c.H, VEC);
+    const size_t smem = chan::chan_smem<KP>(g, bwd).total;
+    if (smem > (size_t)di.max_smem) return fail(MMX_E_UNSUPPORTED, "channel half: tile does not fit shared memory (H=%d ch=%d)", c.H, c.ch);
     const int ntiles = (c.B + g.seq_per_tile - 1) / g.seq_per_tile;
     // TMEM: forward 2*KP columns (<= 2 CTAs / SM at KP = 64), backward 4*KP columns
     int per_sm = (int)((di.max_smem + 1024) / (smem + 1024));
     const int tm_cols = bwd ? 512 : (3 * KP <= 256 ? 256 : 512);
     per_sm = imax(1, imin(per_sm, 512 / tm_cols));
     const int grid = imin(ntiles, di.sms * per_sm);
-    return bwd ? launch_tc5(chan::chan_bwd_kernel<ACT, KP, VEC>, c, grid, chan::kThreadsChan, smem, stream)
-               : launch_tc5(chan::chan_fwd_kernel<ACT, KP, VEC>, c, grid, chan::kThreadsChan, smem, stream);
+    return bwd ? launch_tc5(chan::chan_bwd_kernel<ACT, KP, VEC>, c, grid, tc5::kCtaThreads, smem, stream)
+               : launch_tc5(chan::chan_fwd_kernel<ACT, KP, VEC>, c, grid, tc5::kCtaThreads, smem, stream);
 }
 
 template <int ACT>

@@ -46,21 +46,20 @@ static int wide_workspace(const float* key, uint8_t** out) {
 template <int ACT, int VEC, int KP>
 static int run_wide(bool bwd, const chan::ChanArgs& c, void* stream) {
     const DevInfo di = dev_info();
-    const size_t smem = chanw::wide_smem_bytes<KP>(c.T, c.H, VEC, bwd);
+    const chan::Geo g = chan::make_geo(c.T, c.H, VEC);
+    const size_t smem = chanw::wide_smem<KP>(g, bwd).total;
     if (smem > (size_t)di.max_smem) return fail(MMX_E_UNSUPPORTED, "wide channel half: tile does not fit shared memory (H=%d ch=%d)", c.H, c.ch);
     uint8_t* ws = nullptr;
     int rc = wide_workspace(c.w1, &ws);
     if (rc) return rc;
     if ((rc = launch_tc5v(chanw::chan_prep_kernel<KP>, KP <= 64 ? 8 : 32, 256, 0, stream, c, ws))) return rc;
-    const chan::Geo g = chan::make_geo(c.T, c.H, VEC);
     const int ntiles = (c.B + g.seq_per_tile - 1) / g.seq_per_tile;
     // KP = 128: 512 TMEM columns, ~205 KB shared -> one CTA per SM; KP = 64: 256 columns, < 100 KB -> two CTAs per SM
-    int per_sm = KP <= 64 ? imin(2, (int)((di.max_smem + 1024) / (smem + 1024))) : 1;
-    per_sm = imax(1, imin(per_sm, env_int("MMX_CHAN_CTAS", 2)));
+    const int per_sm = KP <= 64 ? imax(1, imin(2, (int)((di.max_smem + 1024) / (smem + 1024)))) : 1;
     const int grid = balanced_grid(ntiles, di.sms * per_sm);
     const uint8_t* wsc = ws;
-    return bwd ? launch_tc5v(chanw::chan_wide_bwd_kernel<ACT, VEC, KP>, grid, chan::kThreadsChan, smem, stream, c, wsc)
-               : launch_tc5v(chanw::chan_wide_fwd_kernel<ACT, VEC, KP>, grid, chan::kThreadsChan, smem, stream, c, wsc);
+    return bwd ? launch_tc5v(chanw::chan_wide_bwd_kernel<ACT, VEC, KP>, grid, tc5::kCtaThreads, smem, stream, c, wsc)
+               : launch_tc5v(chanw::chan_wide_fwd_kernel<ACT, VEC, KP>, grid, tc5::kCtaThreads, smem, stream, c, wsc);
 }
 
 template <int KP>

@@ -3,22 +3,13 @@
 //     y = x1 + SE(reg2(fc2(reg1(act(fc1(LN2(x1)))))))          reference: h36m/mlp_mixer.py:157-164 (MixerBlock.forward, second
 //     half), MlpBlock :87-96, SELayer :30-34; restated in oracle/mixer_np.py (MlpMixerOracle.forward / backward).
 //
-// Work unit: a tile of 4 * (32 / T) whole sequences = one 128-row MMA tile.  Row r of the tile is TMEM lane r; the two warps
+// Work unit: a tile of 4 * (32 / T) whole sequences = one 128-row MMA tile.  Row r of the tile is TMEM lane r; the kHalves warps
 // that may touch a lane quarter (warp % 4) split the row's 8-column chunks between them, so LayerNorm, the activation,
-// dropout, the squeeze sum and the LayerNorm backward are per-thread loops over half a row plus one shared-memory exchange
+// dropout, the squeeze sum and the LayerNorm backward are per-thread loops over part of a row plus one shared-memory exchange
 // of the partial sums.  The T frames of a sequence sit in T consecutive lanes of one warp: the SE excitation is a handful of
 // shuffles.  Lanes 32/T*T .. 31 of every warp are padding rows (all-zero operands).
 //
-// Contractions: tcgen05.mma kind::f16 on bf16 operands with fp32 accumulation in TMEM.  Every fp32 operand x is split as
-// x = hi + lo (+ <= 2^-18 |x|), hi = bf16(x), lo = bf16(x - hi), and a product is issued as three MMAs hi*hi + lo*hi + hi*lo
-// ("bf16x3"): measured 5e-6 .. 2e-5 on predictions / gradients of the whole model against the fp64 oracle.
-// Operands live in shared memory in the 16-bit PANEL layout
-//     element (row r, col c)  ->  plane + (c / 8) * (R * 16) + r * 16 + (c % 8) * 2        (hi plane, lo plane)
-// which the tensor core reads in both orientations (SWIZZLE_NONE canonical layouts, checked by tools/micro/umma_layout_probe_bf16):
-//   K-major  (rows = M/N index, cols = K): SBO = 128, LBO = R*16     -> forward GEMMs   D = A W^T
-//   MN-major (rows = K index, cols = M/N): SBO = R*16, LBO = 128     -> weight gradients dW = dY^T A  (K = the tile's rows)
-//                                                                       and data gradients dA = dY W with the UNtransposed weight
-// so one copy of each activation / weight serves the forward, the data-gradient and the weight-gradient product.
+// Contractions and operands: the bf16x3 products on the 16-bit panel layout of mmx_tc5.cuh (read its header first).
 // LN2's affine is folded into fc1 (W1' = W1 * gamma2, b1' = b1 + W1 beta2): the A operand is the plain normalised row and
 // dgamma2, dbeta2, dW1 are derived at flush time from ONE accumulated product  Wt = dU^T xhat.  Bias gradients ride along as a
 // column of ones in the B operand of the weight-gradient products.  dW1 / dW2 accumulate in TMEM across the CTA's whole
@@ -27,7 +18,6 @@
 // (small code: the first version, fully unrolled over register-resident rows, was 300 KB of SASS and instruction-fetch bound).
 // Activations enter and leave through the bulk-copy engine (cp.async.bulk, SASS UBLKCP) with mbarrier completion.
 #pragma once
-#include "mmx_common.cuh"
 #include "mmx_tc5.cuh"
 
 namespace mmx {
@@ -35,11 +25,6 @@ namespace chan {
 
 using namespace tc5;
 
-#ifndef MMX_CHAN_HALVES
-#define MMX_CHAN_HALVES 4
-#endif
-constexpr int kHalves = MMX_CHAN_HALVES;        // warps per TMEM lane quarter (they split a row's 8-column chunks)
-constexpr int kThreadsChan = 128 * kHalves;
 constexpr int kMaxRR = 4;                      // SE bottleneck width served (T // r_se)
 
 struct ChanArgs {
@@ -54,101 +39,6 @@ struct ChanArgs {
     int* abort_count;              // device counter, incremented if a pipeline wait times out (tests assert it stays 0)
 };
 
-// ------------------------------------------------------------------------------------------ dropout masks of the tcgen05 family
-// A dropout site is a [rows][W] tensor; chunk c8 of row `row` covers its columns [8*c8, 8*c8+8).  Four counter-based 32-bit
-// hashes (lowbias32 finaliser over counter ^ key) give 16 random bits per element; an element is kept iff its field >=
-// thresh16.  The key mixes (seed, site, step).  tests/tc5_masks.py is the numpy twin (bit-exact; pinned by a GPU test), which
-// lets the parity tests hand the very same masks to the oracle.
-MMX_HD uint32_t mix32(uint32_t x) {
-    x ^= x >> 16; x *= 0x21f0aaadu; x ^= x >> 15; x *= 0x735a2d97u; x ^= x >> 15;
-    return x;
-}
-MMX_HD uint32_t drop_key(uint32_t seed_lo, uint32_t seed_hi, uint32_t site, uint32_t step) {
-    return mix32(seed_lo ^ mix32(seed_hi ^ mix32(site * 0x9E3779B1u + step)));
-}
-// bit j of the result = keep element 8*c8 + j
-MMX_HD uint32_t keep8(uint32_t key, uint32_t thresh16, uint32_t row, uint32_t W8, uint32_t c8) {
-    const uint32_t base = (row * W8 + c8) * 4u;
-    uint32_t bits = 0;
-#if defined(__CUDA_ARCH__)
-#pragma unroll
-#endif
-    for (uint32_t i = 0; i < 4; ++i) {
-        const uint32_t r = mix32((base + i) ^ key);
-        bits |= ((r & 0xffffu) >= thresh16 ? 1u : 0u) << (2 * i);
-        bits |= ((r >> 16) >= thresh16 ? 1u : 0u) << (2 * i + 1);
-    }
-    return bits;
-}
-
-// ------------------------------------------------------------------------------------------ small device helpers
-MMX_D uint32_t pack_bf16x2(float lo_elem, float hi_elem) {   // lo_elem -> bits [0,16) (lower address)
-    uint32_t r;
-    asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi_elem), "f"(lo_elem));
-    return r;
-}
-// 8 fp32 values -> 8 bf16 "hi" (16 bytes) + 8 bf16 "lo" (16 bytes)
-MMX_D void split8(const float (&v)[8], uint4& hi, uint4& lo) {
-    uint32_t h[4], l[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        h[i] = pack_bf16x2(v[2 * i], v[2 * i + 1]);
-        const float h0 = __uint_as_float(h[i] << 16), h1 = __uint_as_float(h[i] & 0xffff0000u);
-        l[i] = pack_bf16x2(v[2 * i] - h0, v[2 * i + 1] - h1);
-    }
-    hi = make_uint4(h[0], h[1], h[2], h[3]);
-    lo = make_uint4(l[0], l[1], l[2], l[3]);
-}
-
-// instruction descriptor: kind::f16, bf16 x bf16 -> fp32
-MMX_HD uint32_t idesc_bf16(int M, int N, int a_mn_major, int b_mn_major) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)a_mn_major << 15) | ((uint32_t)b_mn_major << 16) |
-           ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-MMX_D void mma_f16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// 16-bit panel operand, rows = M/N index, cols = K index; k0 = first column of this K=16 step
-MMX_D uint64_t dk(uint32_t plane, uint32_t panel_bytes, int k0) { return smem_desc(plane + (uint32_t)(k0 >> 3) * panel_bytes, panel_bytes, 128u); }
-// 16-bit panel operand, rows = K index, cols = M/N index; r0 = first row of this K=16 step
-MMX_D uint64_t dmn(uint32_t plane, uint32_t panel_bytes, int r0) { return smem_desc(plane + (uint32_t)r0 * 16u, 128u, panel_bytes); }
-
-// D (+)= A B^T with split operands: hi*hi + lo*hi + hi*lo.  A: buffer (planes a_hi, a_lo, panel bytes a_ps), B likewise.
-// A_MN / B_MN: orientation of each operand; ksteps K=16 steps.  Issued by ONE thread.
-template <int A_MN, int B_MN>
-MMX_D void gemm3(uint32_t d_tmem, uint32_t a_hi, uint32_t a_lo, uint32_t a_ps, uint32_t b_hi, uint32_t b_lo, uint32_t b_ps, int N,
-                 int ksteps, bool accumulate_first) {
-    const uint32_t id = idesc_bf16(128, N, A_MN, B_MN);
-#pragma unroll 1
-    for (int s = 0; s < ksteps; ++s) {
-        const int k0 = 16 * s;
-        const uint64_t ah = A_MN ? dmn(a_hi, a_ps, k0) : dk(a_hi, a_ps, k0);
-        const uint64_t al = A_MN ? dmn(a_lo, a_ps, k0) : dk(a_lo, a_ps, k0);
-        const uint64_t bh = B_MN ? dmn(b_hi, b_ps, k0) : dk(b_hi, b_ps, k0);
-        const uint64_t bl = B_MN ? dmn(b_lo, b_ps, k0) : dk(b_lo, b_ps, k0);
-        mma_f16(d_tmem, ah, bh, id, (s > 0 || accumulate_first) ? 1u : 0u);
-        mma_f16(d_tmem, al, bh, id, 1u);
-        mma_f16(d_tmem, ah, bl, id, 1u);
-    }
-}
-
-// ------------------------------------------------------------------------------------------ shared-memory plan
-template <int KP>
-struct Plan {
-    static constexpr uint32_t PS = 128 * 16;                 // activation panel: 128 rows x 16 B
-    static constexpr uint32_t PLANE = (KP / 8) * PS;
-    static constexpr uint32_t BUF = 2 * PLANE;               // hi plane + lo plane
-    static constexpr uint32_t WPS = KP * 16;                 // weight panel: KP rows x 16 B
-    static constexpr uint32_t WPLANE = (KP / 8) * WPS;
-    static constexpr uint32_t WBUF = 2 * WPLANE;
-    static constexpr uint32_t SMALL = (4 * KP + 2 * 32 * kMaxRR + 4 * kHalves * 128 + 64) * 4;   // c1f, c2, gamma2, spare | se1, se2 | exchange | barriers
-};
-
 struct Geo {
     int spw, rpw, seq_per_tile, tile_rows, pitch;
 };
@@ -161,114 +51,41 @@ MMX_HD Geo make_geo(int T, int H, int vec) {
     g.pitch = vec == 4 ? H + 4 : H;
     return g;
 }
+// fp32 staging tile of one 128-row tile (+ slack: chunk loads of the last row may run past the row)
+MMX_HD uint32_t stage_bytes(const Geo& g) { return up128((uint32_t)g.tile_rows * g.pitch * 4u + 64u); }
+
+// shared-memory layout (byte offsets from the 1024-aligned base; total includes the alignment slack)
+struct ChanSmem {
+    uint32_t x, y, w1, w2, s1, s2, small, total;
+};
 template <int KP>
-MMX_HD size_t chan_smem_bytes(int T, int H, int vec, bool bwd) {
-    const Geo g = make_geo(T, H, vec);
-    size_t stage = (size_t)g.tile_rows * g.pitch * 4 + 64;    // + slack: chunk loads of the last row may run past the row
-    stage = (stage + 127) / 128 * 128;
-    size_t buf = Plan<KP>::BUF;
-    if (buf < stage) buf = stage;                             // the X region doubles as the output staging tile
-    return 1024 + (bwd ? 2 : 1) * buf + 2 * Plan<KP>::WBUF + (bwd ? 2 : 1) * stage + Plan<KP>::SMALL;
-}
-
-// bulk copy of a tile of activation rows global -> shared (issued by warp 0), completion on `bar`
-template <int VEC>
-MMX_D void stage_in(float* S, const float* g, size_t row0, int nrows, int H, int pitch, uint64_t* bar, int lane) {
-    if (lane == 0) mbar_expect_tx(bar, (uint32_t)nrows * H * 4u);
-    __syncwarp();
-    if (VEC == 2) {
-        if (lane == 0) bulk_g2s(S, g + row0 * H, (uint32_t)nrows * H * 4u, bar);
-    } else {
-        for (int r = lane; r < nrows; r += 32) bulk_g2s(S + (size_t)r * pitch, g + (row0 + r) * H, (uint32_t)H * 4u, bar);
-    }
-}
-template <int VEC>
-MMX_D void stage_out(float* g, const float* S, size_t row0, int nrows, int H, int pitch, int lane) {
-    if (VEC == 2) {
-        if (lane == 0) bulk_s2g(g + row0 * H, S, (uint32_t)nrows * H * 4u);
-    } else {
-        for (int r = lane; r < nrows; r += 32) bulk_s2g(g + (row0 + r) * H, S + (size_t)r * pitch, (uint32_t)H * 4u);
-    }
-    bulk_commit();
-}
-
-// 8 consecutive columns [k0, k0+8) of a staged row; columns >= H read as zero (H % VEC == 0)
-template <int VEC>
-MMX_D void ld8(const float* srow, int k0, int H, float (&v)[8]) {
-#pragma unroll
-    for (int j = 0; j < 8; j += VEC) {
-        if (k0 + j < H) {
-            if (VEC == 4) { const float4 t = *reinterpret_cast<const float4*>(srow + k0 + j); v[j] = t.x; v[j + 1] = t.y; v[j + 2] = t.z; v[j + 3] = t.w; }
-            else { const float2 t = *reinterpret_cast<const float2*>(srow + k0 + j); v[j] = t.x; v[j + 1] = t.y; }
-        } else {
-#pragma unroll
-            for (int i = 0; i < VEC; ++i) v[j + i] = 0.0f;
-        }
-    }
-}
-template <int VEC>
-MMX_D void st8(float* srow, int k0, int H, const float (&v)[8]) {
-#pragma unroll
-    for (int j = 0; j < 8; j += VEC) {
-        if (k0 + j < H) {
-            if (VEC == 4) *reinterpret_cast<float4*>(srow + k0 + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
-            else *reinterpret_cast<float2*>(srow + k0 + j) = make_float2(v[j], v[j + 1]);
-        }
-    }
-}
-MMX_D void ld8s(const float* p, float (&v)[8]) {   // 8 floats from a 16-byte aligned shared array
-    const float4 a = *reinterpret_cast<const float4*>(p), b = *reinterpret_cast<const float4*>(p + 4);
-    v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
-}
-
-MMX_D void put_chunk(uint8_t* buf, uint32_t plane_bytes, uint32_t ps, int row, int c8, const float (&t)[8]) {
-    uint4 hi, lo;
-    split8(t, hi, lo);
-    *reinterpret_cast<uint4*>(buf + c8 * ps + row * 16) = hi;
-    *reinterpret_cast<uint4*>(buf + plane_bytes + c8 * ps + row * 16) = lo;
-}
-
-// stage one weight matrix W[rows][cols] (row-major, optional per-column scale) into a weight buffer (panel layout, KP x KP,
-// zero padded; the buffer must have been zeroed)
-template <int KP>
-MMX_D void stage_weight(uint8_t* wbuf, const float* W, int rows, int cols, const float* colscale, int tid) {
-    if ((cols & 1) == 0) {
-        const int n2 = rows * cols / 2;
-        for (int i = tid; i < n2; i += kThreadsChan) {
-            const int e = 2 * i, r = e / cols, c = e - r * cols;
-            float2 v = *reinterpret_cast<const float2*>(W + e);
-            if (colscale) { v.x *= colscale[c]; v.y *= colscale[c + 1]; }
-            const uint32_t h = pack_bf16x2(v.x, v.y);
-            const uint32_t l = pack_bf16x2(v.x - __uint_as_float(h << 16), v.y - __uint_as_float(h & 0xffff0000u));
-            const uint32_t off = (uint32_t)(c >> 3) * Plan<KP>::WPS + (uint32_t)r * 16u + (uint32_t)(c & 7) * 2u;
-            *reinterpret_cast<uint32_t*>(wbuf + off) = h;
-            *reinterpret_cast<uint32_t*>(wbuf + Plan<KP>::WPLANE + off) = l;
-        }
-    } else {
-        for (int i = tid; i < rows * cols; i += kThreadsChan) {
-            const int r = i / cols, c = i - r * cols;
-            float v = W[i];
-            if (colscale) v *= colscale[c];
-            const uint32_t h = pack_bf16x2(v, 0.0f) & 0xffffu;
-            const uint32_t l = pack_bf16x2(v - __uint_as_float(h << 16), 0.0f) & 0xffffu;
-            const uint32_t off = (uint32_t)(c >> 3) * Plan<KP>::WPS + (uint32_t)r * 16u + (uint32_t)(c & 7) * 2u;
-            *reinterpret_cast<uint16_t*>(wbuf + off) = (uint16_t)h;
-            *reinterpret_cast<uint16_t*>(wbuf + Plan<KP>::WPLANE + off) = (uint16_t)l;
-        }
-    }
+MMX_HD ChanSmem chan_smem(const Geo& g, bool bwd) {
+    using P = Panels<KP>;
+    const uint32_t st = stage_bytes(g), buf = umax(P::BUF, st);    // the X region doubles as the output staging tile
+    ChanSmem m;
+    uint32_t o = 0;
+    m.x = o; o += buf;
+    m.y = bwd ? o : m.x; o += bwd ? buf : 0;                        // backward: second operand
+    m.w1 = o; o += P::WBUF;
+    m.w2 = o; o += P::WBUF;
+    m.s1 = o; o += st;                                              // x1 tile
+    m.s2 = bwd ? o : m.s1; o += bwd ? st : 0;                       // backward: dy tile
+    m.small = o; o += (4 * KP + 2 * 32 * kMaxRR + 4 * kHalves * 128 + 64) * 4;   // c1f, c2, gamma2, spare | se1, se2 | exchange | barriers
+    m.total = o + 1024;
+    return m;
 }
 
 // per-CTA constants: weights (LN2 affine folded into fc1), biases, SE weights.  Contains CTA barriers.
 template <int KP>
 MMX_D void prologue(const ChanArgs& a, uint8_t* w1b, uint8_t* w2b, float* c1f, float* c2, float* gam, float* se1, float* se2, int tid) {
     const int H = a.H, ch = a.ch, T = a.T, rr = a.rr;
-    for (int i = tid; i < (int)(2 * Plan<KP>::WBUF / 16); i += kThreadsChan) reinterpret_cast<uint4*>(w1b)[i] = make_uint4(0, 0, 0, 0);   // w1b, w2b contiguous
-    for (int c = tid; c < KP; c += kThreadsChan) {
+    for (int i = tid; i < (int)(2 * Panels<KP>::WBUF / 16); i += kCtaThreads) reinterpret_cast<uint4*>(w1b)[i] = make_uint4(0, 0, 0, 0);   // w1b, w2b contiguous
+    for (int c = tid; c < KP; c += kCtaThreads) {
         c2[c] = c < H ? a.b2[c] : 0.0f;
         gam[c] = c < H ? a.ln_g[c] : 0.0f;
         c1f[c] = 0.0f;
     }
-    for (int i = tid; i < 32 * kMaxRR; i += kThreadsChan) {
+    for (int i = tid; i < 32 * kMaxRR; i += kCtaThreads) {
         se1[i] = (rr > 0 && i < rr * T) ? a.se1[i] : 0.0f;
         se2[i] = (rr > 0 && i < rr * T) ? a.se2[i] : 0.0f;
     }
@@ -277,7 +94,7 @@ MMX_D void prologue(const ChanArgs& a, uint8_t* w1b, uint8_t* w2b, float* c1f, f
     stage_weight<KP>(w2b, a.w2, H, ch, nullptr, tid);
     // b1'[c] = b1[c] + sum_h W1[c][h] beta2[h]: one warp per row, lanes over h
     const int warp = tid >> 5, lane = tid & 31;
-    for (int c = warp; c < ch; c += kThreadsChan / 32) {
+    for (int c = warp; c < ch; c += kCtaThreads / 32) {
         float s = 0.0f;
         for (int h = lane; h < H; h += 32) s = fmaf(a.w1[(size_t)c * H + h], a.ln_b[h], s);
 #pragma unroll
@@ -306,18 +123,7 @@ MMX_D SeOut se_excite(float s, int t, int seq_base, int T, int rr, const float* 
     return o;
 }
 
-// sum the two halves' partial sums of a row (both halves get the totals).  Contains a CTA barrier.
-MMX_D void row_exchange(float* ex, int half, int prow, float& a, float& b) {
-    if (kHalves == 1) { __syncthreads(); return; }
-    ex[(0 * kHalves + half) * 128 + prow] = a;
-    ex[(1 * kHalves + half) * 128 + prow] = b;
-    __syncthreads();
-    a = 0.0f; b = 0.0f;
-#pragma unroll
-    for (int i = 0; i < kHalves; ++i) { a += ex[(0 * kHalves + i) * 128 + prow]; b += ex[(1 * kHalves + i) * 128 + prow]; }
-}
-
-// common carve-up of the dynamic shared memory
+// pointers into the dynamic shared memory
 template <int KP>
 struct Carve {
     uint8_t *bufX, *bufY, *w1b, *w2b;
@@ -325,19 +131,16 @@ struct Carve {
     uint64_t* bars;
     uint32_t* tslot;
     volatile int* abortf;
-    uint32_t buf_bytes;
     MMX_D Carve(uint8_t* raw, const Geo& g, bool bwd) {
-        using P = Plan<KP>;
         uint8_t* sm = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(raw) + 1023) & ~(uintptr_t)1023);
-        const uint32_t stage_bytes = ((uint32_t)g.tile_rows * g.pitch * 4u + 64u + 127u) / 128u * 128u;
-        buf_bytes = P::BUF > stage_bytes ? P::BUF : stage_bytes;
-        bufX = sm;
-        bufY = bwd ? bufX + buf_bytes : bufX;
-        w1b = bufY + buf_bytes;
-        w2b = w1b + P::WBUF;
-        S1 = reinterpret_cast<float*>(w2b + P::WBUF);
-        S2 = bwd ? reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(S1) + stage_bytes) : S1;
-        c1f = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(S2) + stage_bytes);
+        const ChanSmem m = chan_smem<KP>(g, bwd);
+        bufX = sm + m.x;
+        bufY = sm + m.y;
+        w1b = sm + m.w1;
+        w2b = sm + m.w2;
+        S1 = reinterpret_cast<float*>(sm + m.s1);
+        S2 = reinterpret_cast<float*>(sm + m.s2);
+        c1f = reinterpret_cast<float*>(sm + m.small);
         c2 = c1f + KP;
         gam = c2 + KP;
         se1 = gam + 2 * KP;
@@ -353,8 +156,8 @@ struct Carve {
 // forward
 // ==========================================================================================
 template <int ACT, int KP, int VEC>
-__global__ void __launch_bounds__(kThreadsChan) chan_fwd_kernel(const ChanArgs a) {
-    using P = Plan<KP>;
+__global__ void __launch_bounds__(kCtaThreads) chan_fwd_kernel(const ChanArgs a) {
+    using P = Panels<KP>;
     extern __shared__ uint8_t smem_raw[];
     const Geo g = make_geo(a.T, a.H, VEC);
     Carve<KP> cv(smem_raw, g, false);
@@ -372,13 +175,7 @@ __global__ void __launch_bounds__(kThreadsChan) chan_fwd_kernel(const ChanArgs a
     constexpr int TM_COLS = 3 * KP <= 256 ? 256 : 512;
     constexpr int NCH = KP / 8;
 
-    if (tid == 0) {
-        mbar_init(&bars[0], 1);   // X1 tile landed
-        mbar_init(&bars[1], 1);   // MMA group done
-        *abortf = 0;
-        fence_mbar_init();
-    }
-    if (warp == 0) tmem_alloc<TM_COLS>(cv.tslot);
+    cta_begin<TM_COLS>(bars, 2, abortf, cv.tslot, tid);   // bars: X1 tile landed | MMA group done
     pdl_launch_dependents();
     const int ntiles = (a.B + g.seq_per_tile - 1) / g.seq_per_tile;
     auto tile_nrows = [&](int tile) { return min(g.seq_per_tile, a.B - tile * g.seq_per_tile) * a.T; };
@@ -527,19 +324,15 @@ __global__ void __launch_bounds__(kThreadsChan) chan_fwd_kernel(const ChanArgs a
         __syncthreads();
         if (warp == 0) stage_out<VEC>(a.out, reinterpret_cast<const float*>(bufX), (size_t)tile * g.tile_rows, nrows, H, g.pitch, lane);
     }
-    if (warp == 0) bulk_wait_all0();
-    if (tid == 0 && *abortf) atomicAdd(a.abort_count, 1);
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) tmem_dealloc<TM_COLS>(tmem);
+    cta_end<TM_COLS>(abortf, a.abort_count, tmem, tid);
 }
 
 // ==========================================================================================
 // backward (forward recomputed from x1)
 // ==========================================================================================
 template <int ACT, int KP, int VEC>
-__global__ void __launch_bounds__(kThreadsChan) chan_bwd_kernel(const ChanArgs a) {
-    using P = Plan<KP>;
+__global__ void __launch_bounds__(kCtaThreads) chan_bwd_kernel(const ChanArgs a) {
+    using P = Panels<KP>;
     extern __shared__ uint8_t smem_raw[];
     const Geo g = make_geo(a.T, a.H, VEC);
     Carve<KP> cv(smem_raw, g, true);
@@ -560,14 +353,7 @@ __global__ void __launch_bounds__(kThreadsChan) chan_bwd_kernel(const ChanArgs a
     static_assert(5 * KP <= 512, "TMEM: five KP-column regions");
     constexpr int NCH = KP / 8;
 
-    if (tid == 0) {
-        mbar_init(&bars[0], 1);   // x1 tile landed
-        mbar_init(&bars[1], 1);   // MMA group done
-        mbar_init(&bars[2], 1);   // dy tile landed
-        *abortf = 0;
-        fence_mbar_init();
-    }
-    if (warp == 0) tmem_alloc<TM_COLS>(cv.tslot);
+    cta_begin<TM_COLS>(bars, 3, abortf, cv.tslot, tid);   // bars: x1 tile landed | MMA group done | dy tile landed
     pdl_launch_dependents();
     const int ntiles = (a.B + g.seq_per_tile - 1) / g.seq_per_tile;
     auto tile_nrows = [&](int tile) { return min(g.seq_per_tile, a.B - tile * g.seq_per_tile) * a.T; };
@@ -861,11 +647,11 @@ __global__ void __launch_bounds__(kThreadsChan) chan_bwd_kernel(const ChanArgs a
                 for (int j = 0; j < 8; ++j) stg[prow * SP + 8 * c8 + j] = u[j];
         }
         __syncthreads();
-        for (int i = tid; i < ch * H; i += kThreadsChan) {
+        for (int i = tid; i < ch * H; i += kCtaThreads) {
             const int c = i / H, h = i - c * H;
             red_add(a.g_w1 + i, stg[c * SP + h] * cv.gam[h]);
         }
-        for (int h = tid; h < H; h += kThreadsChan) {
+        for (int h = tid; h < H; h += kCtaThreads) {
             float sg = 0.0f, sb = 0.0f;
 #pragma unroll 8
             for (int c = 0; c < ch; ++c) {
@@ -876,7 +662,7 @@ __global__ void __launch_bounds__(kThreadsChan) chan_bwd_kernel(const ChanArgs a
             red_add(a.g_ln_g + h, sg);
             red_add(a.g_ln_b + h, sb);
         }
-        for (int c = tid; c < ch; c += kThreadsChan) red_add(a.g_b1 + c, stg[c * SP + H]);
+        for (int c = tid; c < ch; c += kCtaThreads) red_add(a.g_b1 + c, stg[c * SP + H]);
         __syncthreads();
 #pragma unroll 1
         for (int c8 = half; c8 < NCH; c8 += kHalves) {
@@ -888,15 +674,15 @@ __global__ void __launch_bounds__(kThreadsChan) chan_bwd_kernel(const ChanArgs a
                 for (int j = 0; j < 8; ++j) stg[prow * SP + 8 * c8 + j] = u[j];
         }
         __syncthreads();
-        for (int i = tid; i < H * ch; i += kThreadsChan) {
+        for (int i = tid; i < H * ch; i += kCtaThreads) {
             const int h = i / ch, c = i - h * ch;
             red_add(a.g_w2 + i, stg[h * SP + c]);
         }
-        for (int h = tid; h < H; h += kThreadsChan) red_add(a.g_b2 + h, stg[h * SP + ch]);
+        for (int h = tid; h < H; h += kCtaThreads) red_add(a.g_b2 + h, stg[h * SP + ch]);
         if (rr > 0) {
             __syncthreads();
             float* acc = stg;                                  // [2][rr*T]
-            for (int i = tid; i < 2 * rr * T; i += kThreadsChan) acc[i] = 0.0f;
+            for (int i = tid; i < 2 * rr * T; i += kCtaThreads) acc[i] = 0.0f;
             __syncthreads();
             if (lane_ok && half == 0)
                 for (int k = 0; k < rr; ++k) {
@@ -904,16 +690,13 @@ __global__ void __launch_bounds__(kThreadsChan) chan_bwd_kernel(const ChanArgs a
                     atomicAdd(acc + rr * T + t * rr + k, gS2[k]);    // dS2[t][k]
                 }
             __syncthreads();
-            for (int i = tid; i < rr * T; i += kThreadsChan) {
+            for (int i = tid; i < rr * T; i += kCtaThreads) {
                 red_add(a.g_se1 + i, acc[i]);
                 red_add(a.g_se2 + i, acc[rr * T + i]);
             }
         }
     }
-    if (tid == 0 && *abortf) atomicAdd(a.abort_count, 1);
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) tmem_dealloc<TM_COLS>(tmem);
+    cta_end<TM_COLS>(abortf, a.abort_count, tmem, tid);
 }
 
 }  // namespace chan

@@ -22,22 +22,29 @@ using namespace tc5;
 using namespace chan;
 
 constexpr int KPW = 128;                                    // widest operand served
-template <int KP> constexpr uint32_t ws_bytes() { return 2 * Plan<KP>::WBUF + KP * 4; }      // W1' planes | W2 planes | b1'
-constexpr uint32_t kWsBytes = 2 * Plan<KPW>::WBUF + KPW * 4;                                  // allocation size (any KP <= KPW)
-template <int KP> constexpr uint32_t small_w() { return (6 * KP + 2 * 32 * kMaxRR + 4 * kHalves * 128 + 64) * 4; }   // c1f, c2, gamma2, db1, db2, spare | se1, se2 | exchange | barriers
+constexpr uint32_t kWsBytes = 2 * Panels<KPW>::WBUF + KPW * 4;    // workspace: W1' planes | W2 planes | b1' (any KP <= KPW)
 
-MMX_HD uint32_t stage_bytes_of(const Geo& g) { return ((uint32_t)g.tile_rows * g.pitch * 4u + 64u + 127u) / 128u * 128u; }
+// shared-memory layout (byte offsets from the 1024-aligned base; total includes the alignment slack)
+struct WideSmem {
+    uint32_t x, y, slot, s, small, total;
+};
 template <int KP>
-MMX_HD size_t wide_smem_bytes(int T, int H, int vec, bool bwd) {
-    const Geo g = make_geo(T, H, vec);
-    const uint32_t st = stage_bytes_of(g);
-    const uint32_t buf = Plan<KP>::BUF > st ? Plan<KP>::BUF : st;
-    return 1024 + (bwd ? 2 * buf : buf + st) + Plan<KP>::WBUF + small_w<KP>();
+MMX_HD WideSmem wide_smem(const Geo& g, bool bwd) {
+    using P = Panels<KP>;
+    const uint32_t st = stage_bytes(g), buf = umax(P::BUF, st);
+    WideSmem m;
+    uint32_t o = 0;
+    m.x = o; o += buf;
+    m.y = bwd ? o : m.x; o += bwd ? buf : 0;
+    m.slot = o; o += P::WBUF;
+    m.s = bwd ? m.y : o; o += bwd ? 0 : st;                         // backward: the x1 tile lands in the Y region
+    m.small = o; o += (6 * KP + 2 * 32 * kMaxRR + 4 * kHalves * 128 + 64) * 4;   // c1f, c2, gamma2, db1, db2, spare | se1, se2 | exchange | barriers
+    m.total = o + 1024;
+    return m;
 }
 
-template <int KPW>
+template <int KP>
 struct CarveW {
-    using PW = Plan<KPW>;
     uint8_t *bufX, *bufY, *slot;
     float *S, *c1f, *c2, *gam, *db1, *db2, *se1, *se2, *ex;
     uint64_t* bars;
@@ -45,18 +52,17 @@ struct CarveW {
     volatile int* abortf;
     MMX_D CarveW(uint8_t* raw, const Geo& g, bool bwd) {
         uint8_t* sm = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(raw) + 1023) & ~(uintptr_t)1023);
-        const uint32_t st = stage_bytes_of(g);
-        const uint32_t buf = PW::BUF > st ? PW::BUF : st;
-        bufX = sm;
-        bufY = bwd ? bufX + buf : bufX;
-        slot = bufY + buf;
-        S = bwd ? reinterpret_cast<float*>(bufY) : reinterpret_cast<float*>(slot + PW::WBUF);     // backward: the x1 tile lands in the Y region
-        c1f = reinterpret_cast<float*>(slot + PW::WBUF + (bwd ? 0 : st));
-        c2 = c1f + KPW;
-        gam = c2 + KPW;
-        db1 = gam + KPW;
-        db2 = db1 + KPW;
-        se1 = db2 + 2 * KPW;
+        const WideSmem m = wide_smem<KP>(g, bwd);
+        bufX = sm + m.x;
+        bufY = sm + m.y;
+        slot = sm + m.slot;
+        S = reinterpret_cast<float*>(sm + m.s);
+        c1f = reinterpret_cast<float*>(sm + m.small);
+        c2 = c1f + KP;
+        gam = c2 + KP;
+        db1 = gam + KP;
+        db2 = db1 + KP;
+        se1 = db2 + 2 * KP;
         se2 = se1 + 32 * kMaxRR;
         ex = se2 + 32 * kMaxRR;
         bars = reinterpret_cast<uint64_t*>(ex + 4 * kHalves * 128);
@@ -69,30 +75,28 @@ struct CarveW {
 // ws: W1' (hi plane, lo plane) | W2 (hi, lo) | b1'   -- panel layout, KPW x KPW, zero padded
 template <int KPW>
 static __global__ void __launch_bounds__(256) chan_prep_kernel(const ChanArgs a, uint8_t* ws) {
-    using PW = Plan<KPW>;
+    using PW = Panels<KPW>;
     pdl_launch_dependents();
     pdl_wait();                // the previous kernel in the stream may still be reading the workspace
     const int H = a.H, ch = a.ch;
     const int gt = blockIdx.x * blockDim.x + threadIdx.x, nt = gridDim.x * blockDim.x;
     for (int i = gt; i < KPW * KPW / 2; i += nt) {
         const int e = 2 * i, r = e / KPW, c = e - r * KPW;
-        const uint32_t off = (uint32_t)(c >> 3) * PW::WPS + (uint32_t)r * 16u + (uint32_t)(c & 7) * 2u;
+        const uint32_t off = panel_off(r, c, PW::WPS);
         float2 v = make_float2(0.0f, 0.0f);
         if (r < ch && c < H) {
             v = *reinterpret_cast<const float2*>(a.w1 + (size_t)r * H + c);
             v.x *= a.ln_g[c];
             v.y *= a.ln_g[c + 1];
         }
-        uint32_t h = pack_bf16x2(v.x, v.y);
-        uint32_t l = pack_bf16x2(v.x - __uint_as_float(h << 16), v.y - __uint_as_float(h & 0xffff0000u));
-        *reinterpret_cast<uint32_t*>(ws + off) = h;
-        *reinterpret_cast<uint32_t*>(ws + PW::WPLANE + off) = l;
+        Split sp = split2(v.x, v.y);
+        *reinterpret_cast<uint32_t*>(ws + off) = sp.hi;
+        *reinterpret_cast<uint32_t*>(ws + PW::WPLANE + off) = sp.lo;
         v = make_float2(0.0f, 0.0f);
         if (r < H && c < ch) v = *reinterpret_cast<const float2*>(a.w2 + (size_t)r * ch + c);
-        h = pack_bf16x2(v.x, v.y);
-        l = pack_bf16x2(v.x - __uint_as_float(h << 16), v.y - __uint_as_float(h & 0xffff0000u));
-        *reinterpret_cast<uint32_t*>(ws + PW::WBUF + off) = h;
-        *reinterpret_cast<uint32_t*>(ws + PW::WBUF + PW::WPLANE + off) = l;
+        sp = split2(v.x, v.y);
+        *reinterpret_cast<uint32_t*>(ws + PW::WBUF + off) = sp.hi;
+        *reinterpret_cast<uint32_t*>(ws + PW::WBUF + PW::WPLANE + off) = sp.lo;
     }
     float* c1f = reinterpret_cast<float*>(ws + 2 * PW::WBUF);
     const int warp = gt >> 5, lane = gt & 31, nw = nt >> 5;
@@ -110,13 +114,13 @@ static __global__ void __launch_bounds__(256) chan_prep_kernel(const ChanArgs a,
 template <int KPW>
 MMX_D void small_params(const ChanArgs& a, const CarveW<KPW>& cv, int tid) {
     const int H = a.H, T = a.T, rr = a.rr;
-    for (int c = tid; c < KPW; c += kThreadsChan) {
+    for (int c = tid; c < KPW; c += kCtaThreads) {
         cv.c2[c] = c < H ? a.b2[c] : 0.0f;
         cv.gam[c] = c < H ? a.ln_g[c] : 0.0f;
         cv.db1[c] = 0.0f;
         cv.db2[c] = 0.0f;
     }
-    for (int i = tid; i < 32 * kMaxRR; i += kThreadsChan) {
+    for (int i = tid; i < 32 * kMaxRR; i += kCtaThreads) {
         cv.se1[i] = (rr > 0 && i < rr * T) ? a.se1[i] : 0.0f;
         cv.se2[i] = (rr > 0 && i < rr * T) ? a.se2[i] : 0.0f;
     }
@@ -125,8 +129,8 @@ MMX_D void small_params(const ChanArgs& a, const CarveW<KPW>& cv, int tid) {
 
 template <int KPW>
 MMX_D void load_weight(uint8_t* slot, const uint8_t* ws, int which, uint64_t* bar) {   // one thread
-    mbar_expect_tx(bar, Plan<KPW>::WBUF);
-    bulk_g2s(slot, ws + (size_t)which * Plan<KPW>::WBUF, Plan<KPW>::WBUF, bar);
+    mbar_expect_tx(bar, Panels<KPW>::WBUF);
+    bulk_g2s(slot, ws + (size_t)which * Panels<KPW>::WBUF, Panels<KPW>::WBUF, bar);
 }
 
 // column sums over the warp's 32 rows of an 8-column chunk: lanes with (lane & 3) == 0 return the total of column
@@ -158,7 +162,7 @@ MMX_D void col_accumulate(float* dst, int c8, const float (&v)[8], int lane) {
 // xhat chunk from the operand's hi + lo planes (|error| <= 2^-17 |xhat|)
 template <int KPW>
 MMX_D void xhat_from_planes(const uint8_t* buf, int row, int c8, float (&xh)[8]) {
-    using PW = Plan<KPW>;
+    using PW = Panels<KPW>;
     const uint4 h = *reinterpret_cast<const uint4*>(buf + c8 * PW::PS + row * 16);
     const uint4 l = *reinterpret_cast<const uint4*>(buf + PW::PLANE + c8 * PW::PS + row * 16);
     const uint32_t hw[4] = {h.x, h.y, h.z, h.w}, lw[4] = {l.x, l.y, l.z, l.w};
@@ -173,8 +177,8 @@ MMX_D void xhat_from_planes(const uint8_t* buf, int row, int c8, float (&xh)[8])
 // forward
 // ==========================================================================================
 template <int ACT, int VEC, int KP>
-__global__ void __launch_bounds__(kThreadsChan, KP <= 64 ? 2 : 1) chan_wide_fwd_kernel(const ChanArgs a, const uint8_t* ws) {
-    using P = Plan<KP>;
+__global__ void __launch_bounds__(kCtaThreads, KP <= 64 ? 2 : 1) chan_wide_fwd_kernel(const ChanArgs a, const uint8_t* ws) {
+    using P = Panels<KP>;
     extern __shared__ uint8_t smem_raw[];
     const Geo g = make_geo(a.T, a.H, VEC);
     const CarveW<KP> cv(smem_raw, g, false);
@@ -193,20 +197,13 @@ __global__ void __launch_bounds__(kThreadsChan, KP <= 64 ? 2 : 1) chan_wide_fwd_
     static_assert(TM_COLS == 256 || TM_COLS == 512, "KP = 64 or 128");
     constexpr int NCH = KP / 8;
 
-    if (tid == 0) {
-        mbar_init(&bars[0], 1);   // x1 tile landed
-        mbar_init(&bars[1], 1);   // MMA group done
-        mbar_init(&bars[2], 1);   // weight slot landed
-        *abortf = 0;
-        fence_mbar_init();
-    }
-    if (warp == 0) tmem_alloc<TM_COLS>(cv.tslot);
+    cta_begin<TM_COLS>(bars, 3, abortf, cv.tslot, tid);   // bars: x1 tile landed | MMA group done | weight slot landed
     pdl_launch_dependents();
     const int ntiles = (a.B + g.seq_per_tile - 1) / g.seq_per_tile;
     auto tile_nrows = [&](int tile) { return min(g.seq_per_tile, a.B - tile * g.seq_per_tile) * a.T; };
     small_params(a, cv, tid);
     pdl_wait();                // the prep kernel (and everything before it) has completed: workspace and x1 are readable
-    for (int c = tid; c < KP; c += kThreadsChan) cv.c1f[c] = reinterpret_cast<const float*>(ws + 2 * P::WBUF)[c];
+    for (int c = tid; c < KP; c += kCtaThreads) cv.c1f[c] = reinterpret_cast<const float*>(ws + 2 * P::WBUF)[c];
     uint32_t ph_w = 0;
     if ((int)blockIdx.x < ntiles) {
         if (tid == 0) load_weight<KP>(cv.slot, ws, 0, &bars[2]);
@@ -357,19 +354,15 @@ __global__ void __launch_bounds__(kThreadsChan, KP <= 64 ? 2 : 1) chan_wide_fwd_
         __syncthreads();
         if (warp == 0) stage_out<VEC>(a.out, reinterpret_cast<const float*>(bufX), (size_t)tile * g.tile_rows, nrows, H, g.pitch, lane);
     }
-    if (warp == 0) bulk_wait_all0();
-    if (tid == 0 && *abortf) atomicAdd(a.abort_count, 1);
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) tmem_dealloc<TM_COLS>(tmem);
+    cta_end<TM_COLS>(abortf, a.abort_count, tmem, tid);
 }
 
 // ==========================================================================================
 // backward (forward recomputed from x1)
 // ==========================================================================================
 template <int ACT, int VEC, int KP>
-__global__ void __launch_bounds__(kThreadsChan, KP <= 64 ? 2 : 1) chan_wide_bwd_kernel(const ChanArgs a, const uint8_t* ws) {
-    using P = Plan<KP>;
+__global__ void __launch_bounds__(kCtaThreads, KP <= 64 ? 2 : 1) chan_wide_bwd_kernel(const ChanArgs a, const uint8_t* ws) {
+    using P = Panels<KP>;
     extern __shared__ uint8_t smem_raw[];
     const Geo g = make_geo(a.T, a.H, VEC);
     const CarveW<KP> cv(smem_raw, g, true);
@@ -390,20 +383,13 @@ __global__ void __launch_bounds__(kThreadsChan, KP <= 64 ? 2 : 1) chan_wide_bwd_
     constexpr int NCH = KP / 8;
     constexpr int CPT = NCH / kHalves;        // chunks per thread and pass
 
-    if (tid == 0) {
-        mbar_init(&bars[0], 1);   // x1 tile landed
-        mbar_init(&bars[1], 1);   // MMA group done
-        mbar_init(&bars[2], 1);   // weight slot landed
-        *abortf = 0;
-        fence_mbar_init();
-    }
-    if (warp == 0) tmem_alloc<TM_COLS>(cv.tslot);
+    cta_begin<TM_COLS>(bars, 3, abortf, cv.tslot, tid);   // bars: x1 tile landed | MMA group done | weight slot landed
     pdl_launch_dependents();
     const int ntiles = (a.B + g.seq_per_tile - 1) / g.seq_per_tile;
     auto tile_nrows = [&](int tile) { return min(g.seq_per_tile, a.B - tile * g.seq_per_tile) * a.T; };
     small_params(a, cv, tid);
     pdl_wait();
-    for (int c = tid; c < KP; c += kThreadsChan) cv.c1f[c] = reinterpret_cast<const float*>(ws + 2 * P::WBUF)[c];
+    for (int c = tid; c < KP; c += kCtaThreads) cv.c1f[c] = reinterpret_cast<const float*>(ws + 2 * P::WBUF)[c];
     uint32_t ph_w = 0;
     if ((int)blockIdx.x < ntiles) {
         if (tid == 0) load_weight<KP>(cv.slot, ws, 0, &bars[2]);
@@ -697,11 +683,11 @@ __global__ void __launch_bounds__(kThreadsChan, KP <= 64 ? 2 : 1) chan_wide_bwd_
                 for (int j = 0; j < 8; ++j) stg[prow * KP + ((8 * c8 + j + prow) & (KP - 1))] = u[j];
         }
         __syncthreads();
-        for (int i = tid; i < ch * H; i += kThreadsChan) {
+        for (int i = tid; i < ch * H; i += kCtaThreads) {
             const int c = i / H, h = i - c * H;
             red_add(a.g_w1 + i, stg[c * KP + ((h + c) & (KP - 1))] * cv.gam[h]);
         }
-        for (int h = tid; h < H; h += kThreadsChan) {
+        for (int h = tid; h < H; h += kCtaThreads) {
             float sg = 0.0f, sb = 0.0f;
 #pragma unroll 8
             for (int c = 0; c < ch; ++c) {
@@ -712,7 +698,7 @@ __global__ void __launch_bounds__(kThreadsChan, KP <= 64 ? 2 : 1) chan_wide_bwd_
             red_add(a.g_ln_g + h, sg);
             red_add(a.g_ln_b + h, sb);
         }
-        for (int c = tid; c < ch; c += kThreadsChan) red_add(a.g_b1 + c, cv.db1[c]);
+        for (int c = tid; c < ch; c += kCtaThreads) red_add(a.g_b1 + c, cv.db1[c]);
         __syncthreads();
 #pragma unroll 1
         for (int c8 = half; c8 < NCH; c8 += kHalves) {
@@ -724,15 +710,15 @@ __global__ void __launch_bounds__(kThreadsChan, KP <= 64 ? 2 : 1) chan_wide_bwd_
                 for (int j = 0; j < 8; ++j) stg[prow * KP + ((8 * c8 + j + prow) & (KP - 1))] = u[j];
         }
         __syncthreads();
-        for (int i = tid; i < H * ch; i += kThreadsChan) {
+        for (int i = tid; i < H * ch; i += kCtaThreads) {
             const int h = i / ch, c = i - h * ch;
             red_add(a.g_w2 + i, stg[h * KP + ((c + h) & (KP - 1))]);
         }
-        for (int h = tid; h < H; h += kThreadsChan) red_add(a.g_b2 + h, cv.db2[h]);
+        for (int h = tid; h < H; h += kCtaThreads) red_add(a.g_b2 + h, cv.db2[h]);
         if (rr > 0) {
             __syncthreads();
             float* acc = stg;                                  // [2][rr*T]
-            for (int i = tid; i < 2 * rr * T; i += kThreadsChan) acc[i] = 0.0f;
+            for (int i = tid; i < 2 * rr * T; i += kCtaThreads) acc[i] = 0.0f;
             __syncthreads();
             if (lane_ok && half == 0)
                 for (int k = 0; k < rr; ++k) {
@@ -740,16 +726,13 @@ __global__ void __launch_bounds__(kThreadsChan, KP <= 64 ? 2 : 1) chan_wide_bwd_
                     atomicAdd(acc + rr * T + t * rr + k, gS2[k]);    // dS2[t][k]
                 }
             __syncthreads();
-            for (int i = tid; i < rr * T; i += kThreadsChan) {
+            for (int i = tid; i < rr * T; i += kCtaThreads) {
                 red_add(a.g_se1 + i, acc[i]);
                 red_add(a.g_se2 + i, acc[rr * T + i]);
             }
         }
     }
-    if (tid == 0 && *abortf) atomicAdd(a.abort_count, 1);
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) tmem_dealloc<TM_COLS>(tmem);
+    cta_end<TM_COLS>(abortf, a.abort_count, tmem, tid);
 }
 
 }  // namespace chanw

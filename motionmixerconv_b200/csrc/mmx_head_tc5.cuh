@@ -11,23 +11,21 @@
 //     out = P Wf^T + bf
 // Backward (forward recomputed): dP = dOut Wf, dWf += dOut^T [P | 1], dZ = Wbd^T dP, and the time-mix weight gradient comes
 // out of G += dP Z^T (128 x 128, accumulated in TMEM over the CTA's tiles) whose diagonal blocks are summed at the end.
-// All products use bf16 hi+lo split operands (three MMAs each, fp32 accumulation), as in mmx_chan_tc5.cuh.
+// All products use bf16 hi+lo split operands (three MMAs each, fp32 accumulation): the bf16x3 toolkit of mmx_tc5.cuh.
 #pragma once
-#include "mmx_chan_tc5.cuh"
+#include "mmx_tc5.cuh"
 
 namespace mmx {
 namespace head {
 
 using namespace tc5;
-using chan::kHalves;
-using chan::kThreadsChan;
 
 constexpr int KH = 64;     // padded hidden width: H + 1 <= KH (the ones column of the bias gradient)
 constexpr int KD = 80;     // padded output width: D <= KD
-constexpr uint32_t PS = 128 * 16;
-constexpr uint32_t HPLANE = (KH / 8) * PS, HBUF = 2 * HPLANE;       // operands with H-wide rows
-constexpr uint32_t DPLANE = (KD / 8) * PS, DBUF = 2 * DPLANE;       // operands with D-wide rows
-constexpr uint32_t BDPLANE = 16 * PS, BDBUF = 2 * BDPLANE;          // block-diagonal time-mix matrix 128 x 128
+using PH = Panels<KH>;      // operands with H-wide rows
+using PD = Panels<KD>;      // operands with D-wide rows, and the weight Wf [D][H]
+using PB = Panels<128>;     // block-diagonal time-mix matrix 128 x 128
+constexpr uint32_t PS = PH::PS;
 constexpr int CPT = KH / 8 / kHalves;                               // chunks of a hidden row per thread
 static_assert(CPT * kHalves * 8 == KH, "KH must split evenly over the halves");
 
@@ -41,8 +39,6 @@ struct HeadArgs {
     int* abort_count;
 };
 
-MMX_HD uint32_t up128(uint32_t v) { return (v + 127u) / 128u * 128u; }
-MMX_HD uint32_t umax(uint32_t a, uint32_t b) { return a > b ? a : b; }
 constexpr uint32_t kSmallFloats = 128 + KD + 2 * KH + 4 * kHalves * 128 + 2 * KH + 128 + 64;   // bt per row | bf | gamma, beta | exchange | dgamma, dbeta | dbt | barriers
 
 struct HeadSmem {
@@ -52,12 +48,12 @@ MMX_HD HeadSmem head_smem(int H, int D, bool bwd) {
     HeadSmem m;
     const uint32_t st_in = up128(128u * H * 4u + 64u), st_out = up128(128u * D * 4u + 64u);
     uint32_t o = 0;
-    m.x = o; o += bwd ? umax(HBUF, st_in) : umax(HBUF, st_out);     // Z operand; doubles as the output staging tile
-    m.y = o; o += bwd ? umax(HBUF, st_out) : HBUF;                  // P operand (backward: also the landing zone of the dOut tile)
-    m.o = o; o += bwd ? umax(DBUF, st_in) : 0;                      // backward: dOut / dP operand (also the landing zone of the x tile)
-    m.wbd = o; o += BDBUF;
-    m.wf = o; o += chan::Plan<KD>::WBUF;
-    m.s1 = o; o += bwd ? 0 : st_in;                                 // forward: x tile
+    m.x = o; o += bwd ? umax(PH::BUF, st_in) : umax(PH::BUF, st_out);   // Z operand; doubles as the output staging tile
+    m.y = o; o += bwd ? umax(PH::BUF, st_out) : PH::BUF;                // P operand (backward: also the landing zone of the dOut tile)
+    m.o = o; o += bwd ? umax(PD::BUF, st_in) : 0;                       // backward: dOut / dP operand (also the landing zone of the x tile)
+    m.wbd = o; o += PB::BUF;
+    m.wf = o; o += PD::WBUF;
+    m.s1 = o; o += bwd ? 0 : st_in;                                     // forward: x tile
     m.small = o; o += kSmallFloats * 4;
     m.total = o + 1024;
     return m;
@@ -86,26 +82,24 @@ struct Small {
 // parameters -> shared memory.  Contains CTA barriers.
 MMX_D void head_prologue(const HeadArgs& a, uint8_t* wbd, uint8_t* wfb, const Small& sm, int tid) {
     const int T = a.T, To = a.To, S = a.S;
-    for (int i = tid; i < (int)((BDBUF + chan::Plan<KD>::WBUF) / 16); i += kThreadsChan) reinterpret_cast<uint4*>(wbd)[i] = make_uint4(0, 0, 0, 0);   // wbd, wf contiguous
-    for (int r = tid; r < 128; r += kThreadsChan) { sm.btrow[r] = r < S * To ? a.bt[r % To] : 0.0f; sm.dbt[r] = 0.0f; }
-    for (int c = tid; c < KD; c += kThreadsChan) sm.bf[c] = c < a.D ? a.bf[c] : 0.0f;
-    for (int c = tid; c < KH; c += kThreadsChan) {
+    for (int i = tid; i < (int)((PB::BUF + PD::WBUF) / 16); i += kCtaThreads) reinterpret_cast<uint4*>(wbd)[i] = make_uint4(0, 0, 0, 0);   // wbd, wf contiguous
+    for (int r = tid; r < 128; r += kCtaThreads) { sm.btrow[r] = r < S * To ? a.bt[r % To] : 0.0f; sm.dbt[r] = 0.0f; }
+    for (int c = tid; c < KD; c += kCtaThreads) sm.bf[c] = c < a.D ? a.bf[c] : 0.0f;
+    for (int c = tid; c < KH; c += kCtaThreads) {
         sm.gam[c] = c < a.H ? a.ln_g[c] : 0.0f;
         sm.bet[c] = c < a.H ? a.ln_b[c] : 0.0f;
         sm.dgam[c] = 0.0f;
         sm.dbet[c] = 0.0f;
     }
     __syncthreads();
-    chan::stage_weight<KD>(wfb, a.wf, a.D, a.H, nullptr, tid);
-    for (int i = tid; i < S * To * T; i += kThreadsChan) {
+    stage_weight<KD>(wfb, a.wf, a.D, a.H, nullptr, tid);
+    for (int i = tid; i < S * To * T; i += kCtaThreads) {
         const int s = i / (To * T), ot = i - s * To * T, o = ot / T, t = ot - o * T;
         const int row = s * To + o, col = s * T + t;
-        const float v = a.wt[ot];
-        const uint32_t h = chan::pack_bf16x2(v, 0.0f) & 0xffffu;
-        const uint32_t l = chan::pack_bf16x2(v - __uint_as_float(h << 16), 0.0f) & 0xffffu;
-        const uint32_t off = (uint32_t)(col >> 3) * PS + (uint32_t)row * 16u + (uint32_t)(col & 7) * 2u;
-        *reinterpret_cast<uint16_t*>(wbd + off) = (uint16_t)h;
-        *reinterpret_cast<uint16_t*>(wbd + BDPLANE + off) = (uint16_t)l;
+        const Split sp = split1(a.wt[ot]);
+        const uint32_t off = panel_off(row, col, PS);
+        *reinterpret_cast<uint16_t*>(wbd + off) = (uint16_t)sp.hi;
+        *reinterpret_cast<uint16_t*>(wbd + PB::PLANE + off) = (uint16_t)sp.lo;
     }
 }
 
@@ -118,7 +112,7 @@ MMX_D void ln_row_stats(const float* srow, bool valid, int H, int half, int prow
 #pragma unroll 1
         for (int c8 = half; c8 < nchH; c8 += kHalves) {
             float v[8];
-            chan::ld8<2>(srow, 8 * c8, H, v);
+            ld8<2>(srow, 8 * c8, H, v);
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
                 const float dv = 8 * c8 + j < H ? v[j] - c0 : 0.0f;
@@ -127,7 +121,7 @@ MMX_D void ln_row_stats(const float* srow, bool valid, int H, int half, int prow
             }
         }
     }
-    chan::row_exchange(ex, half, prow, s, ss);
+    row_exchange(ex, half, prow, s, ss);
     const float ms = s / (float)H;
     mean = c0 + ms;
     rstd = 1.0f / sqrtf(fmaxf(ss / (float)H - ms * ms, 0.0f) + 1e-5f);
@@ -136,7 +130,7 @@ MMX_D void ln_row_stats(const float* srow, bool valid, int H, int half, int prow
 // ==========================================================================================
 // forward
 // ==========================================================================================
-__global__ void __launch_bounds__(kThreadsChan) head_fwd_kernel(const HeadArgs a) {
+__global__ void __launch_bounds__(kCtaThreads) head_fwd_kernel(const HeadArgs a) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
     const HeadSmem m = head_smem(a.H, a.D, false);
@@ -149,8 +143,7 @@ __global__ void __launch_bounds__(kThreadsChan) head_fwd_kernel(const HeadArgs a
     const int prow = qtr * 32 + lane;
     const int T = a.T, To = a.To, H = a.H, D = a.D, S = a.S;
     constexpr int TM_COLS = 256;
-    if (tid == 0) { mbar_init(&bars[0], 1); mbar_init(&bars[1], 1); *abortf = 0; fence_mbar_init(); }
-    if (warp == 0) tmem_alloc<TM_COLS>(sm.tslot);
+    cta_begin<TM_COLS>(bars, 2, abortf, sm.tslot, tid);
     pdl_launch_dependents();
     head_prologue(a, wbd, wfb, sm, tid);
     pdl_wait();
@@ -184,12 +177,12 @@ __global__ void __launch_bounds__(kThreadsChan) head_fwd_kernel(const HeadArgs a
 #pragma unroll 1
         for (int c8 = half; c8 < KH / 8; c8 += kHalves) {
             float v[8], g[8], b[8];
-            chan::ld8<2>(srow, 8 * c8, vin ? H : 0, v);
-            chan::ld8s(sm.gam + 8 * c8, g);
-            chan::ld8s(sm.bet + 8 * c8, b);
+            ld8<2>(srow, 8 * c8, vin ? H : 0, v);
+            ld8s(sm.gam + 8 * c8, g);
+            ld8s(sm.bet + 8 * c8, b);
 #pragma unroll
             for (int j = 0; j < 8; ++j) v[j] = (vin && 8 * c8 + j < H) ? fmaf((v[j] - mean) * rstd, g[j], b[j]) : 0.0f;
-            chan::put_chunk(bufX, HPLANE, PS, prow, c8, v);
+            put_chunk(bufX, PH::PLANE, PS, prow, c8, v);
         }
         fence_async_smem();
         tc_fence_before();
@@ -199,7 +192,7 @@ __global__ void __launch_bounds__(kThreadsChan) head_fwd_kernel(const HeadArgs a
             if (next < ntiles) load_x(next);
             tc_fence_after();
             // P[(s,o)][h] = sum_(s',t) Wbd[(s,o)][(s',t)] Z[(s',t)][h]     (A K-major, B = Z read MN-major: K = rows)
-            chan::gemm3<0, 1>(tP, bdB, bdB + BDPLANE, PS, xB, xB + HPLANE, PS, KH, 128 / 16, false);
+            gemm3<0, 1>(tP, bdB, bdB + PB::PLANE, PS, xB, xB + PH::PLANE, PS, KH, 128 / 16, false);
             mma_commit(&bars[1]);
         }
         // ---------------- E1: P + bt -> operand Y
@@ -215,7 +208,7 @@ __global__ void __launch_bounds__(kThreadsChan) head_fwd_kernel(const HeadArgs a
                 tmem_wait_ld();
 #pragma unroll
                 for (int j = 0; j < 8; ++j) u[j] = (vout && 8 * c8 + j < H) ? u[j] + bt : 0.0f;
-                chan::put_chunk(bufY, HPLANE, PS, prow, c8, u);
+                put_chunk(bufY, PH::PLANE, PS, prow, c8, u);
             }
         }
         fence_async_smem();
@@ -223,7 +216,7 @@ __global__ void __launch_bounds__(kThreadsChan) head_fwd_kernel(const HeadArgs a
         __syncthreads();
         if (tid == 0) {
             tc_fence_after();
-            chan::gemm3<0, 0>(tO, yB, yB + HPLANE, PS, wfB, wfB + chan::Plan<KD>::WPLANE, chan::Plan<KD>::WPS, KD, KH / 16, false);
+            gemm3<0, 0>(tO, yB, yB + PH::PLANE, PS, wfB, wfB + PD::WPLANE, PD::WPS, KD, KH / 16, false);
             mma_commit(&bars[1]);
         }
         // ---------------- E2: out = . + bf -> staged rows -> global
@@ -236,11 +229,11 @@ __global__ void __launch_bounds__(kThreadsChan) head_fwd_kernel(const HeadArgs a
             for (int c8 = half; c8 < nchD; c8 += kHalves) {
                 float u[8], b[8];
                 tmem_ld8(tmem_addr(tO, qtr, 8 * c8), u);
-                chan::ld8s(sm.bf + 8 * c8, b);
+                ld8s(sm.bf + 8 * c8, b);
                 tmem_wait_ld();
 #pragma unroll
                 for (int j = 0; j < 8; ++j) u[j] += b[j];
-                if (vout) chan::st8<2>(orow, 8 * c8, D, u);
+                if (vout) st8<2>(orow, 8 * c8, D, u);
             }
         }
         tc_fence_before();
@@ -251,17 +244,13 @@ __global__ void __launch_bounds__(kThreadsChan) head_fwd_kernel(const HeadArgs a
             bulk_commit();
         }
     }
-    if (warp == 0) bulk_wait_all0();
-    if (tid == 0 && *abortf) atomicAdd(a.abort_count, 1);
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) tmem_dealloc<TM_COLS>(tmem);
+    cta_end<TM_COLS>(abortf, a.abort_count, tmem, tid);
 }
 
 // ==========================================================================================
 // backward
 // ==========================================================================================
-__global__ void __launch_bounds__(kThreadsChan) head_bwd_kernel(const HeadArgs a) {
+__global__ void __launch_bounds__(kCtaThreads) head_bwd_kernel(const HeadArgs a) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
     const HeadSmem m = head_smem(a.H, a.D, true);
@@ -275,8 +264,7 @@ __global__ void __launch_bounds__(kThreadsChan) head_bwd_kernel(const HeadArgs a
     const int prow = qtr * 32 + lane;
     const int T = a.T, To = a.To, H = a.H, D = a.D, S = a.S;
     constexpr int TM_COLS = 512;
-    if (tid == 0) { mbar_init(&bars[0], 1); mbar_init(&bars[1], 1); *abortf = 0; fence_mbar_init(); }
-    if (warp == 0) tmem_alloc<TM_COLS>(sm.tslot);
+    cta_begin<TM_COLS>(bars, 2, abortf, sm.tslot, tid);
     pdl_launch_dependents();
     head_prologue(a, wbd, wfb, sm, tid);
     pdl_wait();
@@ -320,16 +308,16 @@ __global__ void __launch_bounds__(kThreadsChan) head_bwd_kernel(const HeadArgs a
 #pragma unroll 1
         for (int c8 = half; c8 < KH / 8; c8 += kHalves) {
             float v[8], z[8], g[8], b[8];
-            chan::ld8<2>(srow, 8 * c8, vin ? H : 0, v);
-            chan::ld8s(sm.gam + 8 * c8, g);
-            chan::ld8s(sm.bet + 8 * c8, b);
+            ld8<2>(srow, 8 * c8, vin ? H : 0, v);
+            ld8s(sm.gam + 8 * c8, g);
+            ld8s(sm.bet + 8 * c8, b);
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
                 const bool ok = vin && 8 * c8 + j < H;
                 v[j] = ok ? (v[j] - mean) * rstd : 0.0f;
                 z[j] = ok ? fmaf(v[j], g[j], b[j]) : 0.0f;
             }
-            chan::put_chunk(bufX, HPLANE, PS, prow, c8, z);
+            put_chunk(bufX, PH::PLANE, PS, prow, c8, z);
             tmem_st8(tmem_addr(tXH, qtr, 8 * c8), v);
         }
         tmem_wait_st();
@@ -338,15 +326,15 @@ __global__ void __launch_bounds__(kThreadsChan) head_bwd_kernel(const HeadArgs a
         __syncthreads();           // operand X complete; the x tile (O region) is consumed
         if (tid == 0) {
             tc_fence_after();
-            chan::gemm3<0, 1>(tP, bdB, bdB + BDPLANE, PS, xB, xB + HPLANE, PS, KH, 128 / 16, false);
+            gemm3<0, 1>(tP, bdB, bdB + PB::PLANE, PS, xB, xB + PH::PLANE, PS, KH, 128 / 16, false);
             mma_commit(&bars[1]);
         }
         // ---------------- P1: dOut -> operand O
 #pragma unroll 1
         for (int c8 = half; c8 < KD / 8; c8 += kHalves) {
             float v[8];
-            chan::ld8<2>(drow, 8 * c8, vout ? D : 0, v);
-            chan::put_chunk(bufO, DPLANE, PS, prow, c8, v);
+            ld8<2>(drow, 8 * c8, vout ? D : 0, v);
+            put_chunk(bufO, PD::PLANE, PS, prow, c8, v);
         }
         __syncthreads();           // the dOut tile (Y region) is consumed
         // ---------------- E1: P + bt (+ ones column at H) -> operand Y
@@ -365,7 +353,7 @@ __global__ void __launch_bounds__(kThreadsChan) head_bwd_kernel(const HeadArgs a
                     const int c = 8 * c8 + j;
                     u[j] = !vout ? 0.0f : (c < H ? u[j] + bt : (c == H ? 1.0f : 0.0f));
                 }
-                chan::put_chunk(bufY, HPLANE, PS, prow, c8, u);
+                put_chunk(bufY, PH::PLANE, PS, prow, c8, u);
             }
         }
         fence_async_smem();
@@ -374,9 +362,9 @@ __global__ void __launch_bounds__(kThreadsChan) head_bwd_kernel(const HeadArgs a
         if (tid == 0) {
             tc_fence_after();
             // dP = dOut Wf                 (A = dOut K-major, B = Wf [D rows][H cols] read MN-major: K = d)
-            chan::gemm3<0, 1>(tDP, oB, oB + DPLANE, PS, wfB, wfB + chan::Plan<KD>::WPLANE, chan::Plan<KD>::WPS, KH, KD / 16, false);
+            gemm3<0, 1>(tDP, oB, oB + PD::PLANE, PS, wfB, wfB + PD::WPLANE, PD::WPS, KH, KD / 16, false);
             // dWf[d][h] += sum_r dOut[r][d] P[r][h]   (both MN-major, K = the 128 rows); column H of P is all ones -> dbf
-            chan::gemm3<1, 1>(tDWF, oB, oB + DPLANE, PS, yB, yB + HPLANE, PS, KH, 128 / 16, !first);
+            gemm3<1, 1>(tDWF, oB, oB + PD::PLANE, PS, yB, yB + PH::PLANE, PS, KH, 128 / 16, !first);
             mma_commit(&bars[1]);
         }
         // ---------------- E2: dP -> operand O (over dOut); its row sums -> dbt
@@ -393,7 +381,7 @@ __global__ void __launch_bounds__(kThreadsChan) head_bwd_kernel(const HeadArgs a
                 u[j] = (vout && 8 * c8 + j < H) ? u[j] : 0.0f;
                 dbt_acc += u[j];
             }
-            chan::put_chunk(bufO, DPLANE, PS, prow, c8, u);
+            put_chunk(bufO, PD::PLANE, PS, prow, c8, u);
         }
         fence_async_smem();
         tc_fence_before();
@@ -401,9 +389,9 @@ __global__ void __launch_bounds__(kThreadsChan) head_bwd_kernel(const HeadArgs a
         if (tid == 0) {
             tc_fence_after();
             // dZ[(s',t)][h] = sum_(s,o) Wbd[(s,o)][(s',t)] dP[(s,o)][h]     (A = Wbd read MN-major, B = dP read MN-major)
-            chan::gemm3<1, 1>(tP, bdB, bdB + BDPLANE, PS, oB, oB + DPLANE, PS, KH, 128 / 16, false);
+            gemm3<1, 1>(tP, bdB, bdB + PB::PLANE, PS, oB, oB + PD::PLANE, PS, KH, 128 / 16, false);
             // G[(s,o)][(s',t)] += sum_h dP[(s,o)][h] Z[(s',t)][h]           (both K-major)
-            chan::gemm3<0, 0>(tG, oB, oB + DPLANE, PS, xB, xB + HPLANE, PS, 128, KH / 16, !first);
+            gemm3<0, 0>(tG, oB, oB + PD::PLANE, PS, xB, xB + PH::PLANE, PS, 128, KH / 16, !first);
             mma_commit(&bars[1]);
         }
         first = false;
@@ -424,7 +412,7 @@ __global__ void __launch_bounds__(kThreadsChan) head_bwd_kernel(const HeadArgs a
                 float dz[8], g[8];
                 tmem_ld8(tmem_addr(tP, qtr, 8 * c8), dz);
                 tmem_ld8(tmem_addr(tXH, qtr, 8 * c8), xh[i]);
-                chan::ld8s(sm.gam + 8 * c8, g);
+                ld8s(sm.gam + 8 * c8, g);
                 tmem_wait_ld();
 #pragma unroll
                 for (int j = 0; j < 8; ++j) {
@@ -436,7 +424,7 @@ __global__ void __launch_bounds__(kThreadsChan) head_bwd_kernel(const HeadArgs a
                     m2 = fmaf(dxh[i][j], xh[i][j], m2);
                 }
             }
-            chan::row_exchange(sm.ex, half, prow, m1, m2);
+            row_exchange(sm.ex, half, prow, m1, m2);
             m1 /= (float)H;
             m2 /= (float)H;
             float* orow = reinterpret_cast<float*>(bufX) + (size_t)prow * H;
@@ -445,7 +433,7 @@ __global__ void __launch_bounds__(kThreadsChan) head_bwd_kernel(const HeadArgs a
                 const int c8 = half + kHalves * i;
 #pragma unroll
                 for (int j = 0; j < 8; ++j) dxh[i][j] = rstd * (dxh[i][j] - m1 - xh[i][j] * m2);
-                if (vin) chan::st8<2>(orow, 8 * c8, H, dxh[i]);
+                if (vin) st8<2>(orow, 8 * c8, H, dxh[i]);
             }
         }
         tc_fence_before();
@@ -497,12 +485,12 @@ __global__ void __launch_bounds__(kThreadsChan) head_bwd_kernel(const HeadArgs a
             for (int j = 0; j < 8; ++j) gst[prow * 128 + ((8 * c8 + j + prow) & 127)] = u[j];
         }
         __syncthreads();
-        for (int i = tid; i < D * H; i += kThreadsChan) {
+        for (int i = tid; i < D * H; i += kCtaThreads) {
             const int d = i / H, h = i - d * H;
             red_add(a.g_wf + i, stg[d * SP + h]);
         }
-        for (int d = tid; d < D; d += kThreadsChan) red_add(a.g_bf + d, stg[d * SP + H]);
-        for (int i = tid; i < To * T; i += kThreadsChan) {
+        for (int d = tid; d < D; d += kCtaThreads) red_add(a.g_bf + d, stg[d * SP + H]);
+        for (int i = tid; i < To * T; i += kCtaThreads) {
             const int o = i / T, t = i - o * T;
             float v = 0.0f;
             for (int s = 0; s < S; ++s) {
@@ -511,13 +499,10 @@ __global__ void __launch_bounds__(kThreadsChan) head_bwd_kernel(const HeadArgs a
             }
             red_add(a.g_wt + i, v);
         }
-        for (int o = tid; o < To; o += kThreadsChan) red_add(a.g_bt + o, sm.dbt[o]);
-        for (int h = tid; h < H; h += kThreadsChan) { red_add(a.g_ln_g + h, sm.dgam[h]); red_add(a.g_ln_b + h, sm.dbet[h]); }
+        for (int o = tid; o < To; o += kCtaThreads) red_add(a.g_bt + o, sm.dbt[o]);
+        for (int h = tid; h < H; h += kCtaThreads) { red_add(a.g_ln_g + h, sm.dgam[h]); red_add(a.g_ln_b + h, sm.dbet[h]); }
     }
-    if (tid == 0 && *abortf) atomicAdd(a.abort_count, 1);
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) tmem_dealloc<TM_COLS>(tmem);
+    cta_end<TM_COLS>(abortf, a.abort_count, tmem, tid);
 }
 
 }  // namespace head

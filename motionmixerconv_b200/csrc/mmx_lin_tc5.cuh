@@ -3,19 +3,17 @@
 //     y[r, :] = W x[r, :] + b          W: [N, K] (nn.Linear layout), rows r = 0 .. R-1
 //
 // Serves MlpMixer.conv (Conv2d(1,H,(1,D)) == per-frame Linear D -> H, h36m/mlp_mixer.py:268,325-327) and fc_out (Linear H -> D,
-// mlp_mixer.py:300,335) in the reduced-precision mode, with the machinery of mmx_chan_tc5.cuh: 128-row tiles, one thread per
+// mlp_mixer.py:300,335) in the reduced-precision mode, with the bf16x3 toolkit of mmx_tc5.cuh: 128-row tiles, one thread per
 // (row, chunk set), bf16 hi+lo split operands in the 16-bit panel layout (one copy, both orientations), three MMAs per
 // product, accumulators in TMEM.  Backward: dW = dY^T X (+ db from a ones column of X) accumulates in TMEM across the CTA's
 // persistent loop and is flushed once; dx = dY W (optional) uses the untransposed weight as an MN-major operand.
 #pragma once
-#include "mmx_chan_tc5.cuh"
+#include "mmx_tc5.cuh"
 
 namespace mmx {
 namespace lin {
 
 using namespace tc5;
-using chan::kHalves;
-using chan::kThreadsChan;
 
 struct LinArgs {
     const float* x;      // [R, K]
@@ -28,55 +26,59 @@ struct LinArgs {
     int* abort_count;
 };
 
-// KP: padded width of BOTH operand buffers (multiple of 16, > K so that column K can carry the ones of the bias gradient, >= N)
-template <int KP>
-struct LPlan {
-    static constexpr uint32_t PS = 128 * 16, PLANE = (KP / 8) * PS, BUF = 2 * PLANE;
-    static constexpr uint32_t WPS = KP * 16, WPLANE = (KP / 8) * WPS, WBUF = 2 * WPLANE;
+// shared-memory layout (byte offsets from the 1024-aligned base; total includes the alignment slack).  KP: padded width of
+// BOTH operand buffers (multiple of 16, > K so that column K can carry the ones of the bias gradient, >= N)
+struct LinSmem {
+    uint32_t x, y, w, sx, sy, bias, bars, total;
 };
 template <int KP>
-MMX_HD size_t lin_smem_bytes(int K, int N, bool bwd) {
-    const size_t sx = ((size_t)128 * K * 4 + 64 + 127) / 128 * 128, sy = ((size_t)128 * N * 4 + 64 + 127) / 128 * 128;
-    size_t bx = LPlan<KP>::BUF;
-    if (bx < sy) bx = sy;
-    if (bx < sx) bx = sx;
-    return 1024 + (bwd ? 2 : 1) * bx + LPlan<KP>::WBUF + sx + (bwd ? sy : 0) + (KP + 64) * 4;
+MMX_HD LinSmem lin_smem(int K, int N, bool bwd) {
+    using P = Panels<KP>;
+    const uint32_t sx = up128(128u * K * 4u + 64u), sy = up128(128u * N * 4u + 64u);
+    const uint32_t bx = umax(P::BUF, umax(sx, sy));               // X doubles as the staging tile of the output
+    LinSmem m;
+    uint32_t o = 0;
+    m.x = o; o += bx;
+    m.y = o; o += bwd ? bx : 0;                                     // backward: operand dY
+    m.w = o; o += P::WBUF;
+    m.sx = o; o += sx;                                              // x tile
+    m.sy = o; o += bwd ? sy : 0;                                    // backward: dy tile
+    m.bias = o; o += KP * 4;
+    m.bars = o; o += 64 * 4;                                        // barriers, TMEM slot, abort flag
+    m.total = o + 1024;
+    return m;
 }
 
 // ------------------------------------------------------------------------------------------ forward
 template <int KP, int VEC>
-__global__ void __launch_bounds__(kThreadsChan) lin_fwd_kernel(const LinArgs a) {
-    using P = LPlan<KP>;
+__global__ void __launch_bounds__(kCtaThreads) lin_fwd_kernel(const LinArgs a) {
+    using P = Panels<KP>;
     extern __shared__ uint8_t smem_raw[];
     uint8_t* sm = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
     const int K = a.K, N = a.N;
-    const uint32_t sx = ((uint32_t)128 * K * 4 + 64 + 127) / 128 * 128, sy = ((uint32_t)128 * N * 4 + 64 + 127) / 128 * 128;
-    uint32_t bx = P::BUF;
-    if (bx < sy) bx = sy;
-    if (bx < sx) bx = sx;
-    uint8_t* bufX = sm;                                       // operand X, later the output staging tile
-    uint8_t* wb = bufX + bx;
-    float* S = reinterpret_cast<float*>(wb + P::WBUF);
-    float* bias = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(S) + sx);
-    uint64_t* bars = reinterpret_cast<uint64_t*>(bias + KP);
+    const LinSmem m = lin_smem<KP>(K, N, false);
+    uint8_t* bufX = sm + m.x;                                 // operand X, later the output staging tile
+    uint8_t* wb = sm + m.w;
+    float* S = reinterpret_cast<float*>(sm + m.sx);
+    float* bias = reinterpret_cast<float*>(sm + m.bias);
+    uint64_t* bars = reinterpret_cast<uint64_t*>(sm + m.bars);
     uint32_t* tslot = reinterpret_cast<uint32_t*>(bars + 4);
     volatile int* abortf = reinterpret_cast<volatile int*>(tslot + 1);
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, qtr = warp & 3, half = warp >> 2;
     const int prow = qtr * 32 + lane;
     constexpr int TM_COLS = KP <= 64 ? 64 : 128;
     constexpr int NCH = KP / 8;
-    if (tid == 0) { mbar_init(&bars[0], 1); mbar_init(&bars[1], 1); *abortf = 0; fence_mbar_init(); }
-    if (warp == 0) tmem_alloc<TM_COLS>(tslot);
+    cta_begin<TM_COLS>(bars, 2, abortf, tslot, tid);
     pdl_launch_dependents();
-    for (int i = tid; i < (int)(P::WBUF / 16); i += kThreadsChan) reinterpret_cast<uint4*>(wb)[i] = make_uint4(0, 0, 0, 0);
-    for (int c = tid; c < KP; c += kThreadsChan) bias[c] = c < N ? a.b[c] : 0.0f;
+    for (int i = tid; i < (int)(P::WBUF / 16); i += kCtaThreads) reinterpret_cast<uint4*>(wb)[i] = make_uint4(0, 0, 0, 0);
+    for (int c = tid; c < KP; c += kCtaThreads) bias[c] = c < N ? a.b[c] : 0.0f;
     __syncthreads();
-    chan::stage_weight<KP>(wb, a.w, N, K, nullptr, tid);
+    stage_weight<KP>(wb, a.w, N, K, nullptr, tid);
     pdl_wait();
     const long long ntiles = (a.R + 127) / 128;
     auto tile_rows = [&](long long t) { return (int)min((long long)128, a.R - t * 128); };
     if (warp == 0 && (long long)blockIdx.x < ntiles)
-        chan::stage_in<VEC>(S, a.x, (size_t)blockIdx.x * 128, tile_rows(blockIdx.x), K, K, &bars[0], lane);
+        stage_in<VEC>(S, a.x, (size_t)blockIdx.x * 128, tile_rows(blockIdx.x), K, K, &bars[0], lane);
     fence_async_smem();
     tc_fence_before();
     __syncthreads();
@@ -96,19 +98,19 @@ __global__ void __launch_bounds__(kThreadsChan) lin_fwd_kernel(const LinArgs a) 
 #pragma unroll 1
         for (int c8 = half; c8 < NCH; c8 += kHalves) {
             float v[8];
-            chan::ld8<VEC>(srow, 8 * c8, (valid && c8 < nchK) ? K : 0, v);
-            chan::put_chunk(bufX, P::PLANE, P::PS, prow, c8, v);
+            ld8<VEC>(srow, 8 * c8, (valid && c8 < nchK) ? K : 0, v);
+            put_chunk(bufX, P::PLANE, P::PS, prow, c8, v);
         }
         fence_async_smem();
         tc_fence_before();
         __syncthreads();
         if (warp == 0) {
             const long long next = tile + gridDim.x;
-            if (next < ntiles) chan::stage_in<VEC>(S, a.x, (size_t)next * 128, tile_rows(next), K, K, &bars[0], lane);
+            if (next < ntiles) stage_in<VEC>(S, a.x, (size_t)next * 128, tile_rows(next), K, K, &bars[0], lane);
         }
         if (tid == 0) {
             tc_fence_after();
-            chan::gemm3<0, 0>(tmem, xB, xB + P::PLANE, P::PS, wB, wB + P::WPLANE, P::WPS, KP, KP / 16, false);
+            gemm3<0, 0>(tmem, xB, xB + P::PLANE, P::PS, wB, wB + P::WPLANE, P::WPS, KP, KP / 16, false);
             mma_commit(&bars[1]);
         }
         mbar_wait(&bars[1], ph_mma, abortf);
@@ -120,11 +122,11 @@ __global__ void __launch_bounds__(kThreadsChan) lin_fwd_kernel(const LinArgs a) 
             for (int c8 = half; c8 < nchN; c8 += kHalves) {
                 float u[8], b[8];
                 tmem_ld8(tmem_addr(tmem, qtr, 8 * c8), u);
-                chan::ld8s(bias + 8 * c8, b);
+                ld8s(bias + 8 * c8, b);
                 tmem_wait_ld();
 #pragma unroll
                 for (int j = 0; j < 8; ++j) u[j] += b[j];
-                if (valid) chan::st8<2>(orow, 8 * c8, N, u);
+                if (valid) st8<2>(orow, 8 * c8, N, u);
             }
         }
         tc_fence_before();
@@ -135,43 +137,35 @@ __global__ void __launch_bounds__(kThreadsChan) lin_fwd_kernel(const LinArgs a) 
             bulk_commit();
         }
     }
-    if (warp == 0) bulk_wait_all0();
-    if (tid == 0 && *abortf) atomicAdd(a.abort_count, 1);
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) tmem_dealloc<TM_COLS>(tmem);
+    cta_end<TM_COLS>(abortf, a.abort_count, tmem, tid);
 }
 
 // ------------------------------------------------------------------------------------------ backward
 template <int KP, int VEC>
-__global__ void __launch_bounds__(kThreadsChan) lin_bwd_kernel(const LinArgs a) {
-    using P = LPlan<KP>;
+__global__ void __launch_bounds__(kCtaThreads) lin_bwd_kernel(const LinArgs a) {
+    using P = Panels<KP>;
     extern __shared__ uint8_t smem_raw[];
     uint8_t* sm = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
     const int K = a.K, N = a.N;
     const bool want_dx = a.out != nullptr;
-    const uint32_t sx = ((uint32_t)128 * K * 4 + 64 + 127) / 128 * 128, sy = ((uint32_t)128 * N * 4 + 64 + 127) / 128 * 128;
-    uint32_t bx = P::BUF;
-    if (bx < sy) bx = sy;
-    if (bx < sx) bx = sx;
-    uint8_t* bufX = sm;                                       // operand X (+ ones column at K), later the dx staging tile
-    uint8_t* bufY = bufX + bx;                                // operand dY
-    uint8_t* wb = bufY + bx;
-    float* SX = reinterpret_cast<float*>(wb + P::WBUF);
-    float* SY = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(SX) + sx);
-    uint64_t* bars = reinterpret_cast<uint64_t*>(reinterpret_cast<uint8_t*>(SY) + sy);
+    const LinSmem m = lin_smem<KP>(K, N, true);
+    uint8_t* bufX = sm + m.x;                                 // operand X (+ ones column at K), later the dx staging tile
+    uint8_t* bufY = sm + m.y;                                 // operand dY
+    uint8_t* wb = sm + m.w;
+    float* SX = reinterpret_cast<float*>(sm + m.sx);
+    float* SY = reinterpret_cast<float*>(sm + m.sy);
+    uint64_t* bars = reinterpret_cast<uint64_t*>(sm + m.bars);
     uint32_t* tslot = reinterpret_cast<uint32_t*>(bars + 4);
     volatile int* abortf = reinterpret_cast<volatile int*>(tslot + 1);
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, qtr = warp & 3, half = warp >> 2;
     const int prow = qtr * 32 + lane;
     constexpr int TM_COLS = 2 * KP <= 128 ? 128 : 256;
     constexpr int NCH = KP / 8;
-    if (tid == 0) { mbar_init(&bars[0], 1); mbar_init(&bars[1], 1); *abortf = 0; fence_mbar_init(); }
-    if (warp == 0) tmem_alloc<TM_COLS>(tslot);
+    cta_begin<TM_COLS>(bars, 2, abortf, tslot, tid);
     pdl_launch_dependents();
-    for (int i = tid; i < (int)(P::WBUF / 16); i += kThreadsChan) reinterpret_cast<uint4*>(wb)[i] = make_uint4(0, 0, 0, 0);
+    for (int i = tid; i < (int)(P::WBUF / 16); i += kCtaThreads) reinterpret_cast<uint4*>(wb)[i] = make_uint4(0, 0, 0, 0);
     __syncthreads();
-    if (want_dx) chan::stage_weight<KP>(wb, a.w, N, K, nullptr, tid);
+    if (want_dx) stage_weight<KP>(wb, a.w, N, K, nullptr, tid);
     pdl_wait();
     const long long ntiles = (a.R + 127) / 128;
     auto tile_rows = [&](long long t) { return (int)min((long long)128, a.R - t * 128); };
@@ -207,13 +201,13 @@ __global__ void __launch_bounds__(kThreadsChan) lin_bwd_kernel(const LinArgs a) 
 #pragma unroll 1
         for (int c8 = half; c8 < NCH; c8 += kHalves) {
             float v[8];
-            chan::ld8<VEC>(xrow, 8 * c8, (valid && c8 < nchK) ? K : 0, v);
+            ld8<VEC>(xrow, 8 * c8, (valid && c8 < nchK) ? K : 0, v);
 #pragma unroll
             for (int j = 0; j < 8; ++j)
                 if (valid && 8 * c8 + j == K) v[j] = 1.0f;          // ones column: dW[:, K] = db
-            chan::put_chunk(bufX, P::PLANE, P::PS, prow, c8, v);
-            chan::ld8<2>(yrow, 8 * c8, (valid && c8 < nchN) ? N : 0, v);
-            chan::put_chunk(bufY, P::PLANE, P::PS, prow, c8, v);
+            put_chunk(bufX, P::PLANE, P::PS, prow, c8, v);
+            ld8<2>(yrow, 8 * c8, (valid && c8 < nchN) ? N : 0, v);
+            put_chunk(bufY, P::PLANE, P::PS, prow, c8, v);
         }
         fence_async_smem();
         tc_fence_before();
@@ -225,9 +219,9 @@ __global__ void __launch_bounds__(kThreadsChan) lin_bwd_kernel(const LinArgs a) 
         if (tid == 0) {
             tc_fence_after();
             // dW[n][k] += sum_r dY[r][n] X[r][k]   (both MN-major, K = the 128 rows)
-            chan::gemm3<1, 1>(tDW, yB, yB + P::PLANE, P::PS, xB, xB + P::PLANE, P::PS, KP, 128 / 16, !first);
+            gemm3<1, 1>(tDW, yB, yB + P::PLANE, P::PS, xB, xB + P::PLANE, P::PS, KP, 128 / 16, !first);
             // dx[r][k] = sum_n dY[r][n] W[n][k]    (A = dY K-major, B = W [N rows][K cols] read MN-major)
-            if (want_dx) chan::gemm3<0, 1>(tDX, yB, yB + P::PLANE, P::PS, wB, wB + P::WPLANE, P::WPS, KP, KP / 16, false);
+            if (want_dx) gemm3<0, 1>(tDX, yB, yB + P::PLANE, P::PS, wB, wB + P::WPLANE, P::WPS, KP, KP / 16, false);
             mma_commit(&bars[1]);
         }
         first = false;
@@ -241,7 +235,7 @@ __global__ void __launch_bounds__(kThreadsChan) lin_bwd_kernel(const LinArgs a) 
                 float u[8];
                 tmem_ld8(tmem_addr(tDX, qtr, 8 * c8), u);
                 tmem_wait_ld();
-                if (valid) chan::st8<VEC>(orow, 8 * c8, K, u);
+                if (valid) st8<VEC>(orow, 8 * c8, K, u);
             }
             tc_fence_before();
             fence_async_smem();
@@ -268,16 +262,13 @@ __global__ void __launch_bounds__(kThreadsChan) lin_bwd_kernel(const LinArgs a) 
                 for (int j = 0; j < 8; ++j) stg[prow * SP + 8 * c8 + j] = u[j];
         }
         __syncthreads();
-        for (int i = tid; i < N * K; i += kThreadsChan) {
+        for (int i = tid; i < N * K; i += kCtaThreads) {
             const int n = i / K, k = i - n * K;
             red_add(a.g_w + i, stg[n * SP + k]);
         }
-        for (int n = tid; n < N; n += kThreadsChan) red_add(a.g_b + n, stg[n * SP + K]);
+        for (int n = tid; n < N; n += kCtaThreads) red_add(a.g_b + n, stg[n * SP + K]);
     }
-    if (tid == 0 && *abortf) atomicAdd(a.abort_count, 1);
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) tmem_dealloc<TM_COLS>(tmem);
+    cta_end<TM_COLS>(abortf, a.abort_count, tmem, tid);
 }
 
 }  // namespace lin

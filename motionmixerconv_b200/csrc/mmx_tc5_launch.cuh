@@ -41,7 +41,7 @@ static int launch_tc5v(K kern, int grid, int block, size_t smem, void* stream, c
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = env_int("MMX_TC5_NO_PDL", 0) ? 0 : 1;
+    cfg.numAttrs = 1;
     cudaError_t e = cudaLaunchKernelEx(&cfg, kern, a...);
     if (e != cudaSuccess) return fail(MMX_E_CUDA, "kernel launch: %s", cudaGetErrorString(e));
     return MMX_OK;

@@ -15,11 +15,9 @@
 // ALL sequences) are computed from operands staged in shared memory by "owner" threads with register-resident 4x4 accumulator
 // tiles that persist across the CTA's loop over tiles (one flush per CTA).
 // Dropout: one keep-bit stream per column covers both sites of the token MLP (bits [0,tok): after the activation, bits
-// [tok, tok+T): after fc2) -- chan::keep8 with row = b*H + h, W8 = ceil((tok+T)/8), site = site_base.
+// [tok, tok+T): after fc2) -- tc5::keep8 with row = b*H + h, W8 = ceil((tok+T)/8), site = site_base.
 #pragma once
-#include "mmx_common.cuh"
 #include "mmx_tc5.cuh"
-#include "mmx_chan_tc5.cuh"   // keep8 / drop_key
 
 namespace mmx {
 namespace tok {
@@ -119,7 +117,7 @@ MMX_D unsigned long long column_keep(const Dropout& dr, uint32_t key, uint32_t c
     if (!dr.thresh) return ~0ull;
     const uint32_t n8 = (uint32_t)(tok + T + 7) >> 3;
     unsigned long long k = 0ull;
-    for (uint32_t c8 = 0; c8 < n8; ++c8) k |= (unsigned long long)chan::keep8(key, dr.thresh >> 16, colrow, n8, c8) << (8 * c8);
+    for (uint32_t c8 = 0; c8 < n8; ++c8) k |= (unsigned long long)keep8(key, dr.thresh >> 16, colrow, n8, c8) << (8 * c8);
     return k;
 }
 
@@ -215,7 +213,7 @@ __global__ void __launch_bounds__(kTokThreads) tok_fwd_kernel(const TokArgs a) {
     volatile int* abortf = reinterpret_cast<volatile int*>(sm + m.misc + 8);
     const int tid = threadIdx.x, T = a.T, H = a.H, S = a.S, rr = a.rr, tok = a.tok;
     const Dropout dr = resolve_dropout(a.dr);
-    const uint32_t key = chan::drop_key(dr.seed_lo, dr.seed_hi, a.site_base, dr.step);
+    const uint32_t key = drop_key(dr.seed_lo, dr.seed_hi, a.site_base, dr.step);
     if (tid == 0) { mbar_init(&bars[0], 1); *abortf = 0; fence_mbar_init(); }
     pdl_launch_dependents();
     load_params(sm, m, a, tid);        // parameters only: overlaps the previous kernel's tail
@@ -328,7 +326,7 @@ __global__ void __launch_bounds__(kTokThreads, 2) tok_bwd_kernel(const TokArgs a
     constexpr int NT = kTokThreads;
     const int tid = threadIdx.x, T = a.T, H = a.H, S = a.S, rr = a.rr, tok = a.tok;
     const Dropout dr = resolve_dropout(a.dr);
-    const uint32_t key = chan::drop_key(dr.seed_lo, dr.seed_hi, a.site_base, dr.step);
+    const uint32_t key = drop_key(dr.seed_lo, dr.seed_hi, a.site_base, dr.step);
     if (tid == 0) { mbar_init(&bars[0], 1); *abortf = 0; fence_mbar_init(); }
     pdl_launch_dependents();
     load_params(sm, m, a, tid);        // parameters only: overlaps the previous kernel's tail

@@ -6,7 +6,7 @@
 #include <cstdlib>
 #include <vector>
 
-#include "../../motionmixerconv_b200/csrc/mmx_tc5.cuh"
+#include "tc5_probe.cuh"
 using namespace mmx::tc5;
 
 constexpr int REGION_WORDS = 40 * 1024;   // 160 KB operand region under test

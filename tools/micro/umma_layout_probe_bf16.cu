@@ -7,24 +7,12 @@
 #include <vector>
 #include <cuda_bf16.h>
 
-#include "../../motionmixerconv_b200/csrc/mmx_tc5.cuh"
+#include "tc5_probe.cuh"
 using namespace mmx::tc5;
 
 constexpr int REGION_ELEMS = 64 * 1024;   // 128 KB operand region under test
 
 struct Cfg { int which; uint32_t lbo, sbo; };   // 0: A MN-major, 1: B MN-major, 2: A K-major (sanity)
-
-__device__ __forceinline__ uint32_t idesc_bf16(int M, int N, int a_mn, int b_mn) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)a_mn << 15) | ((uint32_t)b_mn << 16) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-__device__ __forceinline__ void mma_ss_f16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
 
 __global__ void __launch_bounds__(128) probe(Cfg cfg, int pass, float* out /*[128][16]*/, int* abort_out) {
     extern __shared__ __align__(1024) uint8_t smem[];
@@ -49,9 +37,9 @@ __global__ void __launch_bounds__(128) probe(Cfg cfg, int pass, float* out /*[12
     if (tid == 0) {
         const uint64_t d_x = smem_desc(smem_u32(region), cfg.lbo, cfg.sbo);
         const uint64_t d_oh = smem_desc(smem_u32(onehot), 128 * 16, 128);
-        if (cfg.which == 0) mma_ss_f16(tmem, d_x, d_oh, idesc_bf16(128, 16, 1, 0), 0);        // D[m][n] = A[m][k = n]
-        else if (cfg.which == 1) mma_ss_f16(tmem, d_oh, d_x, idesc_bf16(128, 16, 0, 1), 0);   // D[m][n] = B[n][k = m]   (m < 16)
-        else mma_ss_f16(tmem, d_x, d_oh, idesc_bf16(128, 16, 0, 0), 0);                      // sanity: A K-major
+        if (cfg.which == 0) mma_f16(tmem, d_x, d_oh, idesc_bf16(128, 16, 1, 0), 0);        // D[m][n] = A[m][k = n]
+        else if (cfg.which == 1) mma_f16(tmem, d_oh, d_x, idesc_bf16(128, 16, 0, 1), 0);   // D[m][n] = B[n][k = m]   (m < 16)
+        else mma_f16(tmem, d_x, d_oh, idesc_bf16(128, 16, 0, 0), 0);                      // sanity: A K-major
         mma_commit(&bars[0]);
     }
     mbar_wait(&bars[0], 0, abortf);

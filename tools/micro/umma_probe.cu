@@ -11,7 +11,7 @@
 #include <cstring>
 #include <vector>
 
-#include "../../motionmixerconv_b200/csrc/mmx_tc5.cuh"
+#include "tc5_probe.cuh"
 
 using namespace mmx::tc5;
 
