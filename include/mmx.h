@@ -234,6 +234,18 @@ int mmx_conv2d_large_fwd(const MmxConvHalfDesc* d, int data_gradient, const floa
                          void* stream);
 /* dw [C,C,kt,kp] += dz (*) n, db [C] += sum dz */
 int mmx_conv2d_large_wgrad(const MmxConvHalfDesc* d, const float* dz, const float* n, float* dw, float* db, void* stream);
+/* The same two convolutions with a precision mode.  MMX_PREC_TF32 runs them on the tensor cores (tcgen05, bf16 hi+lo split
+ * operands, three MMAs per product, fp32 accumulation in TMEM; csrc/mmx_conv_tc5.cuh) when mmx_conv2d_tc5_serves(d); MMX_PREC_FP32
+ * and every shape it does not serve give exactly the entry points above.  Served: 1 <= C <= 8, C * round_up(kp, 8) <= 256,
+ * kt * C <= 128, kp <= 121 and the tile (the padded input slab of one sequence and 128 embedding positions, (T-1)*C +
+ * round_up(kt*C, 16) rows) within shared memory -- at T = 10, E any, every kernel of the Optuna grid up to 9x29 at C = 8.
+ * Plain loads and stores: no alignment beyond that of float. */
+int mmx_conv2d_large_fwd_prec(const MmxConvHalfDesc* d, int data_gradient, const float* in, const float* w, const float* bias,
+                              float* out, int precision, void* stream);
+int mmx_conv2d_large_wgrad_prec(const MmxConvHalfDesc* d, const float* dz, const float* n, float* dw, float* db,
+                                int precision, void* stream);
+/* 1 when precision MMX_PREC_TF32 runs this descriptor's convolutions (fwd, data gradient, wgrad) on tcgen05; 0 otherwise.  No launch. */
+int mmx_conv2d_tc5_serves(const MmxConvHalfDesc* d);
 /* y = x + SE(reg(act(z))); reg = dropout of the descriptor, or (bn_aff != null) the BatchNorm affine [scale|shift][C] */
 int mmx_conv_tail_fwd(const MmxConvHalfDesc* d, const float* x, const float* z, const float* bn_aff, const float* se_w1, const float* se_w2,
                       float* y, void* stream);

@@ -104,6 +104,9 @@ SIGNATURES = {
     "mmx_conv_half_plan": (C.c_int, [C.POINTER(MmxConvHalfDesc), C.c_int, C.c_void_p, C.c_void_p]),
     "mmx_conv2d_large_fwd": (C.c_int, [C.POINTER(MmxConvHalfDesc), C.c_int] + [C.c_void_p] * 5),
     "mmx_conv2d_large_wgrad": (C.c_int, [C.POINTER(MmxConvHalfDesc)] + [C.c_void_p] * 5),
+    "mmx_conv2d_large_fwd_prec": (C.c_int, [C.POINTER(MmxConvHalfDesc), C.c_int] + [C.c_void_p] * 4 + [C.c_int, C.c_void_p]),
+    "mmx_conv2d_large_wgrad_prec": (C.c_int, [C.POINTER(MmxConvHalfDesc)] + [C.c_void_p] * 4 + [C.c_int, C.c_void_p]),
+    "mmx_conv2d_tc5_serves": (C.c_int, [C.POINTER(MmxConvHalfDesc)]),
     "mmx_conv_tail_fwd": (C.c_int, [C.POINTER(MmxConvHalfDesc)] + [C.c_void_p] * 7),
     "mmx_conv_tail_bwd1": (C.c_int, [C.POINTER(MmxConvHalfDesc)] + [C.c_void_p] * 10),
     "mmx_conv_tail_bwd2": (C.c_int, [C.POINTER(MmxConvHalfDesc)] + [C.c_void_p] * 7),

@@ -152,6 +152,7 @@ class ConvMixerBlock(nn.Module):
         self.activation = activation
         self.regularization = regularization
         self.block_index = 0      # set by ConvMixer; selects this block's dropout sites
+        self.precision = None     # None / "fp32" | "tf32"; set through ConvMixer.set_precision (not a reference argument)
         self._calls = 0
 
     # ---- kernel plumbing -----------------------------------------------------------------------
@@ -184,7 +185,19 @@ class ConvMixerBlock(nn.Module):
         cache = self.__dict__.setdefault("_fits", {})
         if key not in cache:
             cache[key] = F_.conv_half_fits(max(B, 1), self.conv_nChan, self.in_nTP, self.dimPosEmb, self.half_meta(half))
+        # Precision "tf32" leaves a half the fused fp32 kernels serve on them: chain + tcgen05 convolution measured slower at every
+        # such cell (B200, 1000 W, B = 256 training steps, profiles/r2h_conv_tc5.jsonl): Optuna 5x5 at C = 8 (200 taps C*kt*kp)
+        # 4.98 ms fused vs 5.10 ms chain (once), 8.10 vs 8.30 (twice); K3 (C = 4, 5x9 / 9x5, 180 taps) rollout training 22.8 vs
+        # 31.5 ms.  The halves that already take the chain gain 1.6x (5x9) to 3.2x (9x29) from it.
         return not cache[key]
+
+    def uses_tc5_conv(self, half, B):
+        """True when, in precision "tf32", this half's convolutions run on tcgen05 once the half takes the stage-kernel chain."""
+        key = (half, B > 0)
+        cache = self.__dict__.setdefault("_tc5", {})
+        if key not in cache:
+            cache[key] = F_.conv_tc5_serves(max(B, 1), self.conv_nChan, self.in_nTP, self.dimPosEmb, self.half_meta(half))
+        return self.precision == "tf32" and cache[key]
 
     def _half(self, x, half, seed, step):
         cb = self.conv1 if half == 0 else self.conv2
@@ -192,7 +205,7 @@ class ConvMixerBlock(nn.Module):
         if self.uses_large_path(half, x.shape[0]):
             # shapes the fused kernels do not hold in shared memory (most of the Optuna grid at C = 8, E = 192) and BatchNorm
             # with the max squeeze: the same arithmetic as a chain of stage kernels (functional.ConvHalfLarge)
-            return F_.conv_half_large(x, meta, params, cb.reg if self.regularization == -1.0 else None)
+            return F_.conv_half_large(x, meta, params, cb.reg if self.regularization == -1.0 else None, self.precision)
         if self.regularization == -1.0:
             if self.training:
                 return F_.conv_half_bn(x, meta, cb.reg, params)
@@ -248,6 +261,20 @@ class ConvMixer(nn.Module):
         self.project_channels = nn.Conv2d(self.conv_nChan, 1, kernel_size=(1, 1), stride=1)
         self.conv_out = nn.Conv2d(in_channels=self.in_nTP, out_channels=self.out_nTP, kernel_size=1, stride=1)
         self.fc_out = nn.Linear(self.dimPosEmb, self.dimPosOut)
+        self.precision = None         # fp32; set through set_precision()
+
+    def set_precision(self, precision):
+        """"fp32" / None (1e-5 parity, the default) | "tf32": the ConvBlock convolutions of the halves that run as the stage-kernel
+        chain use the tensor cores (tcgen05, bf16x3; 2e-3 parity) where mmx_conv2d_tc5_serves.  Halves the fused fp32 kernels
+        serve stay on them (faster, see ``ConvMixerBlock.uses_large_path``); the encoder and head stay fp32.  None does NOT follow
+        ``functional.set_precision`` / MMX_PRECISION: the ConvMixer opts in here only.  Not a reference argument and not part of
+        the state_dict.  Returns self."""
+        if precision is not None and precision not in F_.L.MMX_PREC:
+            raise ValueError("unknown precision %r" % (precision,))
+        self.precision = precision
+        for mb in self.Mixer_Block:
+            mb.precision = precision
+        return self
 
     def head_params(self):
         """Parameter tensors in the order of ``MmxConvHeadParams`` (include/mmx.h)."""

@@ -618,6 +618,18 @@ def bn_eval_affine(bn_module):
 
 
 # ---- large halves: shapes the fused kernels do not serve (mmx_conv_half_plan), BatchNorm with the max squeeze ----------------
+def conv_prec(precision):
+    """MMX_PREC_* of a ConvMixer convolution.  ``None`` is fp32: unlike the MlpMixer, the ConvMixer does not follow
+    ``set_precision`` / MMX_PRECISION (ConvMixer runs under those settings have always been fp32 and stay bit for bit); it opts
+    in through ``ConvMixer.set_precision("tf32")``."""
+    return L.MMX_PREC[precision or "fp32"]
+
+
+def conv_tc5_serves(B, C, T, E, meta):
+    """True when precision "tf32" runs this half's convolutions on tcgen05 (mmx_conv2d_tc5_serves)."""
+    return bool(L.load().mmx_conv2d_tc5_serves(C_.byref(conv_half_desc(B, C, T, E, *meta))))
+
+
 def conv_half_fits(B, C, T, E, meta):
     """True when the fused half kernels (forward and backward) serve this shape; else the stage-kernel chain below runs."""
     desc = conv_half_desc(B, C, T, E, *meta)
@@ -631,9 +643,10 @@ class ConvHalfLarge:
     Used by the autograd Function below (fresh buffers per call) and by TrainStep (static buffers inside the captured graph).
     ``params`` = ConvMixerBlock.half_params(half); ``bn``: the half's BatchNorm2d module or None."""
 
-    def __init__(self, B, C, T, E, device, need_backward=True, with_bn=False):
+    def __init__(self, B, C, T, E, device, need_backward=True, with_bn=False, precision=None):
         e = lambda *shape: torch.empty(*shape, dtype=torch.float32, device=device)
         self.B, self.C, self.T, self.E = B, C, T, E
+        self.prec = conv_prec(precision)
         self.n, self.stats, self.z = e(B, C, T, E), e(B * C * T, 2), e(B, C, T, E)
         self.bn = torch.zeros(4 * C, dtype=torch.float32, device=device) if with_bn else None
         self.sums = torch.zeros(2 * C, dtype=torch.float64, device=device) if with_bn else None
@@ -647,7 +660,7 @@ class ConvHalfLarge:
         B, Cn, T, E = self.B, self.C, self.T, self.E
         st = _stream()
         _call("mmx_ln_fwd", B * Cn * T, E, 0, _p(x), _p(ln_w), _p(ln_b), _p(self.n), _p(self.stats), st)
-        _call("mmx_conv2d_large_fwd", C_.byref(desc), 0, _p(self.n), _p(cw), _p(cb), _p(self.z), st)
+        _call("mmx_conv2d_large_fwd_prec", C_.byref(desc), 0, _p(self.n), _p(cw), _p(cb), _p(self.z), self.prec, st)
         aff = None
         self.trained = bool(desc.training)
         if bnm is not None:
@@ -680,8 +693,8 @@ class ConvHalfLarge:
                 self.coef[Cn:3 * Cn].zero_()
             coef = self.coef
         _call("mmx_conv_tail_bwd2", C_.byref(desc), _p(self.z), _p(dy), _p(self.gd), _p(bn), _p(coef), _p(self.dz), st)
-        _call("mmx_conv2d_large_wgrad", C_.byref(desc), _p(self.dz), _p(self.n), _p(g_cw), _p(g_cb), st)
-        _call("mmx_conv2d_large_fwd", C_.byref(desc), 1, _p(self.dz), _p(cw), None, _p(self.dn), st)
+        _call("mmx_conv2d_large_wgrad_prec", C_.byref(desc), _p(self.dz), _p(self.n), _p(g_cw), _p(g_cb), self.prec, st)
+        _call("mmx_conv2d_large_fwd_prec", C_.byref(desc), 1, _p(self.dz), _p(cw), None, _p(self.dn), self.prec, st)
         _call("mmx_ln_bwd", B * Cn * T, E, 0, _p(x), _p(self.stats), _p(ln_w), _p(self.dn), _p(dy), _p(dx), _p(g_ln_w), _p(g_ln_b), st)
         return dx
 
@@ -692,14 +705,14 @@ class ConvHalfLarge:
 
 class _ConvHalfLarge(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, x, meta, bnm, *tensors):
+    def forward(ctx, x, meta, bnm, precision, *tensors):
         x = _chk(x, "x")
         params = [None if q is None else _chk(q, "parameter") for q in tensors[:6]]
         B, C, T, E = x.shape
         desc = conv_half_desc(B, C, T, E, *meta)
         needs_grad = any(ctx.needs_input_grad)
         with torch.cuda.device_of(x):
-            run = ConvHalfLarge(B, C, T, E, x.device, need_backward=needs_grad, with_bn=bnm is not None)
+            run = ConvHalfLarge(B, C, T, E, x.device, need_backward=needs_grad, with_bn=bnm is not None, precision=precision)
             y = torch.empty_like(x)
             run.forward(desc, x, y, params, bnm)
         ctx.run, ctx.params, ctx.x, ctx.meta, ctx.has_bn = run, params, x, meta, bnm is not None
@@ -719,13 +732,14 @@ class _ConvHalfLarge(torch.autograd.Function):
         with torch.cuda.device_of(x):
             run.backward(desc, x, dy, dx, params, grads, bn_grads)
         ctx.run = None
-        return (dx, None, None, *grads, *(bn_grads or []))
+        return (dx, None, None, None, *grads, *(bn_grads or []))
 
 
-def conv_half_large(x, meta, params, bn_module=None):
-    """One ConvMixerBlock half through the stage-kernel chain (large shapes; BatchNorm with max squeeze)."""
+def conv_half_large(x, meta, params, bn_module=None, precision=None):
+    """One ConvMixerBlock half through the stage-kernel chain (large shapes; BatchNorm with max squeeze).  ``precision``: see
+    ``conv_prec``."""
     extra = [bn_module.weight, bn_module.bias] if bn_module is not None else []
-    return _ConvHalfLarge.apply(x, meta, bn_module, *params, *extra)
+    return _ConvHalfLarge.apply(x, meta, bn_module, precision, *params, *extra)
 
 
 class _SeTail(torch.autograd.Function):

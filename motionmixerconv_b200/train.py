@@ -200,7 +200,7 @@ class _ConvMixerPlan:
                 if mb.uses_large_path(half, B):
                     reg = (mb.conv1 if half == 0 else mb.conv2).reg if mb.regularization == -1.0 else None
                     self.large[len(self.ops)] = dict(
-                        run=F_.ConvHalfLarge(B, C, T, E, dev, with_bn=reg is not None), params=hp, grads=[flat.grad_of(q) for q in hp],
+                        run=F_.ConvHalfLarge(B, C, T, E, dev, with_bn=reg is not None, precision=mb.precision), params=hp, grads=[flat.grad_of(q) for q in hp],
                         reg=reg, bn_grads=None if reg is None else [flat.grad_of(reg.weight), flat.grad_of(reg.bias)])
                 elif mb.regularization == -1.0:
                     reg = (mb.conv1 if half == 0 else mb.conv2).reg
