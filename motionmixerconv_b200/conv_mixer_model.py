@@ -27,6 +27,7 @@ class PoseEncoder(nn.Module):
         super().__init__()
         self.n_harmonic_functions = n_harmonic_functions
         self.conv_nChan = conv_nChan
+        self.in_nTP, self.dimPosIn = in_nTP, dimPosIn
         if n_harmonic_functions <= 0:
             dimHarmonic = dimPosIn
         else:
@@ -35,11 +36,12 @@ class PoseEncoder(nn.Module):
         self.embed_mlp = nn.Linear(dimHarmonic, dimPosEmb)
         self.channelUpscaling = nn.Linear(1, conv_nChan)
 
+    def runners(self, B, device, need_backward, dropout=None):
+        return [F_.Encoder(self, B, device, need_backward)]
+
     def forward(self, x):
         """x: [bs, in_nTP, dimPosIn] -> [bs, conv_nChan, in_nTP, dimPosEmb]"""
-        hn = max(int(self.n_harmonic_functions), 0)
-        return F_.pose_encoder(x, hn, self.conv_nChan, self.frequencies if hn > 0 else None, self.embed_mlp.weight,
-                               self.embed_mlp.bias, self.channelUpscaling.weight, self.channelUpscaling.bias)
+        return F_.forward_layers(self, x)
 
 
 class MultiChanSELayer(nn.Module):
@@ -105,7 +107,8 @@ class ConvBlock(nn.Module):
 
 
 class ConvMixerBlock(nn.Module):
-    """conv_mixer_model.py:145-292: one fused kernel per half (LN -> conv -> act -> reg -> SE -> +res)."""
+    """conv_mixer_model.py:145-292: one fused kernel per half (LN -> conv -> act -> reg -> SE -> +res, functional.ConvHalf), or
+    a chain of stage kernels where the fused kernels do not serve the half (functional.ConvHalfLarge)."""
 
     def __init__(self, dimPosEmb: int, in_nTP: int, conv_nChan: int, conv1_kernel_shape: Tuple[int, int] = (1, 3),
                  conv1_stride=None, conv1_padding=None, mode_conv: str = "twice", conv2_kernel_shape=None,
@@ -199,31 +202,19 @@ class ConvMixerBlock(nn.Module):
             cache[key] = F_.conv_tc5_serves(max(B, 1), self.conv_nChan, self.in_nTP, self.dimPosEmb, self.half_meta(half))
         return self.precision == "tf32" and cache[key]
 
-    def _half(self, x, half, seed, step):
-        cb = self.conv1 if half == 0 else self.conv2
-        meta, params = self.half_meta(half, seed, step), self.half_params(half)
-        if self.uses_large_path(half, x.shape[0]):
-            # shapes the fused kernels do not hold in shared memory (most of the Optuna grid at C = 8, E = 192) and BatchNorm
-            # with the max squeeze: the same arithmetic as a chain of stage kernels (functional.ConvHalfLarge)
-            return F_.conv_half_large(x, meta, params, cb.reg if self.regularization == -1.0 else None, self.precision)
-        if self.regularization == -1.0:
-            if self.training:
-                return F_.conv_half_bn(x, meta, cb.reg, params)
-            return F_.conv_half(x, meta, params, bn_aff=F_.bn_eval_affine(cb.reg))
-        return F_.conv_half(x, meta, params)
+    def runners(self, B, device, need_backward, dropout=None):
+        """This block's kernel runners: one per half, then the SE tail in mode_conv="once" (LN2 / conv2 are Identity there but
+        self.se is still applied, conv_mixer_model.py:287-292).  A half runs as the stage-kernel chain where
+        ``uses_large_path``, else as the fused kernels.  ``dropout``: (seed, step, step_dev) of a static plan; None draws this
+        call's own masks (both halves share them)."""
+        dropout = dropout or F_.dropout_source(self)
+        for half in ((0, 1) if self.mode_conv == "twice" else (0,)):
+            yield (F_.ConvHalfLarge if self.uses_large_path(half, B) else F_.ConvHalf)(self, half, B, device, need_backward, dropout)
+        if self.mode_conv != "twice":
+            yield F_.SeTail(self, B, device, need_backward)
 
     def forward(self, x: torch.Tensor):
-        seed = step = 0
-        if self.training and self.regularization > 0.0:
-            seed = torch.initial_seed() & 0xFFFFFFFFFFFFFFFF
-            step = self._calls
-            self._calls = (self._calls + 1) & 0xFFFFFFFF
-        x = self._half(x, 0, seed, step)
-        if self.mode_conv == "twice":
-            return self._half(x, 1, seed, step)
-        # mode_conv="once": LN2 / conv2 are Identity but self.se is still applied (conv_mixer_model.py:287-292)
-        s1, s2 = self.se_weights()
-        return F_.se_tail(x, self.in_nTP // self.r_se if self.use_se else 0, self.use_se, self.use_max_pooling, s1, s2)
+        return F_.forward_layers(self, x)
 
 
 class ConvMixer(nn.Module):
@@ -281,11 +272,16 @@ class ConvMixer(nn.Module):
         return [self.LN.weight, self.LN.bias, self.conv_out.weight, self.conv_out.bias, self.project_channels.weight,
                 self.project_channels.bias, self.fc_out.weight, self.fc_out.bias]
 
+    def runners(self, B, device, need_backward, dropout=None):
+        """The kernel runners of one forward pass in order: encoder, blocks, head (see ``ConvMixerBlock.runners``).  Yielded
+        one at a time, so that ``model(x)`` builds each layer's runner just before the layer runs."""
+        yield F_.Encoder(self.encoder, B, device, need_backward)
+        for mb in self.Mixer_Block:
+            yield from mb.runners(B, device, need_backward, dropout)
+        yield F_.ConvHead(self, B, device, need_backward)
+
     def forward(self, x: torch.Tensor):
         """x: [batch_size, in_nTP, dimPosIn] -> [batch_size, out_nTP, dimPosOut]  (conv_mixer_model.py:428-465)."""
         if x.dim() != 3 or x.shape[1] != self.in_nTP or x.shape[2] != self.dimPosIn:
             raise RuntimeError("ConvMixer.forward: expected [B, %d, %d], got %s" % (self.in_nTP, self.dimPosIn, tuple(x.shape)))
-        y = self.encoder(x)
-        for mb in self.Mixer_Block:
-            y = mb(y)
-        return F_.conv_head(y, *self.head_params())
+        return F_.forward_layers(self, x)

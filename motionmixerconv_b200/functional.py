@@ -1,15 +1,20 @@
-"""torch.autograd.Function wrappers over the libmmx C ABI (include/mmx.h).
+"""Host-side runners over the libmmx C ABI (include/mmx.h), and the autograd Function that applies them.
 
-Every op here launches hand-written sm_100a kernels on ``torch.cuda.current_stream()``; inputs must
-be CUDA fp32 tensors.  There is no CPU / eager-PyTorch implementation: non-CUDA input raises.
-Backward runs on PyTorch's autograd worker thread — the C ABI holds no thread-local CUDA state and
-takes the stream explicitly, and we re-enter the tensor's device before every call.
+A runner is one layer's kernel sequence: the embedding, a MixerBlock, a ConvMixerBlock half, the SE tail, an encoder or a
+head.  It is built once from the module, the batch size, the device and whether a backward follows; it makes its routing
+decision (which kernels, which saved intermediates) in its constructor and owns those intermediates.  ``forward(x, y,
+training)`` and ``backward(x, dy, dx, grads)`` launch its kernels; ``launches`` counts them (forward, backward).  The same
+runners serve both host paths: ``model(x)`` builds fresh ones per call and applies each through ``_Layer`` (autograd), and
+``train.TrainStep`` builds them once per batch size over static buffers and the flat gradient bucket.
+
+Every op launches hand-written sm_100a kernels on ``torch.cuda.current_stream()``; inputs must be CUDA fp32 tensors.  There
+is no CPU / eager-PyTorch implementation: non-CUDA input raises.  Backward runs on PyTorch's autograd worker thread — the C
+ABI holds no thread-local CUDA state and takes the stream explicitly, and we re-enter the tensor's device before every call.
 """
 from __future__ import annotations
 
 import ctypes as C
 import os
-import ctypes as C_   # (the conv wrappers use C for the channel count)
 
 import torch
 
@@ -35,7 +40,9 @@ def _p(t):
 def _zeros_like_many(tensors):
     """One memset for all gradient buffers: a flat zero buffer sliced into views (16-byte aligned)."""
     sizes = [0 if t is None else (t.numel() + 3) // 4 * 4 for t in tensors]
-    ref = next(t for t in tensors if t is not None)
+    ref = next((t for t in tensors if t is not None), None)
+    if ref is None:
+        return list(tensors)
     flat = torch.zeros(sum(sizes), dtype=torch.float32, device=ref.device)
     out, o = [], 0
     for t, n in zip(tensors, sizes):
@@ -47,6 +54,10 @@ def _zeros_like_many(tensors):
 def _call(name, *args):
     lib = L.load()
     L.check(lib, getattr(lib, name)(*args), name)
+
+
+def _empty(device):
+    return lambda *shape: torch.empty(*shape, dtype=torch.float32, device=device)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -86,19 +97,8 @@ def linear(x, weight, bias, precision=None):
 
 
 # ------------------------------------------------------------------------------------------------
-# MixerBlock (mlp_mixer.py:138-164)
+# precision, dropout, and one layer through autograd
 # ------------------------------------------------------------------------------------------------
-_BLOCK_FIELDS = ("ln1_w", "ln1_b", "tok_w1", "tok_b1", "tok_w2", "tok_b2", "ln2_w", "ln2_b",
-                 "ch_w1", "ch_b1", "ch_w2", "ch_b2", "se_w1", "se_w2")
-
-
-def mlp_block_table(tensors):
-    t = L.MmxMlpBlockParams()
-    for f, v in zip(_BLOCK_FIELDS, tensors):
-        setattr(t, f, _p(v))
-    return t
-
-
 _PRECISION = os.environ.get("MMX_PRECISION", "fp32")
 
 
@@ -133,6 +133,109 @@ def _step_dev_ptr(step_dev):
     return None if _STEP_DEV is None else _p(_STEP_DEV)
 
 
+def dropout_source(block):
+    """(seed, step, step_dev) of one autograd call of a Mixer / ConvMixer block: the masks follow ``torch.initial_seed()`` and
+    the block's call count, which advances once per training call with dropout; step_dev None reads ``set_dropout_step_tensor``."""
+    if not (block.training and block.regularization > 0.0):
+        return 0, 0, None
+    step = block._calls
+    block._calls = (block._calls + 1) & 0xFFFFFFFF
+    return torch.initial_seed() & 0xFFFFFFFFFFFFFFFF, step, None
+
+
+class _Layer(torch.autograd.Function):
+    """One runner as one autograd node.  The input and the parameters are saved through ``save_for_backward`` (so autograd's
+    in-place-modification check covers them); the runner holds its own intermediates until the backward."""
+
+    @staticmethod
+    def forward(ctx, run, training, x, *params):
+        x = _chk(x, "x")
+        for q in params:
+            if q is not None:
+                _chk(q, "parameter")
+        y = torch.empty(run.out_shape, dtype=torch.float32, device=x.device)
+        with torch.cuda.device_of(x):
+            run.forward(x, y, training)
+        ctx.run = run
+        ctx.save_for_backward(x, *params)
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        x, *params = ctx.saved_tensors
+        dy = _chk(dy, "grad")
+        grads = _zeros_like_many(params)
+        dx = torch.empty_like(x) if ctx.needs_input_grad[2] or not ctx.run.optional_dx else None
+        with torch.cuda.device_of(x):
+            ctx.run.backward(x, dy, dx, grads)
+        ctx.run = None
+        return (None, None, dx, *grads)
+
+
+def forward_layers(module, x):
+    """``module(x)`` through autograd: the module's runners, built fresh for this call, one autograd node each."""
+    need_backward = torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in module.parameters()))
+    for run in module.runners(x.shape[0], x.device, need_backward):
+        x = _Layer.apply(run, module.training, x, *run.params)
+    return x
+
+
+class _Runner:
+    optional_dx = False     # True: the first layer, whose input gradient is computed only when asked for
+    launches = (1, 1)
+
+
+def bn_vectors(bnm, training, sums, count, out):
+    """Per-channel vectors [scale | shift | xs | xo] (4C floats) of the BatchNorm module ``bnm`` into ``out``.  Training: from
+    the batch sums ``sums`` (float64 [2C], zero on entry and again on exit) over ``count`` elements per channel, by
+    mmx_bn_finalize, which also updates the running statistics as nn.BatchNorm does (biased variance to normalise, unbiased
+    for the running estimate, momentum, num_batches_tracked).  Eval: from the running statistics; the first 2C floats are then
+    the constant affine [scale | shift] that the fused ConvMixer kernels apply."""
+    if training:
+        _call("mmx_bn_finalize", _p(sums), out.numel() // 4, float(count), _p(bnm.weight), _p(bnm.bias), _p(bnm.running_mean),
+              _p(bnm.running_var), _p(bnm.num_batches_tracked), float(bnm.momentum if bnm.momentum is not None else 0.1),
+              float(bnm.eps), _p(out), _stream())
+    else:
+        with torch.no_grad():
+            xs = torch.rsqrt(bnm.running_var + bnm.eps)
+            scale = bnm.weight.detach() * xs
+            out.copy_(torch.cat([scale, bnm.bias.detach() - bnm.running_mean * scale, xs, -bnm.running_mean * xs]))
+    return out
+
+
+# ------------------------------------------------------------------------------------------------
+# MlpMixer: embedding, MixerBlock (mlp_mixer.py:138-164), head
+# ------------------------------------------------------------------------------------------------
+class LinearEmbed(_Runner):
+    """MlpMixer.conv: Conv2d(1, H, (1, D)) is a per-frame Linear D -> H (mlp_mixer.py:325-327)."""
+    optional_dx = True
+
+    def __init__(self, model, B, device, need_backward):
+        self.model = model
+        self.params = [model.conv.weight, model.conv.bias]
+        self.dims = (B * model.seq_len, model.input_size, model.hidden_dim)
+        self.in_shape, self.out_shape = (B, model.seq_len, model.input_size), (B, model.seq_len, model.hidden_dim)
+
+    def forward(self, x, y, training):
+        w, b = self.params
+        self.prec = L.MMX_PREC[self.model.precision or _PRECISION]
+        _call("mmx_linear_fwd_prec", *self.dims, _p(x), _p(w), _p(b), _p(y), self.prec, _stream())
+
+    def backward(self, x, dy, dx, grads):
+        _call("mmx_linear_bwd_prec", *self.dims, _p(x), _p(self.params[0]), _p(dy), _p(grads[0]), _p(grads[1]), _p(dx), self.prec, _stream())
+
+
+_BLOCK_FIELDS = ("ln1_w", "ln1_b", "tok_w1", "tok_b1", "tok_w2", "tok_b2", "ln2_w", "ln2_b",
+                 "ch_w1", "ch_b1", "ch_w2", "ch_b2", "se_w1", "se_w2")
+
+
+def mlp_block_table(tensors):
+    t = L.MmxMlpBlockParams()
+    for f, v in zip(_BLOCK_FIELDS, tensors):
+        setattr(t, f, _p(v))
+    return t
+
+
 def mlp_block_desc(B, T, H, tok, ch, se_hidden, act, use_se, use_max, training, block_index, p, seed, step, precision=None,
                    step_dev=None):
     return L.MmxMlpBlockDesc(B, T, H, tok, ch, se_hidden, L.MMX_ACT[act], int(use_se), int(use_max), int(training),
@@ -140,77 +243,69 @@ def mlp_block_desc(B, T, H, tok, ch, se_hidden, act, use_se, use_max, training, 
                              L.MMX_PREC[precision or _PRECISION])
 
 
-class _MlpBlock(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, x, meta, *params):
-        x = _chk(x, "x")
-        params = [None if q is None else _chk(q, "parameter") for q in params]
-        B, T, H = x.shape
-        desc = mlp_block_desc(B, T, H, *meta)
-        y = torch.empty_like(x)
-        needs_grad = any(ctx.needs_input_grad)
-        # the tcgen05 kernel family can hand the token-half output (+ SE gates) to the backward: one extra saved tile per
-        # block instead of re-running the token half forward
-        ctx.saved_x1 = bool(needs_grad and L.load().mmx_mlp_block_saves(C.byref(desc)))
-        with torch.cuda.device_of(x):
-            if ctx.saved_x1:
-                x1 = torch.empty_like(x)
-                gate = torch.empty(B, T, dtype=x.dtype, device=x.device)
-                _call("mmx_mlp_block_fwd_save", C.byref(desc), C.byref(mlp_block_table(params)), _p(x), _p(y), _p(x1), _p(gate), _stream())
-                ctx.save_for_backward(x, x1, gate, *[q for q in params if q is not None])
-            else:
-                _call("mmx_mlp_block_fwd", C.byref(desc), C.byref(mlp_block_table(params)), _p(x), _p(y), _stream())
-                ctx.save_for_backward(x, *[q for q in params if q is not None])
-        ctx.has = [q is not None for q in params]
-        ctx.meta = meta
-        return y
+class FusedMixerBlock(_Runner):
+    """One MixerBlock as one fused kernel per direction.  The tcgen05 family runs each direction as two kernels (token half,
+    channel half) and, when a training backward follows, can hand the token-half output x1 (+ SE gates) to it: one extra saved
+    tile per block instead of re-running the token half forward (the save variant, ``saves``).
 
-    @staticmethod
-    def backward(ctx, dy):
-        x, *rest = ctx.saved_tensors
-        x1 = gate = None
-        if ctx.saved_x1:
-            x1, gate, *rest = rest
-        it = iter(rest)
-        params = [next(it) if h else None for h in ctx.has]
-        dy = _chk(dy, "grad")
-        B, T, H = x.shape
-        desc = mlp_block_desc(B, T, H, *ctx.meta)
-        grads = _zeros_like_many(params)
-        dx = torch.empty_like(x)
-        with torch.cuda.device_of(x):
-            if ctx.saved_x1:
-                _call("mmx_mlp_block_bwd_saved", C.byref(desc), C.byref(mlp_block_table(params)), C.byref(mlp_block_table(grads)),
-                      _p(x), _p(x1), _p(gate), _p(dy), _p(dx), _stream())
-            else:
-                _call("mmx_mlp_block_bwd", C.byref(desc), C.byref(mlp_block_table(params)), C.byref(mlp_block_table(grads)),
-                      _p(x), _p(dy), _p(dx), _stream())
-        return (dx, None, *grads)
+    ``dropout``: (seed, step, step_dev) of the masks, see ``dropout_source``."""
+
+    def __init__(self, mb, B, device, need_backward, dropout):
+        self.mb, self.B = mb, B
+        self.seed, self.step, self.step_dev = dropout
+        self.params = mb.kernel_params()
+        self.w = mlp_block_table(self.params)
+        self.out_shape = (B, mb.seq_len, mb.hidden_dim)
+        self.saves = bool(need_backward and L.load().mmx_mlp_block_saves(C.byref(self._desc(True))))
+        self.x1 = torch.empty(self.out_shape, device=device) if self.saves else None
+        self.gate = torch.empty(B, mb.seq_len, device=device) if self.saves else None
+        self.launches = (2, 2) if self.saves else (1, 1)
+
+    def _desc(self, training):
+        m = self.mb.meta(self.seed, self.step)
+        return mlp_block_desc(self.B, self.mb.seq_len, self.mb.hidden_dim, *m[:6], training, *m[7:],
+                              step_dev=self.step_dev if training else None)
+
+    def forward(self, x, y, training):
+        self.trained = training
+        d = self._desc(training)
+        if self.saves and training:
+            _call("mmx_mlp_block_fwd_save", C.byref(d), C.byref(self.w), _p(x), _p(y), _p(self.x1), _p(self.gate), _stream())
+        else:
+            _call("mmx_mlp_block_fwd", C.byref(d), C.byref(self.w), _p(x), _p(y), _stream())
+
+    def backward(self, x, dy, dx, grads):
+        d, g = self._desc(self.trained), mlp_block_table(grads)
+        if self.saves and self.trained:
+            _call("mmx_mlp_block_bwd_saved", C.byref(d), C.byref(self.w), C.byref(g), _p(x), _p(self.x1), _p(self.gate), _p(dy), _p(dx),
+                  _stream())
+        else:
+            _call("mmx_mlp_block_bwd", C.byref(d), C.byref(self.w), C.byref(g), _p(x), _p(dy), _p(dx), _stream())
 
 
-def mlp_block(x, meta, params):
-    """meta = (tok, ch, se_hidden, act, use_se, use_max, training, block_index, p, seed, step, precision)."""
-    return _MlpBlock.apply(x, meta, *params)
-
-
-# ------------------------------------------------------------------------------------------------
-# MixerBlock with BatchNorm1d inside the MLP blocks (regularization == -1, mlp_mixer.py:72-73, 88-94)
-# ------------------------------------------------------------------------------------------------
-class MlpBnBlock:
-    """Static buffers + the stage-kernel sequence of one MixerBlock whose MlpBlocks regularise with BatchNorm1d.
+class MlpBnBlock(_Runner):
+    """The stage-kernel sequence of one MixerBlock whose MlpBlocks regularise with BatchNorm1d (regularization == -1,
+    mlp_mixer.py:72-73, 88-94).
 
     Batch statistics are global over the batch, so the block is a chain of stage kernels (include/mmx.h, csrc/mmx_api_bnmlp.cu)
-    with a reduction between them; this class owns the saved tensors and is used both by the autograd Function below (fresh
-    buffers per call) and by TrainStep (static buffers inside the captured graph).  Token MLP: BatchNorm1d(hidden_dim) on
-    [B,H,*]; channel MLP: BatchNorm1d(seq_len) on [B,T,*]; reg1 after the activation, reg2 after fc2 (mlp_mixer.py:88-94).
+    with a reduction between them.  Token MLP: BatchNorm1d(hidden_dim) on [B,H,*]; channel MLP: BatchNorm1d(seq_len) on [B,T,*];
+    reg1 after the activation, reg2 after fc2.  ``params``: MixerBlock.kernel_params() (14, SE weights may be None), then weight
+    and bias of the four BatchNorm1d modules in execution order (token reg1, token reg2, channel reg1, channel reg2); their
+    running statistics are updated in training mode exactly as nn.BatchNorm1d does."""
+    saves = False
+    launches = (16, 22)      # training: 2 LN + 4 fc + 4 x (stats, finalize) + 2 apply + 2 SE | 2 SE + 4 x (reduce, coef, apply) + 4 fc + 2 LN
 
-    ``params`` = MixerBlock.kernel_params() (14, SE weights may be None); ``bns`` = the four BatchNorm1d modules in execution
-    order (token reg1, token reg2, channel reg1, channel reg2).
-    """
-
-    def __init__(self, B, T, H, tok, ch, device, need_backward=True):
-        e = lambda *shape: torch.empty(*shape, dtype=torch.float32, device=device)
+    def __init__(self, mb, B, device, need_backward, dropout=None):
+        e = _empty(device)
+        T, H, tok, ch = mb.seq_len, mb.hidden_dim, mb.tokens_mlp_dim, mb.channels_mlp_dim
+        self.mb = mb
         self.B, self.T, self.H, self.tok, self.ch = B, T, H, tok, ch
+        self.bns = mb.bn_modules()
+        self.params = mb.kernel_params() + [t for m in self.bns for t in (m.weight, m.bias)]
+        self.act = L.MMX_ACT[mb.activation]
+        self.se_hidden = mb.seq_len // mb.r_se if mb.use_se else 0
+        self.use_max = int(mb.use_max_pooling)
+        self.out_shape = (B, T, H)
         self.nT, self.st1 = e(B, H, T), e(B * T, 2)
         self.u1, self.g1, self.v1 = e(B, H, tok), e(B, H, tok), e(B, H, T)
         self.x1 = e(B, T, H)
@@ -224,49 +319,40 @@ class MlpBnBlock:
             self.dA, self.dC = e(B * T * H), e(B, T, H)
             self.dB = e(max(B * T * ch, B * H * tok))
 
-    # channels / elements-per-channel of the four BatchNorm layers: (N, C, L, act?)
+    # channels / elements-per-channel of the four BatchNorm layers: (N, C, L)
     def _geo(self, i):
         B, T, H, tok, ch = self.B, self.T, self.H, self.tok, self.ch
         return [(B, H, tok), (B, H, T), (B, T, ch), (B, T, H)][i]
 
-    def _bn_vectors(self, i, u, act, bnm, training):
+    def _bn_vectors(self, i, u, act, training):
         """per-channel vectors of BatchNorm layer i for the tensor u (pre-activation when act >= 0)."""
         N, Cn, Ln = self._geo(i)
-        st = _stream()
         if training:
-            _call("mmx_bn1d_stats", N, Cn, Ln, act, _p(u), _p(self.sums), st)
-            _call("mmx_bn_finalize", _p(self.sums), Cn, float(N * Ln), _p(bnm.weight), _p(bnm.bias), _p(bnm.running_mean), _p(bnm.running_var),
-                  _p(bnm.num_batches_tracked), float(bnm.momentum if bnm.momentum is not None else 0.1), float(bnm.eps), _p(self.bn[i]), st)
-        else:
-            with torch.no_grad():
-                xs = torch.rsqrt(bnm.running_var + bnm.eps)
-                scale = bnm.weight.detach() * xs
-                self.bn[i].copy_(torch.cat([scale, bnm.bias.detach() - bnm.running_mean * scale, xs, -bnm.running_mean * xs]))
-        return self.bn[i]
+            _call("mmx_bn1d_stats", N, Cn, Ln, act, _p(u), _p(self.sums), _stream())
+        return bn_vectors(self.bns[i], training, self.sums, N * Ln, self.bn[i])
 
-    def forward(self, x, out, params, bns, act, se_hidden, use_max, training):
-        (ln1w, ln1b, tw1, tb1, tw2, tb2, ln2w, ln2b, cw1, cb1, cw2, cb2, s1, s2) = params
+    def forward(self, x, out, training):
+        (ln1w, ln1b, tw1, tb1, tw2, tb2, ln2w, ln2b, cw1, cb1, cw2, cb2, s1, s2) = self.params[:14]
         B, T, H, tok, ch = self.B, self.T, self.H, self.tok, self.ch
         st = _stream()
-        a = L.MMX_ACT[act]
+        a, se_hidden, use_max = self.act, self.se_hidden, self.use_max
         self.trained = bool(training)
         # ---- token half: x1 = x + SE(BN(fc2(BN(act(fc1(LN1(x)^T)))))^T)
         _call("mmx_ln_fwd", B * T, H, T, _p(x), _p(ln1w), _p(ln1b), _p(self.nT), _p(self.st1), st)
         _call("mmx_linear_fwd", B * H, T, tok, _p(self.nT), _p(tw1), _p(tb1), _p(self.u1), st)
-        bn = self._bn_vectors(0, self.u1, a, bns[0], training)
+        bn = self._bn_vectors(0, self.u1, a, training)
         _call("mmx_bn1d_apply", B, H, tok, a, _p(self.u1), _p(bn), _p(self.g1), st)
         _call("mmx_linear_fwd", B * H, tok, T, _p(self.g1), _p(tw2), _p(tb2), _p(self.v1), st)
-        bn = self._bn_vectors(1, self.v1, -1, bns[1], training)
-        _call("mmx_se_res_fwd", B, T, H, se_hidden, int(use_max), 1, 1, _p(x), _p(self.v1), _p(bn), _p(s1), _p(s2), _p(self.x1), st)
+        bn = self._bn_vectors(1, self.v1, -1, training)
+        _call("mmx_se_res_fwd", B, T, H, se_hidden, use_max, 1, 1, _p(x), _p(self.v1), _p(bn), _p(s1), _p(s2), _p(self.x1), st)
         # ---- channel half: out = x1 + SE(BN(fc2(BN(act(fc1(LN2(x1)))))))
         _call("mmx_ln_fwd", B * T, H, 0, _p(self.x1), _p(ln2w), _p(ln2b), _p(self.n2), _p(self.st2), st)
         _call("mmx_linear_fwd", B * T, H, ch, _p(self.n2), _p(cw1), _p(cb1), _p(self.u2), st)
-        bn = self._bn_vectors(2, self.u2, a, bns[2], training)
+        bn = self._bn_vectors(2, self.u2, a, training)
         _call("mmx_bn1d_apply", B, T, ch, a, _p(self.u2), _p(bn), _p(self.g2), st)
         _call("mmx_linear_fwd", B * T, ch, H, _p(self.g2), _p(cw2), _p(cb2), _p(self.v2), st)
-        bn = self._bn_vectors(3, self.v2, -1, bns[3], training)
-        _call("mmx_se_res_fwd", B, T, H, se_hidden, int(use_max), 0, 0, _p(self.x1), _p(self.v2), _p(bn), _p(s1), _p(s2), _p(out), st)
-        return out
+        bn = self._bn_vectors(3, self.v2, -1, training)
+        _call("mmx_se_res_fwd", B, T, H, se_hidden, use_max, 0, 0, _p(self.x1), _p(self.v2), _p(bn), _p(s1), _p(s2), _p(out), st)
 
     def _bn_backward(self, i, u, act, d, gw, gb):
         """d (gradient wrt the BatchNorm output, [N,C,L]) -> gradient wrt u, in place; gw / gb accumulated."""
@@ -278,16 +364,17 @@ class MlpBnBlock:
             self.coef[Cn:3 * Cn].zero_()
         _call("mmx_bn1d_bwd_apply", N, Cn, Ln, act, _p(u), _p(self.bn[i]), _p(self.coef), _p(d), _p(d), st)
 
-    def backward(self, x, dout, dx, params, grads, bn_grads, act, se_hidden, use_max):
-        """grads: tensors matching ``params`` (accumulated); bn_grads: [(d weight, d bias)] x 4 (accumulated)."""
-        (ln1w, ln1b, tw1, tb1, tw2, tb2, ln2w, ln2b, cw1, cb1, cw2, cb2, s1, s2) = params
-        (g_ln1w, g_ln1b, g_tw1, g_tb1, g_tw2, g_tb2, g_ln2w, g_ln2b, g_cw1, g_cb1, g_cw2, g_cb2, g_s1, g_s2) = grads
+    def backward(self, x, dout, dx, grads):
+        """grads: tensors matching ``params`` (accumulated)."""
+        (ln1w, ln1b, tw1, tb1, tw2, tb2, ln2w, ln2b, cw1, cb1, cw2, cb2, s1, s2) = self.params[:14]
+        (g_ln1w, g_ln1b, g_tw1, g_tb1, g_tw2, g_tb2, g_ln2w, g_ln2b, g_cw1, g_cb1, g_cw2, g_cb2, g_s1, g_s2) = grads[:14]
+        bn_grads = [grads[14 + 2 * i:16 + 2 * i] for i in range(4)]
         B, T, H, tok, ch = self.B, self.T, self.H, self.tok, self.ch
         st = _stream()
-        a = L.MMX_ACT[act]
+        a, se_hidden, use_max = self.act, self.se_hidden, self.use_max
         dA, dB, dC = self.dA, self.dB, self.dC
         # ---- channel half
-        _call("mmx_se_res_bwd", B, T, H, se_hidden, int(use_max), 0, 0, _p(self.v2), _p(self.bn[3]), _p(s1), _p(s2), _p(dout),
+        _call("mmx_se_res_bwd", B, T, H, se_hidden, use_max, 0, 0, _p(self.v2), _p(self.bn[3]), _p(s1), _p(s2), _p(dout),
               _p(g_s1), _p(g_s2), _p(dA), st)
         self._bn_backward(3, self.v2, -1, dA, *bn_grads[3])
         _call("mmx_linear_bwd", B * T, ch, H, _p(self.g2), _p(cw2), _p(dA), _p(g_cw2), _p(g_cb2), _p(dB), st)
@@ -295,60 +382,15 @@ class MlpBnBlock:
         _call("mmx_linear_bwd", B * T, H, ch, _p(self.n2), _p(cw1), _p(dB), _p(g_cw1), _p(g_cb1), _p(dA), st)
         _call("mmx_ln_bwd", B * T, H, 0, _p(self.x1), _p(self.st2), _p(ln2w), _p(dA), _p(dout), _p(dC), _p(g_ln2w), _p(g_ln2b), st)
         # ---- token half (dC = gradient wrt x1)
-        _call("mmx_se_res_bwd", B, T, H, se_hidden, int(use_max), 1, 1, _p(self.v1), _p(self.bn[1]), _p(s1), _p(s2), _p(dC),
+        _call("mmx_se_res_bwd", B, T, H, se_hidden, use_max, 1, 1, _p(self.v1), _p(self.bn[1]), _p(s1), _p(s2), _p(dC),
               _p(g_s1), _p(g_s2), _p(dA), st)
         self._bn_backward(1, self.v1, -1, dA, *bn_grads[1])
         _call("mmx_linear_bwd", B * H, tok, T, _p(self.g1), _p(tw2), _p(dA), _p(g_tw2), _p(g_tb2), _p(dB), st)
         self._bn_backward(0, self.u1, a, dB, *bn_grads[0])
         _call("mmx_linear_bwd", B * H, T, tok, _p(self.nT), _p(tw1), _p(dB), _p(g_tw1), _p(g_tb1), _p(dA), st)
         _call("mmx_ln_bwd", B * T, H, T, _p(x), _p(self.st1), _p(ln1w), _p(dA), _p(dC), _p(dx), _p(g_ln1w), _p(g_ln1b), st)
-        return dx
-
-    n_launches_fwd = 16      # training mode: 2 LN + 4 fc + 4 x (stats, finalize) + 2 apply + 2 SE
-    n_launches_bwd = 22      # 2 SE + 4 x (reduce, coef, apply) + 4 fc + 2 LN
 
 
-class _MlpBlockBN(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, x, meta, bns, *tensors):
-        x = _chk(x, "x")
-        params = [None if q is None else _chk(q, "parameter") for q in tensors[:14]]
-        tok, ch, se_hidden, act, use_se, use_max, training = meta[:7]
-        B, T, H = x.shape
-        needs_grad = any(ctx.needs_input_grad)
-        with torch.cuda.device_of(x):
-            run = MlpBnBlock(B, T, H, tok, ch, x.device, need_backward=needs_grad)
-            y = torch.empty_like(x)
-            run.forward(x, y, params, bns, act, se_hidden if use_se else 0, use_max, training)
-        ctx.run, ctx.params, ctx.x = run, params, x
-        ctx.cfg = (act, se_hidden if use_se else 0, use_max)
-        return y
-
-    @staticmethod
-    def backward(ctx, dy):
-        dy = _chk(dy, "grad")
-        run, params, x = ctx.run, ctx.params, ctx.x
-        grads = _zeros_like_many(params)
-        bn_flat = _zeros_like_many([run.bn[i][:run.bn[i].numel() // 4] for i in range(4) for _ in range(2)])
-        bn_grads = [(bn_flat[2 * i], bn_flat[2 * i + 1]) for i in range(4)]
-        dx = torch.empty_like(x)
-        with torch.cuda.device_of(x):
-            run.backward(x, dy, dx, params, grads, bn_grads, *ctx.cfg)
-        ctx.run = None
-        return (dx, None, None, *grads, *bn_flat)
-
-
-def mlp_block_bn(x, meta, params, bns):
-    """MixerBlock forward with BatchNorm1d regularisation.  ``bns``: the four BatchNorm1d modules (token reg1, token reg2,
-    channel reg1, channel reg2); their weights / biases receive gradients, their running statistics are updated in training
-    mode exactly as nn.BatchNorm1d does (momentum, unbiased variance, num_batches_tracked)."""
-    bn_tensors = [t for m in bns for t in (m.weight, m.bias)]
-    return _MlpBlockBN.apply(x, meta, tuple(bns), *params, *bn_tensors)
-
-
-# ------------------------------------------------------------------------------------------------
-# MlpMixer head (mlp_mixer.py:332-335)
-# ------------------------------------------------------------------------------------------------
 _HEAD_FIELDS = ("ln_w", "ln_b", "wt", "bt", "wf", "bf")
 
 
@@ -391,6 +433,25 @@ class _MlpHead(torch.autograd.Function):
 
 def mlp_head(x, ln_w, ln_b, wt, bt, wf, bf, precision=None):
     return _MlpHead.apply(x, ln_w, ln_b, wt, bt, wf, bf, precision)
+
+
+class MlpHead(_Runner):
+    """MlpMixer head: LN -> conv_out -> fc_out (mlp_mixer.py:332-335)."""
+
+    def __init__(self, model, B, device, need_backward):
+        self.model = model
+        self.params = [model.LN.weight, model.LN.bias, model.conv_out.weight, model.conv_out.bias, model.fc_out.weight, model.fc_out.bias]
+        self.w = mlp_head_table(self.params)
+        self.desc = L.MmxMlpHeadDesc(B, model.seq_len, model.pred_len, model.hidden_dim, model.num_classes)
+        self.out_shape = (B, model.pred_len, model.num_classes)
+
+    def forward(self, x, y, training):
+        self.prec = L.MMX_PREC[self.model.precision or _PRECISION]
+        _call("mmx_mlp_head_fwd_prec", C.byref(self.desc), C.byref(self.w), _p(x), _p(y), self.prec, _stream())
+
+    def backward(self, x, dy, dx, grads):
+        _call("mmx_mlp_head_bwd_prec", C.byref(self.desc), C.byref(self.w), C.byref(mlp_head_table(grads)), _p(x), _p(dy), _p(dx),
+              self.prec, _stream())
 
 
 # ------------------------------------------------------------------------------------------------
@@ -449,8 +510,40 @@ def angle_l1_error(pred, gt):
 
 
 # ------------------------------------------------------------------------------------------------
-# ConvMixer (conv_mixer_model.py, positional_encoder.py)
+# ConvMixer (conv_mixer_model.py, positional_encoder.py): encoder, ConvMixerBlock halves, SE tail, head
 # ------------------------------------------------------------------------------------------------
+def encoder_table(tensors):
+    t = L.MmxEncoderParams()
+    for f, v in zip(("freq", "w", "b", "wc", "bc"), tensors):
+        setattr(t, f, _p(v))
+    return t
+
+
+class Encoder(_Runner):
+    """PoseEncoder.forward (positional_encoder.py:79-97): harmonic embedding -> embed_mlp -> channelUpscaling.  Owns the
+    embedding ``m`` [B*T, E] that the backward reads."""
+    optional_dx = True
+
+    def __init__(self, enc, B, device, need_backward):
+        e = _empty(device)
+        Hn = max(int(enc.n_harmonic_functions), 0)
+        T, D, E, Cn = enc.in_nTP, enc.dimPosIn, enc.embed_mlp.out_features, enc.conv_nChan
+        self.params = [enc.embed_mlp.weight, enc.embed_mlp.bias, enc.channelUpscaling.weight, enc.channelUpscaling.bias]
+        self.w = encoder_table([enc.frequencies if Hn > 0 else None, *self.params])
+        self.desc = L.MmxEncoderDesc(B, T, D, E, Cn, Hn)
+        self.in_shape, self.out_shape = (B, T, D), (B, Cn, T, E)
+        self.m = e(B * T, E)
+        self.dm = e(B * T, E) if need_backward else None
+        self.launches = (1, 2 if Hn == 0 else 3)
+
+    def forward(self, x, y, training):
+        _call("mmx_pose_encoder_fwd", C.byref(self.desc), C.byref(self.w), _p(x), _p(self.m), _p(y), _stream())
+
+    def backward(self, x, dy, dx, grads):
+        _call("mmx_pose_encoder_bwd", C.byref(self.desc), C.byref(self.w), C.byref(encoder_table([None, *grads])), _p(x), _p(self.m),
+              _p(dy), _p(self.dm), _p(dx), _stream())
+
+
 def conv_half_table(tensors, bn_aff=None):
     """tensors: (ln_w, ln_b, conv_w, conv_b, se_w1, se_w2) — the order of ``MmxConvHalfParams``; ``bn_aff``: optional
     eval-mode BatchNorm affine [scale | shift] (2C floats)."""
@@ -461,163 +554,11 @@ def conv_half_table(tensors, bn_aff=None):
     return t
 
 
-def conv_half_desc(B, C, T, E, kernel, pad, se_hidden, act, use_se, use_max, training, site, p, seed, step, step_dev=None):
-    return L.MmxConvHalfDesc(B, C, T, E, kernel[0], kernel[1], pad[0], pad[1], se_hidden, L.MMX_ACT[act], int(use_se),
+def conv_half_desc(B, Cn, T, E, kernel, pad, se_hidden, act, use_se, use_max, training, site, p, seed, step, step_dev=None):
+    return L.MmxConvHalfDesc(B, Cn, T, E, kernel[0], kernel[1], pad[0], pad[1], se_hidden, L.MMX_ACT[act], int(use_se),
                              int(use_max), int(training), site, L.MmxDropout(float(p), int(seed), int(step), _step_dev_ptr(step_dev)))
 
 
-class _ConvHalf(torch.autograd.Function):
-    """One half of ConvMixerBlock.forward (conv_mixer_model.py:279-284 / :287-292): y = x + SE(reg(act(conv(LN(x)))))."""
-
-    @staticmethod
-    def forward(ctx, x, meta, *params):
-        x = _chk(x, "x")
-        params = [None if q is None else _chk(q, "parameter") for q in params]
-        B, C, T, E = x.shape
-        desc = conv_half_desc(B, C, T, E, *meta)
-        y = torch.empty_like(x)
-        with torch.cuda.device_of(x):
-            _call("mmx_conv_half_fwd", C_.byref(desc), C_.byref(conv_half_table(params)), _p(x), _p(y), _stream())
-        ctx.save_for_backward(x, *[q for q in params if q is not None])
-        ctx.has = [q is not None for q in params]
-        ctx.meta = meta
-        return y
-
-    @staticmethod
-    def backward(ctx, dy):
-        x, *rest = ctx.saved_tensors
-        it = iter(rest)
-        params = [next(it) if h else None for h in ctx.has]
-        dy = _chk(dy, "grad")
-        B, C, T, E = x.shape
-        desc = conv_half_desc(B, C, T, E, *ctx.meta)
-        grads = _zeros_like_many(params)
-        dx = torch.empty_like(x)
-        with torch.cuda.device_of(x):
-            _call("mmx_conv_half_bwd", C_.byref(desc), C_.byref(conv_half_table(params)), C_.byref(conv_half_table(grads)),
-                  _p(x), _p(dy), _p(dx), _stream())
-        return (dx, None, *grads)
-
-
-def conv_half(x, meta, params, bn_aff=None):
-    """meta = (kernel, pad, se_hidden, act, use_se, use_max, training, site, p, seed, step).  ``bn_aff``: eval-mode
-    BatchNorm folded to [scale | shift] (treated as a constant: no gradient flows to the BN parameters in eval mode)."""
-    if bn_aff is None:
-        return _ConvHalf.apply(x, meta, *params)
-    return _ConvHalfAffine.apply(x, meta, bn_aff, *params)
-
-
-class _ConvHalfAffine(torch.autograd.Function):
-    """The fused half with a constant per-channel affine after the activation (BatchNorm2d in eval mode)."""
-
-    @staticmethod
-    def forward(ctx, x, meta, aff, *params):
-        x, aff = _chk(x, "x"), _chk(aff, "bn affine")
-        params = [None if q is None else _chk(q, "parameter") for q in params]
-        B, C, T, E = x.shape
-        desc = conv_half_desc(B, C, T, E, *meta)
-        y = torch.empty_like(x)
-        with torch.cuda.device_of(x):
-            _call("mmx_conv_half_fwd", C_.byref(desc), C_.byref(conv_half_table(params, aff)), _p(x), _p(y), _stream())
-        ctx.save_for_backward(x, aff, *[q for q in params if q is not None])
-        ctx.has = [q is not None for q in params]
-        ctx.meta = meta
-        return y
-
-    @staticmethod
-    def backward(ctx, dy):
-        x, aff, *rest = ctx.saved_tensors
-        it = iter(rest)
-        params = [next(it) if h else None for h in ctx.has]
-        dy = _chk(dy, "grad")
-        B, C, T, E = x.shape
-        desc = conv_half_desc(B, C, T, E, *ctx.meta)
-        grads = _zeros_like_many(params)
-        dx = torch.empty_like(x)
-        with torch.cuda.device_of(x):
-            _call("mmx_conv_half_bwd", C_.byref(desc), C_.byref(conv_half_table(params, aff)), C_.byref(conv_half_table(grads)),
-                  _p(x), _p(dy), _p(dx), _stream())
-        return (dx, None, None, *grads)
-
-
-# ---- training-mode BatchNorm2d between the activation and the SE layer (regularization == -1) ----------------
-BN_EPS = 1e-5
-
-
-def bn_forward_passes(desc, tw, x, z, y, sums, bn, bn_w, bn_b, running_mean, running_var, num_batches_tracked, momentum=0.1):
-    """statistics pass -> mmx_bn_finalize (per-channel vectors, running statistics as nn.BatchNorm2d: biased variance to
-    normalise, unbiased for the running estimate) -> apply pass.  ``sums`` (float64 [2C]) must be zero on entry and is zero
-    again on exit; ``bn`` (float32 [4C]) receives [scale | shift | xs | xo]."""
-    B, Cn, T, E = x.shape
-    st = _stream()
-    _call("mmx_conv_half_bn_stats", C_.byref(desc), C_.byref(tw), _p(x), _p(z), _p(sums), st)
-    _call("mmx_bn_finalize", _p(sums), Cn, float(B * T * E), _p(bn_w), _p(bn_b), _p(running_mean), _p(running_var),
-          _p(num_batches_tracked), float(momentum), BN_EPS, _p(bn), st)
-    _call("mmx_conv_half_bn_apply", C_.byref(desc), C_.byref(tw), _p(bn), _p(x), _p(z), _p(y), st)
-    return bn
-
-
-def bn_backward_passes(desc, tw, tg, x, z, dy, dx, bn, gd, sums, coef, gw, gb, n):
-    """pass 1 (SE backward + batch sums) -> mmx_bn_coef (coefficients; gw += d bn.weight, gb += d bn.bias) -> pass 2 (BN / conv /
-    LN backward).  ``sums`` zero on entry and on exit."""
-    Cn = bn.numel() // 4
-    st = _stream()
-    _call("mmx_conv_half_bn_bwd1", C_.byref(desc), C_.byref(tw), C_.byref(tg), _p(bn), _p(z), _p(dy), _p(gd), _p(sums), st)
-    _call("mmx_bn_coef", _p(sums), Cn, float(n), _p(bn), _p(coef), _p(gw), _p(gb), st)
-    _call("mmx_conv_half_bn_bwd2", C_.byref(desc), C_.byref(tw), C_.byref(tg), _p(bn), _p(coef), _p(x), _p(z), _p(dy), _p(gd), _p(dx), st)
-
-
-class _ConvHalfBN(torch.autograd.Function):
-    """One half with training-mode BatchNorm2d: y = x + SE(BN(act(conv(LN(x)))))  (conv_mixer_model.py:139-141,279-292)."""
-
-    @staticmethod
-    def forward(ctx, x, meta, bn_w, bn_b, running_mean, running_var, num_batches_tracked, *params):
-        x = _chk(x, "x")
-        params = [None if q is None else _chk(q, "parameter") for q in params]
-        bn_w, bn_b = _chk(bn_w, "bn weight"), _chk(bn_b, "bn bias")
-        B, C, T, E = x.shape
-        desc = conv_half_desc(B, C, T, E, *meta)
-        z, y = torch.empty_like(x), torch.empty_like(x)
-        sums = torch.zeros(2 * C, dtype=torch.float64, device=x.device)
-        bn = torch.empty(4 * C, dtype=torch.float32, device=x.device)
-        with torch.cuda.device_of(x):
-            bn_forward_passes(desc, conv_half_table(params), x, z, y, sums, bn, bn_w, bn_b, running_mean, running_var, num_batches_tracked)
-        ctx.save_for_backward(x, z, bn, *[q for q in params if q is not None])
-        ctx.has = [q is not None for q in params]
-        ctx.meta = meta
-        return y
-
-    @staticmethod
-    def backward(ctx, dy):
-        x, z, bn, *rest = ctx.saved_tensors
-        it = iter(rest)
-        params = [next(it) if h else None for h in ctx.has]
-        dy = _chk(dy, "grad")
-        B, C, T, E = x.shape
-        desc = conv_half_desc(B, C, T, E, *ctx.meta)
-        grads = _zeros_like_many(params)
-        dx = torch.empty_like(x)
-        gd = torch.empty(B, T, 2, dtype=torch.float32, device=x.device)
-        sums = torch.zeros(2 * C, dtype=torch.float64, device=x.device)
-        coef = torch.empty(3 * C, dtype=torch.float32, device=x.device)
-        dw, db = torch.zeros(C, dtype=torch.float32, device=x.device), torch.zeros(C, dtype=torch.float32, device=x.device)
-        with torch.cuda.device_of(x):
-            bn_backward_passes(desc, conv_half_table(params), conv_half_table(grads), x, z, dy, dx, bn, gd, sums, coef, dw, db, B * T * E)
-        return (dx, None, dw, db, None, None, None, *grads)
-
-
-def conv_half_bn(x, meta, bn_module, params):
-    return _ConvHalfBN.apply(x, meta, bn_module.weight, bn_module.bias, bn_module.running_mean, bn_module.running_var,
-                             bn_module.num_batches_tracked, *params)
-
-
-def bn_eval_affine(bn_module):
-    """BatchNorm2d in eval mode as [scale | shift] (2C floats)."""
-    scale = bn_module.weight.detach() * torch.rsqrt(bn_module.running_var + bn_module.eps)
-    return torch.cat([scale, bn_module.bias.detach() - bn_module.running_mean * scale]).contiguous()
-
-
-# ---- large halves: shapes the fused kernels do not serve (mmx_conv_half_plan), BatchNorm with the max squeeze ----------------
 def conv_prec(precision):
     """MMX_PREC_* of a ConvMixer convolution.  ``None`` is fp32: unlike the MlpMixer, the ConvMixer does not follow
     ``set_precision`` / MMX_PRECISION (ConvMixer runs under those settings have always been fp32 and stay bit for bit); it opts
@@ -625,208 +566,148 @@ def conv_prec(precision):
     return L.MMX_PREC[precision or "fp32"]
 
 
-def conv_tc5_serves(B, C, T, E, meta):
+def conv_tc5_serves(B, Cn, T, E, meta):
     """True when precision "tf32" runs this half's convolutions on tcgen05 (mmx_conv2d_tc5_serves)."""
-    return bool(L.load().mmx_conv2d_tc5_serves(C_.byref(conv_half_desc(B, C, T, E, *meta))))
+    return bool(L.load().mmx_conv2d_tc5_serves(C.byref(conv_half_desc(B, Cn, T, E, *meta))))
 
 
-def conv_half_fits(B, C, T, E, meta):
-    """True when the fused half kernels (forward and backward) serve this shape; else the stage-kernel chain below runs."""
-    desc = conv_half_desc(B, C, T, E, *meta)
+def conv_half_fits(B, Cn, T, E, meta):
+    """True when the fused half kernels (forward and backward) serve this shape; else the stage-kernel chain runs."""
+    desc = conv_half_desc(B, Cn, T, E, *meta)
     lib = L.load()
-    return lib.mmx_conv_half_plan(C_.byref(desc), 0, None, None) == 0 and lib.mmx_conv_half_plan(C_.byref(desc), 1, None, None) == 0
+    return lib.mmx_conv_half_plan(C.byref(desc), 0, None, None) == 0 and lib.mmx_conv_half_plan(C.byref(desc), 1, None, None) == 0
 
 
-class ConvHalfLarge:
-    """Static buffers + the stage-kernel sequence of one ConvMixerBlock half that does not fit the fused kernels (include/mmx.h,
-    csrc/mmx_api_conv_large.cu): LN -> conv2d -> [BatchNorm statistics] -> act / reg / SE / residual, intermediates in HBM.
-    Used by the autograd Function below (fresh buffers per call) and by TrainStep (static buffers inside the captured graph).
-    ``params`` = ConvMixerBlock.half_params(half); ``bn``: the half's BatchNorm2d module or None."""
+class _Half(_Runner):
+    """What both runners of one ConvMixerBlock half share: y = x + SE(reg(act(conv(LN(x))))) (conv_mixer_model.py:279-284 /
+    :287-292).  ``params``: ConvMixerBlock.half_params(half), then the BatchNorm2d weight and bias when the half regularises
+    with BatchNorm (regularization == -1).  ``dropout``: (seed, step, step_dev), see ``dropout_source``."""
 
-    def __init__(self, B, C, T, E, device, need_backward=True, with_bn=False, precision=None):
-        e = lambda *shape: torch.empty(*shape, dtype=torch.float32, device=device)
-        self.B, self.C, self.T, self.E = B, C, T, E
-        self.prec = conv_prec(precision)
-        self.n, self.stats, self.z = e(B, C, T, E), e(B * C * T, 2), e(B, C, T, E)
-        self.bn = torch.zeros(4 * C, dtype=torch.float32, device=device) if with_bn else None
-        self.sums = torch.zeros(2 * C, dtype=torch.float64, device=device) if with_bn else None
+    def __init__(self, mb, half, B, device, dropout):
+        self.mb, self.half, self.B = mb, half, B
+        self.seed, self.step, self.step_dev = dropout
+        self.bnm = (mb.conv1 if half == 0 else mb.conv2).reg if mb.regularization == -1.0 else None
+        self.params = mb.half_params(half) + ([self.bnm.weight, self.bnm.bias] if self.bnm is not None else [])
+        self.C, self.T, self.E = mb.conv_nChan, mb.in_nTP, mb.dimPosEmb
+        self.out_shape = (B, self.C, self.T, self.E)
+        self.bn = torch.zeros(4 * self.C, dtype=torch.float32, device=device) if self.bnm is not None else None
+        self.sums = torch.zeros(2 * self.C, dtype=torch.float64, device=device) if self.bnm is not None else None
         self.trained = True
+
+    def _desc(self, training):
+        m = self.mb.half_meta(self.half, self.seed, self.step)
+        return conv_half_desc(self.B, self.C, self.T, self.E, *m[:6], training, *m[7:], step_dev=self.step_dev if training else None)
+
+
+class ConvHalf(_Half):
+    """One half as the fused kernels: one kernel per direction.  BatchNorm2d in training splits each direction at the batch
+    reduction: statistics pass -> mmx_bn_finalize -> apply pass, and pass 1 (SE backward + batch sums) -> mmx_bn_coef -> pass 2
+    (BN / conv / LN backward); the half owns ``z``, ``gd``, ``sums``, ``bn`` and ``coef``.  BatchNorm2d in eval is the constant
+    affine [scale | shift] applied after the activation, and its parameters take no gradient."""
+
+    def __init__(self, mb, half, B, device, need_backward, dropout):
+        super().__init__(mb, half, B, device, dropout)
+        self.w = conv_half_table(self.params[:6])
+        if self.bnm is not None:
+            e = _empty(device)
+            self.w_eval = conv_half_table(self.params[:6], self.bn)
+            self.z = e(self.out_shape)
+            if need_backward:
+                self.gd = e(B, self.T, 2)
+                self.coef = torch.zeros(3 * self.C, dtype=torch.float32, device=device)
+
+    def forward(self, x, y, training):
+        self.trained = training
+        d, st = self._desc(training), _stream()
+        if self.bnm is None:
+            _call("mmx_conv_half_fwd", C.byref(d), C.byref(self.w), _p(x), _p(y), st)
+        elif training:
+            _call("mmx_conv_half_bn_stats", C.byref(d), C.byref(self.w), _p(x), _p(self.z), _p(self.sums), st)
+            bn_vectors(self.bnm, True, self.sums, self.B * self.T * self.E, self.bn)
+            _call("mmx_conv_half_bn_apply", C.byref(d), C.byref(self.w), _p(self.bn), _p(x), _p(self.z), _p(y), st)
+        else:
+            bn_vectors(self.bnm, False, None, 0, self.bn)
+            _call("mmx_conv_half_fwd", C.byref(d), C.byref(self.w_eval), _p(x), _p(y), st)
+
+    def backward(self, x, dy, dx, grads):
+        d, g, st = self._desc(self.trained), conv_half_table(grads[:6]), _stream()
+        if self.bnm is None:
+            _call("mmx_conv_half_bwd", C.byref(d), C.byref(self.w), C.byref(g), _p(x), _p(dy), _p(dx), st)
+        elif self.trained:
+            _call("mmx_conv_half_bn_bwd1", C.byref(d), C.byref(self.w), C.byref(g), _p(self.bn), _p(self.z), _p(dy), _p(self.gd),
+                  _p(self.sums), st)
+            _call("mmx_bn_coef", _p(self.sums), self.C, float(self.B * self.T * self.E), _p(self.bn), _p(self.coef), _p(grads[6]),
+                  _p(grads[7]), st)
+            _call("mmx_conv_half_bn_bwd2", C.byref(d), C.byref(self.w), C.byref(g), _p(self.bn), _p(self.coef), _p(x), _p(self.z),
+                  _p(dy), _p(self.gd), _p(dx), st)
+        else:
+            _call("mmx_conv_half_bwd", C.byref(d), C.byref(self.w_eval), C.byref(g), _p(x), _p(dy), _p(dx), st)
+            grads[6:] = [None, None]
+
+
+class ConvHalfLarge(_Half):
+    """One half that the fused kernels do not serve (mmx_conv_half_plan), or BatchNorm with the max squeeze, as a chain of
+    stage kernels (include/mmx.h, csrc/mmx_api_conv_large.cu): LN -> conv2d -> [BatchNorm statistics] -> act / reg / SE /
+    residual, intermediates in HBM.  The convolutions follow the block's precision, see ``conv_prec``."""
+
+    def __init__(self, mb, half, B, device, need_backward, dropout):
+        super().__init__(mb, half, B, device, dropout)
+        e = _empty(device)
+        B, Cn, T, E = self.out_shape
+        self.prec = conv_prec(mb.precision)
+        self.n, self.stats, self.z = e(B, Cn, T, E), e(B * Cn * T, 2), e(B, Cn, T, E)
         if need_backward:
-            self.gd, self.dz, self.dn = e(B, T, 3), e(B, C, T, E), e(B, C, T, E)
-            self.coef = e(3 * C) if with_bn else None
+            self.gd, self.dz, self.dn = e(B, T, 3), e(B, Cn, T, E), e(B, Cn, T, E)
+            self.coef = e(3 * Cn) if self.bnm is not None else None
+        self.launches = (5, 7) if self.bnm is not None else (3, 6)
 
-    def forward(self, desc, x, y, params, bnm=None):
-        ln_w, ln_b, cw, cb, s1, s2 = params
-        B, Cn, T, E = self.B, self.C, self.T, self.E
-        st = _stream()
+    def forward(self, x, y, training):
+        ln_w, ln_b, cw, cb, s1, s2 = self.params[:6]
+        B, Cn, T, E = self.out_shape
+        desc, st = self._desc(training), _stream()
         _call("mmx_ln_fwd", B * Cn * T, E, 0, _p(x), _p(ln_w), _p(ln_b), _p(self.n), _p(self.stats), st)
-        _call("mmx_conv2d_large_fwd_prec", C_.byref(desc), 0, _p(self.n), _p(cw), _p(cb), _p(self.z), self.prec, st)
-        aff = None
-        self.trained = bool(desc.training)
-        if bnm is not None:
-            if desc.training:
-                _call("mmx_bn1d_stats", B, Cn, T * E, desc.act, _p(self.z), _p(self.sums), st)
-                _call("mmx_bn_finalize", _p(self.sums), Cn, float(B * T * E), _p(bnm.weight), _p(bnm.bias), _p(bnm.running_mean),
-                      _p(bnm.running_var), _p(bnm.num_batches_tracked), float(bnm.momentum if bnm.momentum is not None else 0.1),
-                      float(bnm.eps), _p(self.bn), st)
-            else:
-                with torch.no_grad():
-                    xs = torch.rsqrt(bnm.running_var + bnm.eps)
-                    scale = bnm.weight.detach() * xs
-                    self.bn.copy_(torch.cat([scale, bnm.bias.detach() - bnm.running_mean * scale, xs, -bnm.running_mean * xs]))
-            aff = self.bn
-        _call("mmx_conv_tail_fwd", C_.byref(desc), _p(x), _p(self.z), _p(aff), _p(s1), _p(s2), _p(y), st)
-        return y
+        _call("mmx_conv2d_large_fwd_prec", C.byref(desc), 0, _p(self.n), _p(cw), _p(cb), _p(self.z), self.prec, st)
+        self.trained = bool(training)
+        if self.bnm is not None and training:
+            _call("mmx_bn1d_stats", B, Cn, T * E, desc.act, _p(self.z), _p(self.sums), st)
+        if self.bnm is not None:
+            bn_vectors(self.bnm, training, self.sums, B * T * E, self.bn)
+        _call("mmx_conv_tail_fwd", C.byref(desc), _p(x), _p(self.z), _p(self.bn), _p(s1), _p(s2), _p(y), st)
 
-    def backward(self, desc, x, dy, dx, params, grads, bn_grads=None):
-        ln_w, ln_b, cw, cb, s1, s2 = params
-        g_ln_w, g_ln_b, g_cw, g_cb, g_s1, g_s2 = grads
-        B, Cn, T, E = self.B, self.C, self.T, self.E
-        st = _stream()
-        bn = self.bn if bn_grads is not None else None
-        _call("mmx_conv_tail_bwd1", C_.byref(desc), _p(self.z), _p(dy), _p(bn), _p(s1), _p(s2), _p(g_s1), _p(g_s2), _p(self.gd),
-              _p(self.sums) if bn is not None else None, st)
-        coef = None
+    def backward(self, x, dy, dx, grads):
+        ln_w, ln_b, cw, cb, s1, s2 = self.params[:6]
+        g_ln_w, g_ln_b, g_cw, g_cb, g_s1, g_s2 = grads[:6]
+        B, Cn, T, E = self.out_shape
+        desc, st = self._desc(self.trained), _stream()
+        bn = self.bn
+        _call("mmx_conv_tail_bwd1", C.byref(desc), _p(self.z), _p(dy), _p(bn), _p(s1), _p(s2), _p(g_s1), _p(g_s2), _p(self.gd),
+              _p(self.sums), st)
         if bn is not None:
-            _call("mmx_bn_coef", _p(self.sums), Cn, float(B * T * E), _p(self.bn), _p(self.coef), _p(bn_grads[0]), _p(bn_grads[1]), st)
+            _call("mmx_bn_coef", _p(self.sums), Cn, float(B * T * E), _p(bn), _p(self.coef), _p(grads[6]), _p(grads[7]), st)
             if not self.trained:
                 self.coef[Cn:3 * Cn].zero_()
-            coef = self.coef
-        _call("mmx_conv_tail_bwd2", C_.byref(desc), _p(self.z), _p(dy), _p(self.gd), _p(bn), _p(coef), _p(self.dz), st)
-        _call("mmx_conv2d_large_wgrad_prec", C_.byref(desc), _p(self.dz), _p(self.n), _p(g_cw), _p(g_cb), self.prec, st)
-        _call("mmx_conv2d_large_fwd_prec", C_.byref(desc), 1, _p(self.dz), _p(cw), None, _p(self.dn), self.prec, st)
+        _call("mmx_conv_tail_bwd2", C.byref(desc), _p(self.z), _p(dy), _p(self.gd), _p(bn), _p(self.coef), _p(self.dz), st)
+        _call("mmx_conv2d_large_wgrad_prec", C.byref(desc), _p(self.dz), _p(self.n), _p(g_cw), _p(g_cb), self.prec, st)
+        _call("mmx_conv2d_large_fwd_prec", C.byref(desc), 1, _p(self.dz), _p(cw), None, _p(self.dn), self.prec, st)
         _call("mmx_ln_bwd", B * Cn * T, E, 0, _p(x), _p(self.stats), _p(ln_w), _p(self.dn), _p(dy), _p(dx), _p(g_ln_w), _p(g_ln_b), st)
-        return dx
-
-    @staticmethod
-    def launches(with_bn):
-        return (5 if with_bn else 3), (7 if with_bn else 6)
 
 
-class _ConvHalfLarge(torch.autograd.Function):
-    @staticmethod
-    def forward(ctx, x, meta, bnm, precision, *tensors):
-        x = _chk(x, "x")
-        params = [None if q is None else _chk(q, "parameter") for q in tensors[:6]]
-        B, C, T, E = x.shape
-        desc = conv_half_desc(B, C, T, E, *meta)
-        needs_grad = any(ctx.needs_input_grad)
-        with torch.cuda.device_of(x):
-            run = ConvHalfLarge(B, C, T, E, x.device, need_backward=needs_grad, with_bn=bnm is not None, precision=precision)
-            y = torch.empty_like(x)
-            run.forward(desc, x, y, params, bnm)
-        ctx.run, ctx.params, ctx.x, ctx.meta, ctx.has_bn = run, params, x, meta, bnm is not None
-        return y
-
-    @staticmethod
-    def backward(ctx, dy):
-        dy = _chk(dy, "grad")
-        run, params, x = ctx.run, ctx.params, ctx.x
-        B, C, T, E = x.shape
-        desc = conv_half_desc(B, C, T, E, *ctx.meta)
-        grads = _zeros_like_many(params)
-        bn_grads = None
-        if ctx.has_bn:
-            bn_grads = [torch.zeros(C, dtype=torch.float32, device=x.device), torch.zeros(C, dtype=torch.float32, device=x.device)]
-        dx = torch.empty_like(x)
-        with torch.cuda.device_of(x):
-            run.backward(desc, x, dy, dx, params, grads, bn_grads)
-        ctx.run = None
-        return (dx, None, None, None, *grads, *(bn_grads or []))
-
-
-def conv_half_large(x, meta, params, bn_module=None, precision=None):
-    """One ConvMixerBlock half through the stage-kernel chain (large shapes; BatchNorm with max squeeze).  ``precision``: see
-    ``conv_prec``."""
-    extra = [bn_module.weight, bn_module.bias] if bn_module is not None else []
-    return _ConvHalfLarge.apply(x, meta, bn_module, precision, *params, *extra)
-
-
-class _SeTail(torch.autograd.Function):
+class SeTail(_Runner):
     """mode_conv='once': y = x + se(x), or 2x without SE (conv_mixer_model.py:259-263,287-292)."""
 
-    @staticmethod
-    def forward(ctx, x, meta, se_w1, se_w2):
-        x = _chk(x, "x")
-        se_hidden, use_se, use_max = meta
-        if use_se:
-            se_w1, se_w2 = _chk(se_w1, "se weight"), _chk(se_w2, "se weight")
-        B, C, T, E = x.shape
-        y = torch.empty_like(x)
-        with torch.cuda.device_of(x):
-            _call("mmx_se_tail_fwd", B, C, T, E, se_hidden, int(use_se), int(use_max), _p(se_w1), _p(se_w2), _p(x), _p(y), _stream())
-        if use_se:
-            ctx.save_for_backward(x, se_w1, se_w2)
-        else:
-            ctx.save_for_backward(x)
-        ctx.meta = meta
-        return y
+    def __init__(self, mb, B, device, need_backward):
+        self.mb = mb
+        self.params = mb.se_weights()
+        self.out_shape = (B, mb.conv_nChan, mb.in_nTP, mb.dimPosEmb)
+        self.args = (*self.out_shape, mb.in_nTP // mb.r_se if mb.use_se else 0, int(mb.use_se), int(mb.use_max_pooling))
 
-    @staticmethod
-    def backward(ctx, dy):
-        se_hidden, use_se, use_max = ctx.meta
-        x, *se = ctx.saved_tensors
-        dy = _chk(dy, "grad")
-        B, C, T, E = x.shape
-        g1 = g2 = None
-        if use_se:
-            g1, g2 = _zeros_like_many(se)
-        dx = torch.empty_like(x)
-        with torch.cuda.device_of(x):
-            _call("mmx_se_tail_bwd", B, C, T, E, se_hidden, int(use_se), int(use_max), _p(se[0]) if use_se else None,
-                  _p(se[1]) if use_se else None, _p(g1), _p(g2), _p(x), _p(dy), _p(dx), _stream())
-        return dx, None, g1, g2
+    def forward(self, x, y, training):
+        s1, s2 = self.params
+        _call("mmx_se_tail_fwd", *self.args, _p(s1), _p(s2), _p(x), _p(y), _stream())
 
-
-def se_tail(x, se_hidden, use_se, use_max, se_w1, se_w2):
-    return _SeTail.apply(x, (se_hidden, use_se, use_max), se_w1, se_w2)
-
-
-def encoder_table(tensors):
-    t = L.MmxEncoderParams()
-    for f, v in zip(("freq", "w", "b", "wc", "bc"), tensors):
-        setattr(t, f, _p(v))
-    return t
-
-
-class _PoseEncoder(torch.autograd.Function):
-    """PoseEncoder.forward (positional_encoder.py:79-97)."""
-
-    @staticmethod
-    def forward(ctx, x, n_harmonic, C, freq, w, b, wc, bc):
-        x, w, b, wc, bc = _chk(x, "x"), _chk(w, "weight"), _chk(b, "bias"), _chk(wc, "weight"), _chk(bc, "bias")
-        if n_harmonic > 0:
-            freq = _chk(freq, "frequencies")
-        B, T, D = x.shape
-        E = b.numel()
-        desc = L.MmxEncoderDesc(B, T, D, E, C, n_harmonic)
-        m = torch.empty(B * T, E, dtype=torch.float32, device=x.device)
-        y = torch.empty(B, C, T, E, dtype=torch.float32, device=x.device)
-        with torch.cuda.device_of(x):
-            _call("mmx_pose_encoder_fwd", C_.byref(desc), C_.byref(encoder_table([freq, w, b, wc, bc])), _p(x), _p(m), _p(y), _stream())
-        ctx.save_for_backward(x, m, w, b, wc, bc, *([freq] if n_harmonic > 0 else []))
-        ctx.dims = (B, T, D, E, C, n_harmonic)
-        ctx.need_dx = ctx.needs_input_grad[0]
-        return y
-
-    @staticmethod
-    def backward(ctx, dy):
-        x, m, w, b, wc, bc, *fr = ctx.saved_tensors
-        freq = fr[0] if fr else None
-        dy = _chk(dy, "grad")
-        B, T, D, E, C, Hn = ctx.dims
-        desc = L.MmxEncoderDesc(B, T, D, E, C, Hn)
-        gw, gb, gwc, gbc = _zeros_like_many([w, b, wc, bc])
-        dm = torch.empty_like(m)
-        dx = torch.empty_like(x) if ctx.need_dx else None
-        with torch.cuda.device_of(x):
-            _call("mmx_pose_encoder_bwd", C_.byref(desc), C_.byref(encoder_table([freq, w, b, wc, bc])),
-                  C_.byref(encoder_table([None, gw, gb, gwc, gbc])), _p(x), _p(m), _p(dy), _p(dm), _p(dx), _stream())
-        return dx, None, None, None, gw, gb, gwc, gbc
-
-
-def pose_encoder(x, n_harmonic, C, freq, w, b, wc, bc):
-    return _PoseEncoder.apply(x, n_harmonic, C, freq, w, b, wc, bc)
+    def backward(self, x, dy, dx, grads):
+        s1, s2 = self.params
+        _call("mmx_se_tail_bwd", *self.args, _p(s1), _p(s2), _p(grads[0]), _p(grads[1]), _p(x), _p(dy), _p(dx), _stream())
 
 
 def conv_head_table(tensors):
@@ -836,39 +717,20 @@ def conv_head_table(tensors):
     return t
 
 
-class _ConvHead(torch.autograd.Function):
+class ConvHead(_Runner):
     """LN -> conv_out -> project_channels -> GELU -> fc_out (conv_mixer_model.py:455-463)."""
 
-    @staticmethod
-    def forward(ctx, y, *params):
-        y = _chk(y, "y")
-        params = [_chk(q, "parameter") for q in params]
-        B, C, T, E = y.shape
-        To, D = params[3].numel(), params[7].numel()
-        desc = L.MmxConvHeadDesc(B, C, T, To, E, D)
-        out = torch.empty(B, To, D, dtype=torch.float32, device=y.device)
-        with torch.cuda.device_of(y):
-            _call("mmx_conv_head_fwd", C_.byref(desc), C_.byref(conv_head_table(params)), _p(y), _p(out), _stream())
-        ctx.save_for_backward(y, *params)
-        return out
+    def __init__(self, model, B, device, need_backward):
+        self.params = model.head_params()
+        self.w = conv_head_table(self.params)
+        self.desc = L.MmxConvHeadDesc(B, model.conv_nChan, model.in_nTP, model.out_nTP, model.dimPosEmb, model.dimPosOut)
+        self.out_shape = (B, model.out_nTP, model.dimPosOut)
 
-    @staticmethod
-    def backward(ctx, dout):
-        y, *params = ctx.saved_tensors
-        dout = _chk(dout, "grad")
-        B, C, T, E = y.shape
-        To, D = params[3].numel(), params[7].numel()
-        desc = L.MmxConvHeadDesc(B, C, T, To, E, D)
-        grads = _zeros_like_many(params)
-        dy = torch.empty_like(y)
-        with torch.cuda.device_of(y):
-            _call("mmx_conv_head_bwd", C_.byref(desc), C_.byref(conv_head_table(params)), C_.byref(conv_head_table(grads)),
-                  _p(y), _p(dout), _p(dy), _stream())
-        return (dy, *grads)
+    def forward(self, x, y, training):
+        _call("mmx_conv_head_fwd", C.byref(self.desc), C.byref(self.w), _p(x), _p(y), _stream())
 
-
-def conv_head(y, ln_w, ln_b, wt, bt, wp, bp, wf, bf):
-    return _ConvHead.apply(y, ln_w, ln_b, wt, bt, wp, bp, wf, bf)
+    def backward(self, x, dy, dx, grads):
+        _call("mmx_conv_head_bwd", C.byref(self.desc), C.byref(self.w), C.byref(conv_head_table(grads)), _p(x), _p(dy), _p(dx), _stream())
 
 
 # ------------------------------------------------------------------------------------------------

@@ -60,8 +60,8 @@ class MlpBlock(nn.Module):
 
 
 class MixerBlock(nn.Module):
-    """One fused kernel forward, one backward (mlp_mixer.py:100-164); with regularization == -1 (BatchNorm1d) a chain of stage
-    kernels around the batch reductions (functional.MlpBnBlock)."""
+    """One fused kernel forward, one backward (mlp_mixer.py:100-164, functional.FusedMixerBlock); with regularization == -1
+    (BatchNorm1d) a chain of stage kernels around the batch reductions (functional.MlpBnBlock)."""
 
     def __init__(self, tokens_mlp_dim, channels_mlp_dim, seq_len, hidden_dim, activation='gelu', regularization=0,
                  initialization='none', r_se=4, use_max_pooling=False, use_se=True):
@@ -105,15 +105,15 @@ class MixerBlock(nn.Module):
                 self.activation, self.use_se, self.use_max_pooling, self.training, self.block_index, p, seed, step,
                 self.precision)
 
+    def runners(self, B, device, need_backward, dropout=None):
+        """This block's kernel runner: the stage-kernel chain with BatchNorm1d (regularization == -1, batch statistics), else
+        the fused kernels.  ``dropout``: (seed, step, step_dev) of a static plan; None draws this call's own masks."""
+        if self.regularization == -1.0:
+            return [F_.MlpBnBlock(self, B, device, need_backward)]
+        return [F_.FusedMixerBlock(self, B, device, need_backward, dropout or F_.dropout_source(self))]
+
     def forward(self, x):
-        if self.regularization == -1.0:          # BatchNorm1d inside the MLP blocks: a chain of stage kernels (batch statistics)
-            return F_.mlp_block_bn(x, self.meta(0, 0), self.kernel_params(), self.bn_modules())
-        seed = step = 0
-        if self.training and self.regularization > 0.0:
-            seed = torch.initial_seed() & 0xFFFFFFFFFFFFFFFF
-            step = self._calls
-            self._calls = (self._calls + 1) & 0xFFFFFFFF
-        return F_.mlp_block(x, self.meta(seed, step), self.kernel_params())
+        return F_.forward_layers(self, x)
 
 
 class MlpMixer(nn.Module):
@@ -159,12 +159,16 @@ class MlpMixer(nn.Module):
             mb.precision = precision
         return self
 
+    def runners(self, B, device, need_backward, dropout=None):
+        """The kernel runners of one forward pass in order: embedding, blocks, head (see ``MixerBlock.runners``).  Yielded one
+        at a time, so that ``model(x)`` builds each layer's runner just before the layer runs."""
+        yield F_.LinearEmbed(self, B, device, need_backward)
+        for mb in self.Mixer_Block:
+            yield from mb.runners(B, device, need_backward, dropout)
+        yield F_.MlpHead(self, B, device, need_backward)
+
     def forward(self, x):
         """x: [B, seq_len, input_size] -> [B, pred_len, num_classes]  (mlp_mixer.py:306-337)."""
         if x.dim() != 3 or x.shape[1] != self.seq_len or x.shape[2] != self.input_size:
             raise RuntimeError("MlpMixer.forward: expected [B, %d, %d], got %s" % (self.seq_len, self.input_size, tuple(x.shape)))
-        y = F_.linear(x, self.conv.weight, self.conv.bias, self.precision)       # Conv2d(1,H,(1,D)) == per-frame Linear
-        for mb in self.Mixer_Block:
-            y = mb(y)
-        return F_.mlp_head(y, self.LN.weight, self.LN.bias, self.conv_out.weight, self.conv_out.bias,
-                           self.fc_out.weight, self.fc_out.bias, self.precision)
+        return F_.forward_layers(self, x)

@@ -139,8 +139,8 @@ class RolloutTrainer:
         self.opt = FusedAdam(model.parameters(), lr=lr, weight_decay=weight_decay, process_group=process_group)
         if process_group is not None:
             import torch.distributed as dist
-            for gi, group in enumerate(self.opt.param_groups):      # flat buffers + rank 0's parameters now (not inside the capture warm-up)
-                self.opt._flatten(gi, group)
+            for gi in range(len(self.opt.param_groups)):           # flat buffers + rank 0's parameters now (not inside the capture warm-up)
+                self.opt.flat(gi)
             for b in model.buffers():
                 dist.broadcast(b, src=dist.get_global_rank(process_group, 0), group=process_group)
         self.use_graph = use_cuda_graph
@@ -190,8 +190,8 @@ class RolloutTrainer:
             with torch.no_grad():
                 for t, sv in zip(list(self.model.parameters()) + list(self.model.buffers()), state):
                     t.copy_(sv)
-                for st in self.opt._flat.values():
-                    st["m"].zero_(); st["v"].zero_(); st["step"].zero_()
+                for f in self.opt._flat.values():
+                    f.m.zero_(); f.v.zero_(); f.step.zero_()
                 self.step_dev.zero_()
             for m in self.model.modules():
                 if hasattr(m, "_calls"):

@@ -96,7 +96,7 @@ for B in [int(v) for v in os.environ.get("ROLLOUT_B", "50,256,4096").split(",")]
     ms = timed(lambda: tr.step(batch), 10)
     cell["train_graph"] = {"ms": ms, "value": WORLD * B / ms * 1e3, "unit": "sequences/s", "nan": bool(tr.nan_flag)}
     if WORLD > 1:
-        pmax, pmin = tr.opt._flat[0]["p"].clone(), tr.opt._flat[0]["p"].clone()
+        pmax, pmin = tr.opt.flat(0).p.clone(), tr.opt.flat(0).p.clone()
         dist.all_reduce(pmax, op=dist.ReduceOp.MAX)
         dist.all_reduce(pmin, op=dist.ReduceOp.MIN)
         cell["dp_params_identical"] = bool(torch.equal(pmax, pmin))
