@@ -19,20 +19,14 @@ extern "C" int mmx_window_split(const float* batch, int B, int Ttot, int Dfull, 
     WindowSplitArgs a;
     a.batch = batch; a.dim_used = dim_used; a.x = x; a.gt = gt; a.B = B; a.Ttot = Ttot; a.Dfull = Dfull; a.D = D; a.T = T; a.To = To;
     a.x_scale = x_scale; a.gt_scale = gt_scale;
-    const DevInfo di = dev_info();
-    const long long want = ((long long)B * (T + To) * D + kThreads * 4 - 1) / (kThreads * 4);
-    const int grid = (int)(want < (long long)di.sms * 8 ? (want > 0 ? want : 1) : (long long)di.sms * 8);
-    return launch<WindowSplitBody>(a, grid, kThreads, 16, stream, 1);
+    return launch<WindowSplitBody>(a, capped_grid(dev_info(), (long long)B * (T + To) * D, kThreads * 4, 8), kThreads, 16, stream);
 }
 
 extern "C" int mmx_pck_hist(const float* pred, const float* gt, long long n_joints, const float* thresh, int n, int* hist, void* stream) {
     if (!pred || !gt || !thresh || !hist) return fail(MMX_E_INVALID, "mmx_pck_hist: null tensor");
     if (n_joints <= 0 || n <= 0 || n > 4096) return fail(MMX_E_INVALID, "mmx_pck_hist: bad sizes");
     PckHistArgs a; a.pred = pred; a.gt = gt; a.thresh = thresh; a.hist = hist; a.n_joints = n_joints; a.n = n;
-    const DevInfo di = dev_info();
-    const long long want = (n_joints + kThreads * 4 - 1) / (kThreads * 4);
-    const int grid = (int)(want < (long long)di.sms * 4 ? want : (long long)di.sms * 4);
-    return launch<PckHistBody>(a, grid, kThreads, (size_t)(2 * n + 8) * 4, stream, 1);
+    return launch<PckHistBody>(a, capped_grid(dev_info(), n_joints, kThreads * 4, 4), kThreads, (size_t)(2 * n + 8) * 4, stream);
 }
 
 extern "C" int mmx_bn_finalize(double* sums, int C, double n, const float* w, const float* b, float* running_mean, float* running_var,
@@ -41,12 +35,12 @@ extern "C" int mmx_bn_finalize(double* sums, int C, double n, const float* w, co
     if (C <= 0 || !(n >= 1.0)) return fail(MMX_E_INVALID, "mmx_bn_finalize: bad sizes");
     BnFinalizeArgs a; a.sums = sums; a.w = w; a.b = b; a.rm = running_mean; a.rv = running_var; a.nbt = num_batches_tracked; a.bn = bn;
     a.n = n; a.momentum = momentum; a.eps = eps; a.C = C;
-    return launch<BnFinalizeBody>(a, (C + 31) / 32, 32, 16, stream, 1);
+    return launch<BnFinalizeBody>(a, (C + 31) / 32, 32, 16, stream);
 }
 
 extern "C" int mmx_bn_coef(double* sums, int C, double n, const float* bn, float* coef, float* g_weight, float* g_bias, void* stream) {
     if (!sums || !bn || !coef || !g_weight || !g_bias) return fail(MMX_E_INVALID, "mmx_bn_coef: null tensor");
     if (C <= 0 || !(n >= 1.0)) return fail(MMX_E_INVALID, "mmx_bn_coef: bad sizes");
     BnCoefArgs a; a.sums = sums; a.bn = bn; a.coef = coef; a.gw = g_weight; a.gb = g_bias; a.n = n; a.C = C;
-    return launch<BnCoefBody>(a, (C + 31) / 32, 32, 16, stream, 1);
+    return launch<BnCoefBody>(a, (C + 31) / 32, 32, 16, stream);
 }

@@ -316,18 +316,6 @@ __global__ void __launch_bounds__(kT) se_res_bwd_kernel(const SeResArgs a) {
         for (int i = tid; i < rr * T; i += nt) { atomicAdd(a.g_se1 + i, gs1[i]); atomicAdd(a.g_se2 + i, gs2[i]); }
 }
 
-int grid_for(long long work_items, int per_block) {
-    const DevInfo di = dev_info();
-    long long want = (work_items + per_block - 1) / per_block;
-    if (want < 1) want = 1;
-    const long long cap = (long long)di.sms * 8;
-    return (int)(want < cap ? want : cap);
-}
-int launch_ok(const char* what) {
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return fail(MMX_E_CUDA, "%s: kernel launch: %s", what, cudaGetErrorString(e));
-    return MMX_OK;
-}
 int act_code(int act) {    // MMX_ACT_GELU / MMX_ACT_MISH / negative: identity
     return act < 0 ? ACT_ID : (act == MMX_ACT_GELU ? ACT_GELU : (act == MMX_ACT_MISH ? ACT_MISH : -1));
 }
@@ -342,22 +330,12 @@ int check_se(int B, int T, int H, int rr, size_t* smem, const char* what) {
     if (*smem > (size_t)dev_info().max_smem) return fail(MMX_E_UNSUPPORTED, "%s: a [%d x %d] tile does not fit shared memory", what, T, H);
     return MMX_OK;
 }
-template <class K>
-int opt_in_smem(K kern, size_t smem) {
-    if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return fail(MMX_E_CUDA, "cudaFuncSetAttribute(%zu): %s", smem, cudaGetErrorString(e));
-    }
-    return MMX_OK;
-}
-
 }  // namespace
 
 extern "C" int mmx_ln_fwd(long long rows, int H, int Tt, const float* x, const float* g, const float* b, float* y, float* stats, void* stream) {
     if (!x || !g || !b || !y || !stats) return fail(MMX_E_INVALID, "mmx_ln_fwd: null tensor");
     if (rows <= 0 || H <= 0 || Tt < 0 || (Tt > 0 && rows % Tt)) return fail(MMX_E_INVALID, "mmx_ln_fwd: bad sizes");
-    ln_fwd_kernel<<<grid_for(rows, kT / 32), kT, 0, (cudaStream_t)stream>>>(x, g, b, y, stats, rows, H, Tt);
-    return launch_ok("mmx_ln_fwd");
+    return launch_kernel(ln_fwd_kernel, capped_grid(dev_info(), rows, kT / 32, 8), kT, 0, stream, kNoPdl, x, g, b, y, stats, rows, H, Tt);
 }
 
 extern "C" int mmx_ln_bwd(long long rows, int H, int Tt, const float* x, const float* stats, const float* g, const float* dy, const float* res,
@@ -365,20 +343,11 @@ extern "C" int mmx_ln_bwd(long long rows, int H, int Tt, const float* x, const f
     if (!x || !stats || !g || !dy || !dx || !dg || !db) return fail(MMX_E_INVALID, "mmx_ln_bwd: null tensor");
     if (rows <= 0 || H <= 0 || Tt < 0 || (Tt > 0 && rows % Tt)) return fail(MMX_E_INVALID, "mmx_ln_bwd: bad sizes");
     if ((size_t)H * 8 > 48 * 1024) return fail(MMX_E_UNSUPPORTED, "mmx_ln_bwd: H = %d too wide", H);
-    const DevInfo di = dev_info();
-    long long want = (rows + 63) / 64;           // >= 8 rows per warp: the per-CTA flush of dg / db is amortised
-    if (want < 1) want = 1;
-    const int grid = (int)(want < (long long)di.sms * 4 ? want : (long long)di.sms * 4);
-    ln_bwd_kernel<<<grid, kT, (size_t)H * 8, (cudaStream_t)stream>>>(x, stats, g, dy, res, dx, dg, db, rows, H, Tt);
-    return launch_ok("mmx_ln_bwd");
+    const int grid = capped_grid(dev_info(), rows, 64, 4);      // >= 8 rows per warp: the per-CTA flush of dg / db is amortised
+    return launch_kernel(ln_bwd_kernel, grid, kT, (size_t)H * 8, stream, kNoPdl, x, stats, g, dy, res, dx, dg, db, rows, H, Tt);
 }
 
-#define MMX_BN_DISPATCH(kern, ...)                                                                                              \
-    switch (code) {                                                                                                             \
-        case ACT_GELU: kern<ACT_GELU> __VA_ARGS__; break;                                                                       \
-        case ACT_MISH: kern<ACT_MISH> __VA_ARGS__; break;                                                                       \
-        default: kern<ACT_ID> __VA_ARGS__; break;                                                                               \
-    }
+#define MMX_BN_KERNEL(kern) (code == ACT_GELU ? kern<ACT_GELU> : code == ACT_MISH ? kern<ACT_MISH> : kern<ACT_ID>)
 
 static int check_bn(long long N, int C, int L, int act, const char* what) {
     if (N <= 0 || C <= 0 || L <= 0) return fail(MMX_E_INVALID, "%s: bad sizes", what);
@@ -393,11 +362,7 @@ extern "C" int mmx_bn1d_stats(long long N, int C, int L, int act, const float* u
     if (rc) return rc;
     const int code = act_code(act);
     const long long NC = N * C;
-    const DevInfo di = dev_info();
-    long long want = (NC + 127) / 128;
-    const int grid = (int)(want < (long long)di.sms * 4 ? (want < 1 ? 1 : want) : (long long)di.sms * 4);
-    MMX_BN_DISPATCH(bn_stats_kernel, <<<grid, kT, (size_t)C * 16, (cudaStream_t)stream>>>(u, sums, NC, C, L))
-    return launch_ok("mmx_bn1d_stats");
+    return launch_kernel(MMX_BN_KERNEL(bn_stats_kernel), capped_grid(dev_info(), NC, 128, 4), kT, (size_t)C * 16, stream, kNoPdl, u, sums, NC, C, L);
 }
 
 extern "C" int mmx_bn1d_apply(long long N, int C, int L, int act, const float* u, const float* bn, float* y, void* stream) {
@@ -406,8 +371,7 @@ extern "C" int mmx_bn1d_apply(long long N, int C, int L, int act, const float* u
     if (rc) return rc;
     const int code = act_code(act);
     const long long total = N * C * L;
-    MMX_BN_DISPATCH(bn_apply_kernel, <<<grid_for(total, kT * 4), kT, 0, (cudaStream_t)stream>>>(u, bn, y, total, C, L))
-    return launch_ok("mmx_bn1d_apply");
+    return launch_kernel(MMX_BN_KERNEL(bn_apply_kernel), capped_grid(dev_info(), total, kT * 4, 8), kT, 0, stream, kNoPdl, u, bn, y, total, C, L);
 }
 
 extern "C" int mmx_bn1d_bwd_reduce(long long N, int C, int L, int act, const float* u, const float* bn, const float* dy, double* sums, void* stream) {
@@ -416,11 +380,8 @@ extern "C" int mmx_bn1d_bwd_reduce(long long N, int C, int L, int act, const flo
     if (rc) return rc;
     const int code = act_code(act);
     const long long NC = N * C;
-    const DevInfo di = dev_info();
-    long long want = (NC + 127) / 128;
-    const int grid = (int)(want < (long long)di.sms * 4 ? (want < 1 ? 1 : want) : (long long)di.sms * 4);
-    MMX_BN_DISPATCH(bn_bwd_reduce_kernel, <<<grid, kT, (size_t)C * 16, (cudaStream_t)stream>>>(u, bn, dy, sums, NC, C, L))
-    return launch_ok("mmx_bn1d_bwd_reduce");
+    return launch_kernel(MMX_BN_KERNEL(bn_bwd_reduce_kernel), capped_grid(dev_info(), NC, 128, 4), kT, (size_t)C * 16, stream, kNoPdl, u, bn, dy, sums,
+                         NC, C, L);
 }
 
 extern "C" int mmx_bn1d_bwd_apply(long long N, int C, int L, int act, const float* u, const float* bn, const float* coef, const float* dy,
@@ -430,8 +391,8 @@ extern "C" int mmx_bn1d_bwd_apply(long long N, int C, int L, int act, const floa
     if (rc) return rc;
     const int code = act_code(act);
     const long long total = N * C * L;
-    MMX_BN_DISPATCH(bn_bwd_apply_kernel, <<<grid_for(total, kT * 4), kT, 0, (cudaStream_t)stream>>>(u, bn, coef, dy, du, total, C, L))
-    return launch_ok("mmx_bn1d_bwd_apply");
+    return launch_kernel(MMX_BN_KERNEL(bn_bwd_apply_kernel), capped_grid(dev_info(), total, kT * 4, 8), kT, 0, stream, kNoPdl, u, bn, coef, dy, du,
+                         total, C, L);
 }
 
 extern "C" int mmx_se_res_fwd(int B, int T, int H, int se_hidden, int use_max_pooling, int v_transposed, int affine_by_h, const float* x,
@@ -440,12 +401,10 @@ extern "C" int mmx_se_res_fwd(int B, int T, int H, int se_hidden, int use_max_po
     size_t smem;
     int rc = check_se(B, T, H, se_hidden, &smem, "mmx_se_res_fwd");
     if (rc) return rc;
-    if ((rc = opt_in_smem(se_res_fwd_kernel, smem))) return rc;
     SeResArgs a = {};
     a.x = x; a.v = v; a.bn = bn; a.se1 = se_w1; a.se2 = se_w2; a.out = out;
     a.B = B; a.T = T; a.H = H; a.rr = se_hidden; a.use_max = use_max_pooling; a.trans = v_transposed; a.by_h = affine_by_h;
-    se_res_fwd_kernel<<<grid_for(B, 1), kT, smem, (cudaStream_t)stream>>>(a);
-    return launch_ok("mmx_se_res_fwd");
+    return launch_kernel(se_res_fwd_kernel, capped_grid(dev_info(), B, 1, 8), kT, smem, stream, kNoPdl, a);
 }
 
 extern "C" int mmx_se_res_bwd(int B, int T, int H, int se_hidden, int use_max_pooling, int v_transposed, int affine_by_h, const float* v,
@@ -455,13 +414,9 @@ extern "C" int mmx_se_res_bwd(int B, int T, int H, int se_hidden, int use_max_po
     size_t smem;
     int rc = check_se(B, T, H, se_hidden, &smem, "mmx_se_res_bwd");
     if (rc) return rc;
-    if ((rc = opt_in_smem(se_res_bwd_kernel, smem))) return rc;
     SeResArgs a = {};
     a.v = v; a.bn = bn; a.se1 = se_w1; a.se2 = se_w2; a.dout = dout; a.dv = dv; a.g_se1 = g_se_w1; a.g_se2 = g_se_w2;
     a.B = B; a.T = T; a.H = H; a.rr = se_hidden; a.use_max = use_max_pooling; a.trans = v_transposed; a.by_h = affine_by_h;
-    const DevInfo di = dev_info();
-    const int grid = B < di.sms * 4 ? B : di.sms * 4;
-    se_res_bwd_kernel<<<grid, kT, smem, (cudaStream_t)stream>>>(a);
-    return launch_ok("mmx_se_res_bwd");
+    return launch_kernel(se_res_bwd_kernel, capped_grid(dev_info(), B, 1, 4), kT, smem, stream, kNoPdl, a);     // B >= 1: check_se
 }
 #endif

@@ -17,10 +17,10 @@ struct SeTailBwdBody { static MMX_D void run(Exec& ex, const SeTailArgs& a) { se
 template <int ACT>
 int dispatch(const ConvHalfFwdArgs& a, int grid, size_t smem, void* stream) {
     switch (conv_cp(a.d.C)) {
-        case 1: return launch<ConvFwdBody<ACT, 1>>(a, grid, kThreads, smem, stream, 1);
-        case 2: return launch<ConvFwdBody<ACT, 2>>(a, grid, kThreads, smem, stream, 1);
-        case 4: return launch<ConvFwdBody<ACT, 4>>(a, grid, kThreads, smem, stream, 1);
-        default: return launch<ConvFwdBody<ACT, 8>>(a, grid, kThreads, smem, stream, 1);
+        case 1: return launch<ConvFwdBody<ACT, 1>>(a, grid, kThreads, smem, stream);
+        case 2: return launch<ConvFwdBody<ACT, 2>>(a, grid, kThreads, smem, stream);
+        case 4: return launch<ConvFwdBody<ACT, 4>>(a, grid, kThreads, smem, stream);
+        default: return launch<ConvFwdBody<ACT, 8>>(a, grid, kThreads, smem, stream);
     }
 }
 
@@ -74,8 +74,8 @@ extern "C" int mmx_conv_half_bn_apply(const MmxConvHalfDesc* d, const MmxConvHal
     if (d->use_se && (!w || !w->se_w1 || !w->se_w2)) return fail(MMX_E_INVALID, "mmx_conv_half_bn_apply: use_se set but SE weights are null");
     a.se1 = w ? w->se_w1 : nullptr; a.se2 = w ? w->se_w2 : nullptr; a.g_se1 = a.g_se2 = nullptr;
     a.bn = bn; a.x = x; a.z = z; a.dy = nullptr; a.y = y; a.gd = nullptr; a.sums = nullptr;
-    return d->act == MMX_ACT_GELU ? launch<BnApplyBody<ACT_GELU>>(a, grid, kThreads, smem, stream, 1)
-                                  : launch<BnApplyBody<ACT_MISH>>(a, grid, kThreads, smem, stream, 1);
+    return d->act == MMX_ACT_GELU ? launch<BnApplyBody<ACT_GELU>>(a, grid, kThreads, smem, stream)
+                                  : launch<BnApplyBody<ACT_MISH>>(a, grid, kThreads, smem, stream);
 }
 
 extern "C" int mmx_conv_half_bn_bwd1(const MmxConvHalfDesc* d, const MmxConvHalfParams* w, const MmxConvHalfParams* grads, const float* bn,
@@ -89,8 +89,8 @@ extern "C" int mmx_conv_half_bn_bwd1(const MmxConvHalfDesc* d, const MmxConvHalf
     a.se1 = w ? w->se_w1 : nullptr; a.se2 = w ? w->se_w2 : nullptr;
     a.g_se1 = grads ? grads->se_w1 : nullptr; a.g_se2 = grads ? grads->se_w2 : nullptr;
     a.bn = bn; a.x = nullptr; a.z = z; a.dy = dy; a.y = nullptr; a.gd = gd; a.sums = sums;
-    return d->act == MMX_ACT_GELU ? launch<BnBwd1Body<ACT_GELU>>(a, grid, kThreads, smem, stream, 1)
-                                  : launch<BnBwd1Body<ACT_MISH>>(a, grid, kThreads, smem, stream, 1);
+    return d->act == MMX_ACT_GELU ? launch<BnBwd1Body<ACT_GELU>>(a, grid, kThreads, smem, stream)
+                                  : launch<BnBwd1Body<ACT_MISH>>(a, grid, kThreads, smem, stream);
 }
 
 extern "C" int mmx_conv_half_fwd(const MmxConvHalfDesc* d, const MmxConvHalfParams* w, const float* x, float* y, void* stream) {
@@ -124,7 +124,7 @@ extern "C" int mmx_se_tail_fwd(int B, int C, int T, int E, int se_hidden, int us
     int rc = plan_se_tail(B, C, T, E, se_hidden, use_se, use_max_pooling, &a.d, &smem, &grid);
     if (rc) return rc;
     a.se1 = se_w1; a.se2 = se_w2; a.g_se1 = a.g_se2 = nullptr; a.x = x; a.dy = nullptr; a.out = y;
-    return launch<SeTailFwdBody>(a, grid, kThreads, smem, stream, 1);
+    return launch<SeTailFwdBody>(a, grid, kThreads, smem, stream);
 }
 
 extern "C" int mmx_se_tail_bwd(int B, int C, int T, int E, int se_hidden, int use_se, int use_max_pooling,
@@ -136,5 +136,5 @@ extern "C" int mmx_se_tail_bwd(int B, int C, int T, int E, int se_hidden, int us
     int rc = plan_se_tail(B, C, T, E, se_hidden, use_se, use_max_pooling, &a.d, &smem, &grid);
     if (rc) return rc;
     a.se1 = se_w1; a.se2 = se_w2; a.g_se1 = g_se_w1; a.g_se2 = g_se_w2; a.x = x; a.dy = dy; a.out = dx;
-    return launch<SeTailBwdBody>(a, grid, kThreads, smem, stream, 1);
+    return launch<SeTailBwdBody>(a, grid, kThreads, smem, stream);
 }

@@ -42,8 +42,7 @@ int plan_enc_fwd(const MmxEncoderDesc* d, EncDims* out, size_t* smem, int* grid)
         e.R = R;
         const size_t bytes = (size_t)enc_smem(e).total * 4;
         if (bytes <= (size_t)di.max_smem && ((R + 3) / 4) * n_ct <= kThreads) {
-            const int per_sm = imax(1, imin(8, (int)((di.max_smem + 1024) / (bytes + 1024))));
-            *out = e; *smem = bytes; *grid = balanced_grid((rows + R - 1) / R, di.sms * per_sm);
+            *out = e; *smem = bytes; *grid = balanced_grid((rows + R - 1) / R, di.sms * ctas_per_sm(di, bytes, 8));
             return MMX_OK;
         }
     }
@@ -62,7 +61,7 @@ int check_head(const MmxConvHeadDesc* d, const MmxConvHeadParams* p, const char*
 int plan_head(const MmxConvHeadDesc* d, bool bwd, ConvHeadDims* out, size_t* smem, int* grid) {
     const DevInfo di = dev_info();
     ConvHeadDims h; h.B = d->B; h.C = d->C; h.T = d->T; h.To = d->To; h.E = d->E; h.D = d->D;
-    const int two_cta_budget = (di.max_smem + 1024) / 2 - 2048;
+    const int two_cta_budget = smem_budget(di, 2);
     const int forced = env_int(bwd ? "MMX_CHEAD_S_BWD" : "MMX_CHEAD_S_FWD", 0);
     int S0 = imax(1, 8192 / (imax(d->C * d->T, d->To) * d->E));
     S0 = imax(1, imin(S0, (d->B + 2 * di.sms - 1) / (2 * di.sms)));
@@ -74,8 +73,7 @@ int plan_head(const MmxConvHeadDesc* d, bool bwd, ConvHeadDims* out, size_t* sme
             if ((size_t)conv_head_smem(h, bwd).total * 4 <= (size_t)budget) {
                 h.S = imin(S, d->B);
                 const size_t bytes = (size_t)conv_head_smem(h, bwd).total * 4;
-                const int per_sm = imax(1, imin(8, (int)((di.max_smem + 1024) / (bytes + 1024))));
-                *out = h; *smem = bytes; *grid = balanced_grid((d->B + h.S - 1) / h.S, di.sms * per_sm);
+                *out = h; *smem = bytes; *grid = balanced_grid((d->B + h.S - 1) / h.S, di.sms * ctas_per_sm(di, bytes, 8));
                 return MMX_OK;
             }
             if (forced > 0) break;
@@ -102,7 +100,7 @@ extern "C" int mmx_pose_encoder_fwd(const MmxEncoderDesc* d, const MmxEncoderPar
     if ((rc = plan_enc_fwd(d, &a.d, &smem, &grid))) return rc;
     a.w.freq = w->freq; a.w.w = w->w; a.w.b = w->b; a.w.wc = w->wc; a.w.bc = w->bc;
     a.x = x; a.m = m; a.y = y;
-    return launch<EncFwdBody>(a, grid, kThreads, smem, stream, 1);
+    return launch<EncFwdBody>(a, grid, kThreads, smem, stream);
 }
 
 extern "C" int mmx_pose_encoder_bwd(const MmxEncoderDesc* d, const MmxEncoderParams* w, const MmxEncoderParams* grads,
@@ -119,7 +117,7 @@ extern "C" int mmx_pose_encoder_bwd(const MmxEncoderDesc* d, const MmxEncoderPar
         a.wc = w->wc; a.m = m; a.dy = dy; a.dm = dm_ws; a.g_wc = grads->wc; a.g_bc = grads->bc; a.g_b = grads->b;
         const size_t smem = (size_t)enc_bwd1_smem(a.d).total * 4;
         if (smem > (size_t)di.max_smem) return fail(MMX_E_UNSUPPORTED, "mmx_pose_encoder_bwd: dimPosEmb %d too large", d->E);
-        if ((rc = launch<EncBwd1Body>(a, balanced_grid((rows + 31) / 32, di.sms * 4), kThreads, smem, stream, 1))) return rc;
+        if ((rc = launch<EncBwd1Body>(a, balanced_grid((rows + 31) / 32, di.sms * 4), kThreads, smem, stream))) return rc;
     }
     if (Hn == 0) return mmx_linear_bwd(rows, d->D, d->E, x, w->w, dm_ws, grads->w, grads->b, dx, stream);
     EncBwd2Args a;
@@ -133,7 +131,7 @@ extern "C" int mmx_pose_encoder_bwd(const MmxEncoderDesc* d, const MmxEncoderPar
     if (smem > (size_t)di.max_smem) return fail(MMX_E_UNSUPPORTED, "mmx_pose_encoder_bwd: tile does not fit shared memory");
     if (dx && (rc = zero_async(dx, (size_t)rows * d->D * sizeof(float), stream))) return rc;
     const int groups = d->D * ((Hn + HC - 1) / HC);
-    return launch<EncBwd2Body>(a, imin(groups, di.sms * 2), kThreads, smem, stream, 1);
+    return launch<EncBwd2Body>(a, imin(groups, di.sms * 2), kThreads, smem, stream);
 }
 
 extern "C" int mmx_conv_head_fwd(const MmxConvHeadDesc* d, const MmxConvHeadParams* w, const float* y, float* out, void* stream) {
@@ -143,7 +141,7 @@ extern "C" int mmx_conv_head_fwd(const MmxConvHeadDesc* d, const MmxConvHeadPara
     ConvHeadFwdArgs a; size_t smem; int grid;
     if ((rc = plan_head(d, false, &a.d, &smem, &grid))) return rc;
     a.w = to_hw(w); a.y = y; a.out = out;
-    return launch<HeadFwdBody>(a, grid, kThreads, smem, stream, 1);
+    return launch<HeadFwdBody>(a, grid, kThreads, smem, stream);
 }
 
 extern "C" int mmx_conv_head_bwd(const MmxConvHeadDesc* d, const MmxConvHeadParams* w, const MmxConvHeadParams* grads,
@@ -156,6 +154,6 @@ extern "C" int mmx_conv_head_bwd(const MmxConvHeadDesc* d, const MmxConvHeadPara
     if ((rc = plan_head(d, true, &a.d, &smem, &grid))) return rc;
     a.w = to_hw(w); a.g = to_hw(grads); a.y = y; a.dout = dout; a.dy = dy;
     const int tiles = ((d->D + 3) / 4) * ((d->E + 3) / 4);
-    if (tiles <= kThreads) return launch<HeadBwdBody<1>>(a, grid, kThreads, smem, stream, 1);
-    return launch<HeadBwdBody<4>>(a, grid, kThreads, smem, stream, 1);
+    if (tiles <= kThreads) return launch<HeadBwdBody<1>>(a, grid, kThreads, smem, stream);
+    return launch<HeadBwdBody<4>>(a, grid, kThreads, smem, stream);
 }

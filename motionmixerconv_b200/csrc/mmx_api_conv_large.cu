@@ -432,7 +432,7 @@ int plan_large(const MmxConvHalfDesc* d, bool wgrad, ConvL* out, size_t* smem, i
     ConvL m;
     m.B = d->B; m.C = d->C; m.T = d->T; m.E = d->E; m.kt = d->kt; m.kp = d->kp; m.pt = d->pad_t; m.pp = d->pad_p; m.transposed = 0;
     m.TP = d->T + d->kt - 1;
-    const size_t budget = ((size_t)di.max_smem + 1024) / 2 - 2048;        // two CTAs per SM
+    const size_t budget = smem_budget(di, 2);
     for (int pass = 0; pass < 2; ++pass) {
         const size_t lim = pass == 0 ? budget : (size_t)di.max_smem;
         for (int EW = round_up(d->E, 4); EW >= 4; EW -= 4) {
@@ -445,41 +445,19 @@ int plan_large(const MmxConvHalfDesc* d, bool wgrad, ConvL* out, size_t* smem, i
     return fail(MMX_E_UNSUPPORTED, "large ConvMixerBlock path: kernel %dx%dx(%d,%d) does not fit shared memory", d->C, d->C, d->kt, d->kp);
 }
 
-template <class K>
-int set_smem(K kern, size_t smem) {
-    if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return fail(MMX_E_CUDA, "cudaFuncSetAttribute(%zu): %s", smem, cudaGetErrorString(e));
-    }
-    return MMX_OK;
-}
-int launched(const char* what) {
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return fail(MMX_E_CUDA, "%s: kernel launch: %s", what, cudaGetErrorString(e));
-    return MMX_OK;
-}
-
 template <int CO>
 int run_fwd(const ConvL& m, size_t smem, const float* in, const float* w, const float* bias, float* out, void* stream) {
-    int rc = set_smem(conv2d_fwd_kernel<CO>, smem);
-    if (rc) return rc;
     const DevInfo di = dev_info();
     int by = imax(1, (4 * di.sms + m.netile - 1) / m.netile);      // each CTA stages the weights once and loops over its sequences
     if (by > m.B) by = m.B;
-    dim3 grid(m.netile, by);
-    conv2d_fwd_kernel<CO><<<grid, kLT, smem, (cudaStream_t)stream>>>(m, in, w, bias, out);
-    return launched("mmx_conv2d_large_fwd");
+    return launch_kernel(conv2d_fwd_kernel<CO>, dim3(m.netile, by), kLT, smem, stream, kNoPdl, m, in, w, bias, out);
 }
 template <int CO>
 int run_wgrad(const ConvL& m, size_t smem, const float* dz, const float* n, float* dw, float* db, void* stream) {
-    int rc = set_smem(conv2d_wgrad_kernel<CO>, smem);
-    if (rc) return rc;
     const DevInfo di = dev_info();
     int by = imax(1, (2 * di.sms + m.netile - 1) / m.netile);
     if (by > m.B) by = m.B;
-    dim3 grid(m.netile, by);
-    conv2d_wgrad_kernel<CO><<<grid, kLT, smem, (cudaStream_t)stream>>>(m, dz, n, dw, db);
-    return launched("mmx_conv2d_large_wgrad");
+    return launch_kernel(conv2d_wgrad_kernel<CO>, dim3(m.netile, by), kLT, smem, stream, kNoPdl, m, dz, n, dw, db);
 }
 
 int fill_tail(TailL& a, const MmxConvHalfDesc* d, const char* what) {
@@ -535,11 +513,8 @@ extern "C" int mmx_conv_tail_fwd(const MmxConvHalfDesc* d, const float* x, const
     if (rc) return rc;
     if (!x || !z || !y || (a.rr > 0 && (!se_w1 || !se_w2))) return fail(MMX_E_INVALID, "mmx_conv_tail_fwd: null tensor");
     a.x = x; a.z = z; a.y = y; a.aff = bn_aff; a.bn = bn_aff != nullptr; a.se1 = se_w1; a.se2 = se_w2;
-    const DevInfo di = dev_info();
-    const int grid = imin(a.B, di.sms * 8);
-    if (a.act == MMX_ACT_GELU) tail_fwd_kernel<ACT_GELU><<<grid, kLT, 0, (cudaStream_t)stream>>>(a);
-    else tail_fwd_kernel<ACT_MISH><<<grid, kLT, 0, (cudaStream_t)stream>>>(a);
-    return launched("mmx_conv_tail_fwd");
+    const auto kern = a.act == MMX_ACT_GELU ? tail_fwd_kernel<ACT_GELU> : tail_fwd_kernel<ACT_MISH>;
+    return launch_kernel(kern, capped_grid(dev_info(), a.B, 1, 8), kLT, 0, stream, kNoPdl, a);        // B >= 1: fill_tail
 }
 
 // SE backward: gd [B,T,3] = (gate, d squeeze, argmax); SE weight gradients accumulated; bn (4C vector) non-null: sums[0:C] += sum dR,
@@ -551,11 +526,8 @@ extern "C" int mmx_conv_tail_bwd1(const MmxConvHalfDesc* d, const float* z, cons
     if (rc) return rc;
     if (!z || !dy || !gd || (a.rr > 0 && (!se_w1 || !se_w2 || !g_se_w1 || !g_se_w2)) || (bn && !sums)) return fail(MMX_E_INVALID, "mmx_conv_tail_bwd1: null tensor");
     a.z = z; a.dy = dy; a.aff = bn; a.bn = bn != nullptr; a.se1 = se_w1; a.se2 = se_w2; a.g_se1 = g_se_w1; a.g_se2 = g_se_w2; a.gd = gd; a.sums = sums;
-    const DevInfo di = dev_info();
-    const int grid = imin(a.B, di.sms * 4);
-    if (a.act == MMX_ACT_GELU) tail_bwd1_kernel<ACT_GELU><<<grid, kLT, 0, (cudaStream_t)stream>>>(a);
-    else tail_bwd1_kernel<ACT_MISH><<<grid, kLT, 0, (cudaStream_t)stream>>>(a);
-    return launched("mmx_conv_tail_bwd1");
+    const auto kern = a.act == MMX_ACT_GELU ? tail_bwd1_kernel<ACT_GELU> : tail_bwd1_kernel<ACT_MISH>;
+    return launch_kernel(kern, capped_grid(dev_info(), a.B, 1, 4), kLT, 0, stream, kNoPdl, a);        // B >= 1: fill_tail
 }
 
 // dz [B,C,T,E] = gradient wrt the conv output from dy, gd (tail_bwd1) and, BatchNorm, bn + coef (mmx_bn_coef)
@@ -566,12 +538,8 @@ extern "C" int mmx_conv_tail_bwd2(const MmxConvHalfDesc* d, const float* z, cons
     if (rc) return rc;
     if (!z || !dy || !gd || !dz || ((bn != nullptr) != (coef != nullptr))) return fail(MMX_E_INVALID, "mmx_conv_tail_bwd2: null tensor");
     a.z = z; a.dy = dy; a.gd_in = gd; a.aff = bn; a.coef = coef; a.bn = bn != nullptr; a.dz = dz;
-    const DevInfo di = dev_info();
     const long long nquads = (long long)a.B * a.C * a.T * ((a.E + 3) / 4);
-    long long want = (nquads + kLT - 1) / kLT;
-    const int grid = (int)(want < (long long)di.sms * 16 ? (want < 1 ? 1 : want) : (long long)di.sms * 16);
-    if (a.act == MMX_ACT_GELU) tail_bwd2_kernel<ACT_GELU><<<grid, kLT, 0, (cudaStream_t)stream>>>(a);
-    else tail_bwd2_kernel<ACT_MISH><<<grid, kLT, 0, (cudaStream_t)stream>>>(a);
-    return launched("mmx_conv_tail_bwd2");
+    const auto kern = a.act == MMX_ACT_GELU ? tail_bwd2_kernel<ACT_GELU> : tail_bwd2_kernel<ACT_MISH>;
+    return launch_kernel(kern, capped_grid(dev_info(), nquads, kLT, 16), kLT, 0, stream, kNoPdl, a);
 }
 #endif

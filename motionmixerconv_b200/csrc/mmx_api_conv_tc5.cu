@@ -13,7 +13,6 @@ static int conv_tc5_wgrad(const MmxConvHalfDesc*, const float*, const float*, fl
 }
 #else
 #include "mmx_conv_tc5.cuh"
-#include "mmx_tc5_launch.cuh"
 
 using namespace mmx;
 
@@ -36,9 +35,7 @@ static ctc5::ConvTc5Args conv_args(const MmxConvHalfDesc* d) {
 // CTAs: one per SM (the plans of the Optuna cells take most of shared memory); more where shared memory and TMEM allow
 static int conv_grid(const ctc5::ConvGeom& g, int B, size_t smem, int tm_cols) {
     const DevInfo di = dev_info();
-    const int per_sm = imax(1, imin(512 / tm_cols, (int)((di.max_smem + 1024) / (smem + 1024))));
-    const long long items = (long long)B * g.nwin;
-    return (int)(items < (long long)di.sms * per_sm ? items : (long long)di.sms * per_sm);
+    return capped_grid(di, (long long)B * g.nwin, 1, ctas_per_sm(di, smem, 512 / tm_cols));      // B, nwin >= 1: conv_tc5_ok
 }
 
 static int conv_tc5_fwd(const MmxConvHalfDesc* d, int data_gradient, const float* in, const float* w, const float* bias, float* out,
@@ -50,9 +47,8 @@ static int conv_tc5_fwd(const MmxConvHalfDesc* d, int data_gradient, const float
     const size_t smem = ctc5::conv_tc5_smem(g, d->C, false).total;
     const int cols = 2 * g.NP <= 128 ? 128 : 2 * g.NP <= 256 ? 256 : 512;
     const int grid = conv_grid(g, d->B, smem, cols);
-    if (cols == 128) return launch_tc5(ctc5::conv_tc5_fwd_kernel<128>, a, grid, tc5::kCtaThreads, smem, stream);
-    if (cols == 256) return launch_tc5(ctc5::conv_tc5_fwd_kernel<256>, a, grid, tc5::kCtaThreads, smem, stream);
-    return launch_tc5(ctc5::conv_tc5_fwd_kernel<512>, a, grid, tc5::kCtaThreads, smem, stream);
+    const auto kern = cols == 128 ? ctc5::conv_tc5_fwd_kernel<128> : cols == 256 ? ctc5::conv_tc5_fwd_kernel<256> : ctc5::conv_tc5_fwd_kernel<512>;
+    return launch_kernel(kern, grid, tc5::kCtaThreads, smem, stream, kPdl, a);
 }
 
 static int conv_tc5_wgrad(const MmxConvHalfDesc* d, const float* dz, const float* n, float* dw, float* db, void* stream) {
@@ -62,8 +58,8 @@ static int conv_tc5_wgrad(const MmxConvHalfDesc* d, const float* dz, const float
     const size_t smem = ctc5::conv_tc5_smem(g, d->C, true).total;
     const int cols = (g.MR / 128) * g.Kp <= 128 ? 128 : 256;
     const int grid = conv_grid(g, d->B, smem, cols);
-    if (cols == 128) return launch_tc5(ctc5::conv_tc5_wgrad_kernel<128>, a, grid, tc5::kCtaThreads, smem, stream);
-    return launch_tc5(ctc5::conv_tc5_wgrad_kernel<256>, a, grid, tc5::kCtaThreads, smem, stream);
+    return launch_kernel(cols == 128 ? ctc5::conv_tc5_wgrad_kernel<128> : ctc5::conv_tc5_wgrad_kernel<256>, grid, tc5::kCtaThreads, smem, stream,
+                         kPdl, a);
 }
 #endif
 

@@ -15,7 +15,6 @@ int mmx_head_tc5(bool, const MmxMlpHeadDesc*, const MmxMlpHeadParams*, const Mmx
 #else
 #include "mmx_head_tc5.cuh"
 #include "mmx_lin_tc5.cuh"
-#include "mmx_tc5_launch.cuh"
 
 using namespace mmx;
 
@@ -37,16 +36,12 @@ int mmx_lin_tc5(bool bwd, long long rows, int K, int N, const float* x, const fl
     a.R = rows; a.K = K; a.N = N;
     a.abort_count = mmx_tc5_abort_ptr();
     const DevInfo di = dev_info();
-    const long long ntiles = (rows + 127) / 128;
     const bool small = (K + 1 > N ? K + 1 : N) <= 64;
     const size_t smem = small ? lin::lin_smem<64>(K, N, bwd).total : lin::lin_smem<80>(K, N, bwd).total;
-    const int per_sm = imax(1, imin(2, (int)((di.max_smem + 1024) / (smem + 1024))));
-    const int grid = (int)(ntiles < (long long)di.sms * per_sm ? ntiles : (long long)di.sms * per_sm);
-    if (bwd)
-        return small ? launch_tc5(lin::lin_bwd_kernel<64, 2>, a, grid, tc5::kCtaThreads, smem, stream)
-                     : launch_tc5(lin::lin_bwd_kernel<80, 2>, a, grid, tc5::kCtaThreads, smem, stream);
-    return small ? launch_tc5(lin::lin_fwd_kernel<64, 2>, a, grid, tc5::kCtaThreads, smem, stream)
-                 : launch_tc5(lin::lin_fwd_kernel<80, 2>, a, grid, tc5::kCtaThreads, smem, stream);
+    const int grid = capped_grid(di, rows, 128, ctas_per_sm(di, smem, 2));        // rows >= 1: mmx_lin_tc5_ok
+    const auto kern = bwd ? (small ? lin::lin_bwd_kernel<64, 2> : lin::lin_bwd_kernel<80, 2>)
+                          : (small ? lin::lin_fwd_kernel<64, 2> : lin::lin_fwd_kernel<80, 2>);
+    return launch_kernel(kern, grid, tc5::kCtaThreads, smem, stream, kPdl, a);
 }
 
 // ------------------------------------------------------------------------------------------ output head
@@ -69,10 +64,8 @@ int mmx_head_tc5(bool bwd, const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, c
     a.S = 128 / imax(d->T, d->To);
     a.x = x; a.dout = bwd ? dout : nullptr; a.out = out;
     a.abort_count = mmx_tc5_abort_ptr();
-    const int ntiles = (d->B + a.S - 1) / a.S;
-    const int grid = imin(ntiles, dev_info().sms);
+    const int grid = capped_grid(dev_info(), d->B, a.S, 1);        // B >= 1 and S >= 1: mmx_head_tc5_ok
     const size_t smem = head::head_smem(d->H, d->D, bwd).total;
-    return bwd ? launch_tc5(head::head_bwd_kernel, a, grid, tc5::kCtaThreads, smem, stream)
-               : launch_tc5(head::head_fwd_kernel, a, grid, tc5::kCtaThreads, smem, stream);
+    return launch_kernel(bwd ? head::head_bwd_kernel : head::head_fwd_kernel, grid, tc5::kCtaThreads, smem, stream, kPdl, a);
 }
 #endif

@@ -37,12 +37,6 @@ extern "C" int mmx_l1_fwd_bwd(const float* pred, const float* gt, float* dpred, 
     if (!pred || !gt || !loss_sum) return fail(MMX_E_INVALID, "mmx_l1_fwd_bwd: null tensor");
     if (rows <= 0 || D <= 0) return fail(MMX_E_INVALID, "mmx_l1_fwd_bwd: bad sizes");
     const long long n = rows * D;
-    const DevInfo di = dev_info();
-    long long want = (n + 1023) / 1024;
-    const int grid = (int)(want < (long long)di.sms * 4 ? (want < 1 ? 1 : want) : (long long)di.sms * 4);
-    l1_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(pred, gt, dpred, loss_sum, n, gscale / (float)rows);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return fail(MMX_E_CUDA, "mmx_l1_fwd_bwd: kernel launch: %s", cudaGetErrorString(e));
-    return MMX_OK;
+    return launch_kernel(l1_kernel, capped_grid(dev_info(), n, 1024, 4), 256, 0, stream, kNoPdl, pred, gt, dpred, loss_sum, n, gscale / (float)rows);
 }
 #endif

@@ -37,7 +37,7 @@ int plan_linear(int rows, int K, int N, bool bwd, LinearDims* out, size_t* smem,
     if (rows <= 0 || K <= 0 || N <= 0) return fail(MMX_E_INVALID, "non-positive dimension");
     const DevInfo di = dev_info();
     LinearDims d; d.rows = rows; d.K = K; d.N = N;
-    const int two_cta_budget = (di.max_smem + 1024) / 2 - 2048;
+    const int two_cta_budget = smem_budget(di, 2);
     for (int pass = 0; pass < 2; ++pass) {
         const int budget = pass == 0 ? two_cta_budget : di.max_smem;
         for (int R = 128; R >= 8; R -= 8) {
@@ -47,8 +47,7 @@ int plan_linear(int rows, int K, int N, bool bwd, LinearDims* out, size_t* smem,
                 d.R = imin(R, round_up(rows, 4));
                 if (d.R == R && R >= 16) d.R = balanced_tile(rows, R, R / 2, 8, di.sms);
                 const size_t b2 = (size_t)linear_smem(d, bwd).total * 4;
-                const int per_sm = imax(1, imin(8, (int)((di.max_smem + 1024) / (b2 + 1024))));
-                *out = d; *smem = b2; *grid = balanced_grid((rows + d.R - 1) / d.R, di.sms * per_sm);
+                *out = d; *smem = b2; *grid = balanced_grid((rows + d.R - 1) / d.R, di.sms * ctas_per_sm(di, b2, 8));
                 return MMX_OK;
             }
         }
@@ -68,7 +67,7 @@ int plan_head(const MmxMlpHeadDesc* d, bool bwd, MlpHeadDims* out, size_t* smem,
     if (((d->To + 3) / 4) * ((d->T + 3) / 4) > kThreads) return fail(MMX_E_UNSUPPORTED, "pred_len %d too large", d->To);
     const DevInfo di = dev_info();
     MlpHeadDims h; h.B = d->B; h.T = d->T; h.To = d->To; h.H = d->H; h.D = d->D;
-    const int two_cta_budget = (di.max_smem + 1024) / 2 - 2048;
+    const int two_cta_budget = smem_budget(di, 2);
     const int forced = env_int(bwd ? "MMX_HEAD_S_BWD" : "MMX_HEAD_S_FWD", 0);
     // wide rows: one CTA per SM with a larger tile beats two CTAs with S = 2 (the forced-S sweep below ran in the full budget)
     for (int pass = (d->H >= 64 && forced <= 0) ? 1 : 0; pass < 2; ++pass) {
@@ -84,8 +83,7 @@ int plan_head(const MmxMlpHeadDesc* d, bool bwd, MlpHeadDims* out, size_t* smem,
                 h.S = imin(S, d->B);
                 if (forced <= 0 && h.S == S && S >= 2) h.S = balanced_tile(d->B, S, (S + 1) / 2, 1, di.sms);
                 const size_t b2 = (size_t)mlp_head_smem(h, bwd).total * 4;
-                const int per_sm = imax(1, imin(8, (int)((di.max_smem + 1024) / (b2 + 1024))));
-                *out = h; *smem = b2; *grid = balanced_grid((d->B + h.S - 1) / h.S, di.sms * per_sm);
+                *out = h; *smem = b2; *grid = balanced_grid((d->B + h.S - 1) / h.S, di.sms * ctas_per_sm(di, b2, 8));
                 return MMX_OK;
             }
             if (forced > 0) break;
@@ -126,7 +124,7 @@ int mmx_linear_fwd_prec(int rows, int K, int N, const float* x, const float* w, 
     int rc = plan_linear(rows, K, N, false, &a.d, &smem, &grid);
     if (rc) return rc;
     a.x = x; a.w = w; a.b = b; a.y = y;
-    return launch<LinFwdBody>(a, grid, kThreads, smem, stream, 1);
+    return launch<LinFwdBody>(a, grid, kThreads, smem, stream);
 }
 
 int mmx_linear_bwd_prec(int rows, int K, int N, const float* x, const float* w, const float* dy, float* dw, float* db,
@@ -138,8 +136,8 @@ int mmx_linear_bwd_prec(int rows, int K, int N, const float* x, const float* w, 
     if (rc) return rc;
     a.x = x; a.w = w; a.dy = dy; a.dw = dw; a.db = db; a.dx = dx;
     const int tiles = ((N + 3) / 4) * ((K + 3) / 4);
-    if (tiles <= kThreads) return launch<LinBwdBody<1>>(a, grid, kThreads, smem, stream, 1);
-    return launch<LinBwdBody<4>>(a, grid, kThreads, smem, stream, 1);
+    if (tiles <= kThreads) return launch<LinBwdBody<1>>(a, grid, kThreads, smem, stream);
+    return launch<LinBwdBody<4>>(a, grid, kThreads, smem, stream);
 }
 
 static MlpHeadW to_hw(const MmxMlpHeadParams* p) {
@@ -168,8 +166,8 @@ int mmx_mlp_head_fwd_prec(const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, co
     MlpHeadFwdArgs a; size_t smem; int grid;
     if ((rc = plan_head(d, false, &a.d, &smem, &grid))) return rc;
     a.w = to_hw(w); a.x = x; a.out = out;
-    if (d->T == 10) return launch<HeadFwdBody<10>>(a, grid, kThreads, smem, stream, 1);
-    return launch<HeadFwdBody<0>>(a, grid, kThreads, smem, stream, 1);
+    if (d->T == 10) return launch<HeadFwdBody<10>>(a, grid, kThreads, smem, stream);
+    return launch<HeadFwdBody<0>>(a, grid, kThreads, smem, stream);
 }
 
 int mmx_mlp_head_bwd_prec(const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, const MmxMlpHeadParams* grads,
@@ -186,11 +184,11 @@ int mmx_mlp_head_bwd_prec(const MmxMlpHeadDesc* d, const MmxMlpHeadParams* w, co
     a.w = to_hw(w); a.g = to_hw(grads); a.x = x; a.dout = dout; a.dx = dx;
     const int tiles = ((d->D + 3) / 4) * ((d->H + 3) / 4);
     if (d->T == 10) {
-        if (tiles <= kThreads) return launch<HeadBwdBody<10, 1>>(a, grid, kThreads, smem, stream, 1);
-        return launch<HeadBwdBody<10, 4>>(a, grid, kThreads, smem, stream, 1);
+        if (tiles <= kThreads) return launch<HeadBwdBody<10, 1>>(a, grid, kThreads, smem, stream);
+        return launch<HeadBwdBody<10, 4>>(a, grid, kThreads, smem, stream);
     }
-    if (tiles <= kThreads) return launch<HeadBwdBody<0, 1>>(a, grid, kThreads, smem, stream, 1);
-    return launch<HeadBwdBody<0, 4>>(a, grid, kThreads, smem, stream, 1);
+    if (tiles <= kThreads) return launch<HeadBwdBody<0, 1>>(a, grid, kThreads, smem, stream);
+    return launch<HeadBwdBody<0, 4>>(a, grid, kThreads, smem, stream);
 }
 
 int mmx_mpjpe_fwd_bwd(const float* pred, const float* gt, float* dpred, float* loss_sum, long long n_joints,
@@ -198,10 +196,7 @@ int mmx_mpjpe_fwd_bwd(const float* pred, const float* gt, float* dpred, float* l
     if (!pred || !gt || !loss_sum) return fail(MMX_E_INVALID, "mmx_mpjpe_fwd_bwd: null tensor");
     if (n_joints <= 0) return fail(MMX_E_INVALID, "mmx_mpjpe_fwd_bwd: n_joints must be positive");
     MpjpeArgs a; a.pred = pred; a.gt = gt; a.dpred = dpred; a.loss_sum = loss_sum; a.n_joints = n_joints; a.gscale = gscale;
-    const DevInfo di = dev_info();
-    const long long want = (n_joints + kThreads - 1) / kThreads;
-    const int grid = (int)(want < (long long)di.sms * 8 ? want : (long long)di.sms * 8);
-    return launch<MpjpeBody>(a, grid, kThreads, kThreads * sizeof(float), stream, 1);
+    return launch<MpjpeBody>(a, capped_grid(dev_info(), n_joints, kThreads, 8), kThreads, kThreads * sizeof(float), stream);
 }
 
 int mmx_adam_step(float* p, const float* g, float* m, float* v, long long n, const float* hyper, void* stream) {
@@ -212,13 +207,13 @@ int mmx_adam_step(float* p, const float* g, float* m, float* v, long long n, con
     const DevInfo di = dev_info();
     const long long want = ((n >> 2) + kThreads - 1) / kThreads + 1;
     const int grid = (int)(want < (long long)di.sms * 8 ? want : (long long)di.sms * 8);
-    return launch<AdamBody>(a, grid, kThreads, 16, stream, 1);
+    return launch<AdamBody>(a, grid, kThreads, 16, stream);
 }
 
 int mmx_adam_advance(float* hyper, unsigned int* step, void* stream) {
     if (!hyper || !step) return fail(MMX_E_INVALID, "mmx_adam_advance: null pointer");
     AdamAdvanceArgs a; a.hp = hyper; a.step = step;
-    return launch<AdamAdvanceBody>(a, 1, 32, 16, stream, 1);
+    return launch<AdamAdvanceBody>(a, 1, 32, 16, stream);
 }
 
 }  // extern "C"

@@ -12,8 +12,8 @@ struct MlpFwdWarpBody { static MMX_D void run(Exec& ex, const MlpBlockFwdArgs& a
 
 template <int ACT>
 int dispatch_mlp_fwd(const MlpBlockFwdArgs& a, int grid, size_t smem, void* stream) {
-    if (a.d.T == 10 && a.d.tok == 20) return launch<MlpFwdBody<ACT, 10, 20>>(a, grid, kThreads, smem, stream, 1);
-    return launch<MlpFwdBody<ACT, 0, 0>>(a, grid, kThreads, smem, stream, 1);
+    if (a.d.T == 10 && a.d.tok == 20) return launch<MlpFwdBody<ACT, 10, 20>>(a, grid, kThreads, smem, stream);
+    return launch<MlpFwdBody<ACT, 0, 0>>(a, grid, kThreads, smem, stream);
 }
 }  // namespace mmx_tu_mlp_fwd
 using namespace mmx_tu_mlp_fwd;
@@ -37,10 +37,10 @@ extern "C" int mmx_mlp_block_fwd(const MmxMlpBlockDesc* d, const MmxMlpBlockPara
         const int thr = nwarp * 32;
         const int occ = env_int("MMX_MLP_FWD_OCC", 2);   // 2: the 128-register build, two CTAs per SM (measured 8 % faster than 1 x 254 registers)
         if (occ >= 2)
-            return d->act == MMX_ACT_GELU ? launch<MlpFwdWarpBody<ACT_GELU, 10, 20>, MlpBlockFwdArgs, 2>(a, grid, thr, smem, stream, 2)
-                                          : launch<MlpFwdWarpBody<ACT_MISH, 10, 20>, MlpBlockFwdArgs, 2>(a, grid, thr, smem, stream, 2);
-        return d->act == MMX_ACT_GELU ? launch<MlpFwdWarpBody<ACT_GELU, 10, 20>>(a, grid, thr, smem, stream, 1)
-                                      : launch<MlpFwdWarpBody<ACT_MISH, 10, 20>>(a, grid, thr, smem, stream, 1);
+            return d->act == MMX_ACT_GELU ? launch<MlpFwdWarpBody<ACT_GELU, 10, 20>, MlpBlockFwdArgs, 2>(a, grid, thr, smem, stream)
+                                          : launch<MlpFwdWarpBody<ACT_MISH, 10, 20>, MlpBlockFwdArgs, 2>(a, grid, thr, smem, stream);
+        return d->act == MMX_ACT_GELU ? launch<MlpFwdWarpBody<ACT_GELU, 10, 20>>(a, grid, thr, smem, stream)
+                                      : launch<MlpFwdWarpBody<ACT_MISH, 10, 20>>(a, grid, thr, smem, stream);
     }
     return d->act == MMX_ACT_GELU ? dispatch_mlp_fwd<ACT_GELU>(a, grid, smem, stream) : dispatch_mlp_fwd<ACT_MISH>(a, grid, smem, stream);
 }

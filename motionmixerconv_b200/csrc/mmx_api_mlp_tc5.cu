@@ -21,7 +21,6 @@ int mmx_mlp_tc5_bwd_saved(const MmxMlpBlockDesc*, const MmxMlpBlockParams*, cons
 }
 #else
 #include "mmx_chan_tc5.cuh"
-#include "mmx_tc5_launch.cuh"
 #include "mmx_tok.cuh"
 
 using namespace mmx;
@@ -60,10 +59,7 @@ static __global__ void tc5_mask_kernel(Dropout dr, uint32_t site, long long rows
 extern "C" int mmx_tc5_dropout_mask(const MmxDropout* d, unsigned int site, long long rows, int W, float* out, void* stream) {
     if (!d || !out || rows <= 0 || W <= 0) return fail(MMX_E_INVALID, "mmx_tc5_dropout_mask: bad argument");
     const Dropout dr = make_dropout(*d, 1);
-    tc5_mask_kernel<<<256, 256, 0, (cudaStream_t)stream>>>(dr, site, rows, W, out);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return fail(MMX_E_CUDA, "kernel launch: %s", cudaGetErrorString(e));
-    return MMX_OK;
+    return launch_kernel(tc5_mask_kernel, 256, 256, 0, stream, kNoPdl, dr, site, rows, W, out);
 }
 
 // defined in mmx_api_mlp_wide.cu: the wide variant of the channel half (80 <= max(H, ch) <= 128, weights streamed from a workspace)
@@ -119,12 +115,9 @@ static int run_tok(bool bwd, const tok::TokArgs& t, void* stream) {
     const size_t smem = (size_t)m.total * 4;
     if (smem > (size_t)di.max_smem) return fail(MMX_E_UNSUPPORTED, "token half: tile does not fit shared memory (H=%d)", t.H);
     const int threads = tok::kTokThreads;
-    int per_sm = (int)((di.max_smem + 1024) / (smem + 1024));
-    per_sm = imax(1, imin(per_sm, bwd ? 2 : 4));
     const int ntiles = (t.B + t.S - 1) / t.S;
-    const int grid = balanced_grid(ntiles, di.sms * per_sm);
-    return bwd ? launch_tc5(tok::tok_bwd_kernel<ACT, TT>, t, grid, threads, smem, stream)
-               : launch_tc5(tok::tok_fwd_kernel<ACT, TT>, t, grid, threads, smem, stream);
+    const int grid = balanced_grid(ntiles, di.sms * ctas_per_sm(di, smem, bwd ? 2 : 4));
+    return launch_kernel(bwd ? tok::tok_bwd_kernel<ACT, TT> : tok::tok_fwd_kernel<ACT, TT>, grid, threads, smem, stream, kPdl, t);
 }
 
 static int tok_dispatch(bool bwd, const MmxMlpBlockDesc* d, const tok::TokArgs& t, void* stream) {
@@ -155,14 +148,11 @@ static int run_chan(bool bwd, const chan::ChanArgs& c, void* stream) {
     const chan::Geo g = chan::make_geo(c.T, c.H, VEC);
     const size_t smem = chan::chan_smem<KP>(g, bwd).total;
     if (smem > (size_t)di.max_smem) return fail(MMX_E_UNSUPPORTED, "channel half: tile does not fit shared memory (H=%d ch=%d)", c.H, c.ch);
-    const int ntiles = (c.B + g.seq_per_tile - 1) / g.seq_per_tile;
     // TMEM: forward 2*KP columns (<= 2 CTAs / SM at KP = 64), backward 4*KP columns
-    int per_sm = (int)((di.max_smem + 1024) / (smem + 1024));
     const int tm_cols = bwd ? 512 : (3 * KP <= 256 ? 256 : 512);
-    per_sm = imax(1, imin(per_sm, 512 / tm_cols));
-    const int grid = imin(ntiles, di.sms * per_sm);
-    return bwd ? launch_tc5(chan::chan_bwd_kernel<ACT, KP, VEC>, c, grid, tc5::kCtaThreads, smem, stream)
-               : launch_tc5(chan::chan_fwd_kernel<ACT, KP, VEC>, c, grid, tc5::kCtaThreads, smem, stream);
+    const int grid = capped_grid(di, c.B, g.seq_per_tile, ctas_per_sm(di, smem, 512 / tm_cols));     // B >= 1: check_common
+    return launch_kernel(bwd ? chan::chan_bwd_kernel<ACT, KP, VEC> : chan::chan_fwd_kernel<ACT, KP, VEC>, grid, tc5::kCtaThreads, smem, stream,
+                         kPdl, c);
 }
 
 template <int ACT>

@@ -16,7 +16,6 @@ int mmx_chan_wide_run(bool, int, const void*, void*) { return fail(MMX_E_UNSUPPO
 #include <unordered_map>
 
 #include "mmx_chan_wide.cuh"
-#include "mmx_tc5_launch.cuh"
 
 using namespace mmx;
 
@@ -52,14 +51,14 @@ static int run_wide(bool bwd, const chan::ChanArgs& c, void* stream) {
     uint8_t* ws = nullptr;
     int rc = wide_workspace(c.w1, &ws);
     if (rc) return rc;
-    if ((rc = launch_tc5v(chanw::chan_prep_kernel<KP>, KP <= 64 ? 8 : 32, 256, 0, stream, c, ws))) return rc;
+    if ((rc = launch_kernel(chanw::chan_prep_kernel<KP>, KP <= 64 ? 8 : 32, 256, 0, stream, kPdl, c, ws))) return rc;
     const int ntiles = (c.B + g.seq_per_tile - 1) / g.seq_per_tile;
     // KP = 128: 512 TMEM columns, ~205 KB shared -> one CTA per SM; KP = 64: 256 columns, < 100 KB -> two CTAs per SM
-    const int per_sm = KP <= 64 ? imax(1, imin(2, (int)((di.max_smem + 1024) / (smem + 1024)))) : 1;
+    const int per_sm = KP <= 64 ? ctas_per_sm(di, smem, 2) : 1;
     const int grid = balanced_grid(ntiles, di.sms * per_sm);
     const uint8_t* wsc = ws;
-    return bwd ? launch_tc5v(chanw::chan_wide_bwd_kernel<ACT, VEC, KP>, grid, tc5::kCtaThreads, smem, stream, c, wsc)
-               : launch_tc5v(chanw::chan_wide_fwd_kernel<ACT, VEC, KP>, grid, tc5::kCtaThreads, smem, stream, c, wsc);
+    return launch_kernel(bwd ? chanw::chan_wide_bwd_kernel<ACT, VEC, KP> : chanw::chan_wide_fwd_kernel<ACT, VEC, KP>, grid, tc5::kCtaThreads, smem,
+                         stream, kPdl, c, wsc);
 }
 
 template <int KP>

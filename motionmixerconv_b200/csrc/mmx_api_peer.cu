@@ -31,9 +31,6 @@ extern "C" int mmx_adam_step_peer(float*, float*, float*, const void*, const voi
 #else
 using namespace mmx;
 
-// defined in mmx_api_mlp_tc5.cu: per-device counter of timed-out waits (mmx_tc5_abort_count() reads it)
-int* mmx_tc5_abort_ptr();
-
 namespace {
 
 constexpr int kPeerCtas = 128;       // flag slots per rank and phase = upper bound of the grid (CTA c owns chunk c of the bucket)
@@ -202,9 +199,6 @@ extern "C" int mmx_adam_step_peer(float* p, float* m, float* v, const void* peer
     // two float4 per thread: K2 (30 K floats) 16 CTAs, K4 (183 K) 90 CTAs; fewer CTAs = fewer flags crossing NVLink
     long long want = ((n >> 2) + 2 * kPeerThreads - 1) / (2 * kPeerThreads);
     a.grid = (int)(want < 16 ? 16 : (want > kPeerCtas ? kPeerCtas : want));
-    adam_peer_kernel<<<a.grid, kPeerThreads, 0, (cudaStream_t)stream>>>(a);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return fail(MMX_E_CUDA, "mmx_adam_step_peer: kernel launch: %s", cudaGetErrorString(e));
-    return MMX_OK;
+    return launch_kernel(adam_peer_kernel, a.grid, kPeerThreads, 0, stream, kNoPdl, a);
 }
 #endif

@@ -37,7 +37,7 @@ static inline int plan_conv_half(const MmxConvHalfDesc* d, bool bwd, ConvDims* o
     m.B = d->B; m.C = d->C; m.T = d->T; m.E = d->E; m.kT = d->kt; m.kP = d->kp; m.pT = d->pad_t; m.pP = d->pad_p;
     m.rr = d->use_se ? d->se_hidden : 0; m.use_se = d->use_se; m.use_max = d->use_max_pooling; m.training = d->training;
     m.site = d->site; m.bn_mode = 0;
-    const int two_cta_budget = (di.max_smem + 1024) / 2 - 2048;
+    const int two_cta_budget = smem_budget(di, 2);
     const int forced = env_int(bwd ? "MMX_CONV_S_BWD" : "MMX_CONV_S_FWD", 0);
     // about kConvTileElems activations per tile, but never fewer tiles than ~2 per SM when the batch is small
     int S0 = imax(1, kConvTileElems / (d->C * d->T * d->E));
@@ -54,8 +54,7 @@ static inline int plan_conv_half(const MmxConvHalfDesc* d, bool bwd, ConvDims* o
                 if ((size_t)conv_smem(m, bwd).total * 4 <= (size_t)budget) {
                     m.S = imin(S, d->B);
                     const size_t bytes = (size_t)conv_smem(m, bwd).total * 4;
-                    const int per_sm = imax(1, imin(8, (int)((di.max_smem + 1024) / (bytes + 1024))));
-                    *out = m; *smem = bytes; *grid = balanced_grid((d->B + m.S - 1) / m.S, di.sms * per_sm);
+                    *out = m; *smem = bytes; *grid = balanced_grid((d->B + m.S - 1) / m.S, di.sms * ctas_per_sm(di, bytes, 8));
                     return MMX_OK;
                 }
                 if (forced > 0) break;

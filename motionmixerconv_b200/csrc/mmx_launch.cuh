@@ -9,12 +9,17 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <map>
+#include <mutex>
+
 #include "../../include/mmx.h"
 #include "mmx_common.cuh"
 
 // defined in mmx_api_misc.cu: records the thread-local message returned by mmx_last_error()
 int mmx_fail(int code, const char* fmt, ...);
 #define fail mmx_fail
+// address of the per-device counter of timed-out pipeline waits of the tcgen05 kernels (defined in mmx_api_mlp_tc5.cu)
+int* mmx_tc5_abort_ptr();
 
 namespace mmx {
 
@@ -29,7 +34,7 @@ struct DevInfo { int sms = 4; int max_smem = 227 * 1024; };
 static inline DevInfo dev_info() { return DevInfo(); }
 
 template <class Body, class Args, int OCC = 1>
-static int launch(const Args& a, int grid, int block, size_t smem_bytes, void*, int /*min_blocks*/) {
+static int launch(const Args& a, int grid, int block, size_t smem_bytes, void*) {
     std::vector<float> buf(smem_bytes / 4 + 8);
     float* sm = buf.data();
     while (((uintptr_t)sm) & 15) ++sm;
@@ -44,17 +49,64 @@ static int launch(const Args& a, int grid, int block, size_t smem_bytes, void*, 
 // ----------------------------------------------------------------------------- CUDA
 struct DevInfo { int sms; int max_smem; };
 static inline DevInfo dev_info() {
+    static std::mutex mu;
     static DevInfo cache[64];
     static bool have[64] = {};
     int dev = 0;
     cudaGetDevice(&dev);
     if (dev < 0 || dev >= 64) dev = 0;
+    std::lock_guard<std::mutex> lk(mu);
     if (!have[dev]) {
         cudaDeviceGetAttribute(&cache[dev].sms, cudaDevAttrMultiProcessorCount, dev);
         cudaDeviceGetAttribute(&cache[dev].max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
         have[dev] = true;
     }
     return cache[dev];
+}
+
+// values of launch_kernel's `pdl` argument
+constexpr bool kPdl = true, kNoPdl = false;
+
+// The one place a kernel of libmmx.so is launched.  Dynamic shared memory above 48 KB needs an opt-in per (kernel, device); with
+// it, and on every programmatic dependent launch, ask for the full shared-memory carve-out: the planners size tiles so that two
+// or more CTAs fit one SM, and otherwise the driver may pick an L1/shared split that holds fewer.
+// pdl = kPdl (programmatic dependent launch): the kernel's parameter-only prologue may overlap the tail of the previous kernel in
+// the stream.  Only for kernels that call griddepcontrol.wait before touching anything a predecessor writes (the tcgen05 family).
+template <class K, class... A>
+static int launch_kernel(K kern, dim3 grid, int block, size_t smem, void* stream, bool pdl, const A&... args) {
+    const bool opt_in = smem > 48 * 1024;
+    if (opt_in || pdl) {
+        static std::mutex mu;
+        static std::map<std::pair<const void*, int>, size_t> configured;     // (kernel, device) -> shared memory opted in to
+        int dev = 0;
+        cudaGetDevice(&dev);
+        std::lock_guard<std::mutex> lk(mu);
+        auto it = configured.find({(const void*)kern, dev});
+        if (it == configured.end() || (opt_in && it->second < smem)) {
+            if (opt_in) {
+                cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+                if (e != cudaSuccess) return fail(MMX_E_CUDA, "cudaFuncSetAttribute(%zu): %s", smem, cudaGetErrorString(e));
+            }
+            cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
+            configured[{(const void*)kern, dev}] = opt_in ? smem : 0;
+        }
+    }
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid;
+    cfg.blockDim = dim3(block);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = (cudaStream_t)stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = pdl ? 1 : 0;
+    cudaError_t e = cudaLaunchKernelEx(&cfg, kern, args...);
+    if (e != cudaSuccess) {
+        cudaGetLastError();             // reported here: keep it from surfacing again at the caller's next error check
+        return fail(MMX_E_CUDA, "kernel launch: %s", cudaGetErrorString(e));
+    }
+    return MMX_OK;
 }
 
 template <class Body, class Args>
@@ -73,28 +125,24 @@ static __global__ void __launch_bounds__(256, 2) mmx_kernel_occ2(const Args a) {
 }
 
 template <class Body, class Args, int OCC = 1>
-static int launch(const Args& a, int grid, int block, size_t smem_bytes, void* stream, int /*min_blocks*/) {
-    constexpr int min_blocks = OCC;
-    auto kern = OCC >= 2 ? mmx_kernel_occ2<Body, Args> : mmx_kernel<Body, Args>;
-    static size_t configured[2][64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64) dev = 0;
-    size_t& conf = configured[min_blocks >= 2 ? 1 : 0][dev];
-    if (smem_bytes > 48 * 1024 && conf < smem_bytes) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes);
-        if (e != cudaSuccess) return fail(MMX_E_CUDA, "cudaFuncSetAttribute(%zu): %s", smem_bytes, cudaGetErrorString(e));
-        // the planners size tiles so that two CTAs fit one SM: ask for the full shared-memory carve-out, otherwise the driver
-        // may pick an L1/shared split that holds only one
-        cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared);
-        conf = smem_bytes;
-    }
-    kern<<<grid, block, smem_bytes, (cudaStream_t)stream>>>(a);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return fail(MMX_E_CUDA, "kernel launch: %s", cudaGetErrorString(e));
-    return MMX_OK;
+static int launch(const Args& a, int grid, int block, size_t smem_bytes, void* stream) {
+    return launch_kernel(OCC >= 2 ? mmx_kernel_occ2<Body, Args> : mmx_kernel<Body, Args>, grid, block, smem_bytes, stream, kNoPdl, a);
 }
 #endif
+
+// Occupancy arithmetic.  Every resident CTA also takes 1 KB of the SM's shared memory that the kernel does not see, which is
+// why an SM holds max_smem + 1 KB in all.
+// CTAs of `smem` bytes of dynamic shared memory that fit on one SM, in [1, cap]
+static inline int ctas_per_sm(const DevInfo& di, size_t smem, int cap) {
+    return imax(1, imin(cap, (int)((di.max_smem + 1024) / (smem + 1024))));
+}
+// dynamic shared memory per CTA that leaves room for n CTAs per SM (and 1 KB of slack)
+static inline int smem_budget(const DevInfo& di, int n) { return (di.max_smem + 1024) / n - 2048; }
+// grid of ceil(work / per_cta) CTAs, in [1, k x SMs]
+static inline int capped_grid(const DevInfo& di, long long work, long long per_cta, int k) {
+    const long long want = (work + per_cta - 1) / per_cta, cap = (long long)di.sms * k;
+    return (int)(want < 1 ? 1 : want < cap ? want : cap);
+}
 
 // grid for a persistent loop over `ntiles` tiles with at most `max_ctas` resident CTAs: balance the
 // tiles so every CTA runs the same number of iterations (no ragged last wave)

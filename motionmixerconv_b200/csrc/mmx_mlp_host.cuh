@@ -36,7 +36,7 @@ static inline int plan_mlp_block(const MmxMlpBlockDesc* d, bool bwd, MlpDims* ou
     m.use_se = d->use_se; m.use_max = d->use_max_pooling; m.training = d->training; m.site_base = d->block_index * 4;
     m.align_mask = 0;
     const int forced = env_int(bwd ? "MMX_MLP_S_BWD" : "MMX_MLP_S_FWD", 0);
-    const int two_cta_budget = (di.max_smem + 1024) / 2 - 1024 - 1024;   // room for 2 CTAs / SM
+    const int two_cta_budget = smem_budget(di, 2);
     const int row_target = bwd ? 96 : 128;
     // Two candidates: channel-MLP weights staged in shared memory, or read from global (L1/L2; needs H, ch % 4 == 0).  Large H:
     // the staged weights leave room for a single sequence per tile (10 rows: GEMM phases with a handful of busy threads),
@@ -62,9 +62,8 @@ static inline int plan_mlp_block(const MmxMlpBlockDesc* d, bool bwd, MlpDims* ou
         m.S = imin(bestS[pick], d->B);
         if (forced <= 0 && m.S == bestS[pick] && m.S >= 2) m.S = balanced_tile(d->B, m.S, (m.S + 1) / 2, 1, di.sms);
         const size_t bytes = (size_t)mlp_block_smem(m, bwd).total * 4;
-        const int per_sm = imax(1, imin(8, (int)((di.max_smem + 1024) / (bytes + 1024))));
         const int ntiles = (d->B + m.S - 1) / m.S;
-        *out = m; *smem = bytes; *grid = balanced_grid(ntiles, di.sms * per_sm);
+        *out = m; *smem = bytes; *grid = balanced_grid(ntiles, di.sms * ctas_per_sm(di, bytes, 8));
         return MMX_OK;
     }
     return fail(MMX_E_UNSUPPORTED, "MixerBlock tile does not fit shared memory (H=%d ch=%d)", d->H, d->ch);
@@ -93,7 +92,7 @@ static inline int plan_mlp_block_warp(const MmxMlpBlockDesc* d, bool bwd, MlpDim
         if (bytes <= (size_t)di.max_smem) break;
     }
     if (nwarp < 2) return fail(MMX_E_UNSUPPORTED, "MixerBlock (warp variant) does not fit shared memory");
-    const int per_sm = imax(1, imin(4, (int)((di.max_smem + 1024) / (bytes + 1024))));
+    const int per_sm = ctas_per_sm(di, bytes, 4);
     const int groups = (d->B + kSPW - 1) / kSPW;
     const int max_warps = di.sms * per_sm * nwarp;
     const int waves = (groups + max_warps - 1) / max_warps;
