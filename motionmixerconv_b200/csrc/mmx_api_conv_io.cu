@@ -22,13 +22,16 @@ int check_enc(const MmxEncoderDesc* d, const MmxEncoderParams* w, const char* wh
     return MMX_OK;
 }
 
+constexpr int kEncChunkCols = 256;     // harmonic PoseEncoder forward: embedding columns (sin and cos) per chunk of input dimensions
+constexpr int kEncBwdRows = 128;       // harmonic PoseEncoder backward, stage 2: frames staged per step of its sweep over the batch
+
 int plan_enc_fwd(const MmxEncoderDesc* d, EncDims* out, size_t* smem, int* grid) {
     const DevInfo di = dev_info();
     EncDims e;
     e.B = d->B; e.T = d->T; e.D = d->D; e.E = d->E; e.C = d->C; e.Hn = d->n_harmonic > 0 ? d->n_harmonic : 0;
     e.K = e.Hn > 0 ? 2 * e.Hn * e.D : e.D;
     if (e.Hn > 0) {       // a chunk = DC input dimensions: their sin and cos columns (2*DC*Hn embedding columns)
-        e.DC = imax(1, imin(e.D, env_int("MMX_ENC_KC", 256) / (2 * e.Hn)));
+        e.DC = imax(1, imin(e.D, kEncChunkCols / (2 * e.Hn)));
         e.KC = round_up(2 * e.DC * e.Hn, 4);
     } else {
         e.DC = 0;
@@ -61,23 +64,16 @@ int check_head(const MmxConvHeadDesc* d, const MmxConvHeadParams* p, const char*
 int plan_head(const MmxConvHeadDesc* d, bool bwd, ConvHeadDims* out, size_t* smem, int* grid) {
     const DevInfo di = dev_info();
     ConvHeadDims h; h.B = d->B; h.C = d->C; h.T = d->T; h.To = d->To; h.E = d->E; h.D = d->D;
-    const int two_cta_budget = smem_budget(di, 2);
-    const int forced = env_int(bwd ? "MMX_CHEAD_S_BWD" : "MMX_CHEAD_S_FWD", 0);
+    const int forced = env_int(bwd ? "MMX_CHEAD_S_BWD" : "MMX_CHEAD_S_FWD", 0);   // tests: force the tile
     int S0 = imax(1, 8192 / (imax(d->C * d->T, d->To) * d->E));
     S0 = imax(1, imin(S0, (d->B + 2 * di.sms - 1) / (2 * di.sms)));
     if (forced > 0) S0 = forced;
-    for (int pass = 0; pass < 2; ++pass) {
-        const int budget = pass == 0 ? two_cta_budget : di.max_smem;
-        for (int S = S0; S >= 1; --S) {
-            h.S = S;
-            if ((size_t)conv_head_smem(h, bwd).total * 4 <= (size_t)budget) {
-                h.S = imin(S, d->B);
-                const size_t bytes = (size_t)conv_head_smem(h, bwd).total * 4;
-                *out = h; *smem = bytes; *grid = balanced_grid((d->B + h.S - 1) / h.S, di.sms * ctas_per_sm(di, bytes, 8));
-                return MMX_OK;
-            }
-            if (forced > 0) break;
-        }
+    const int S = fit_tile(di, S0, forced > 0 ? forced : 1, 1, true, [&](int s) { h.S = s; return (size_t)conv_head_smem(h, bwd).total * 4; });
+    if (S) {
+        h.S = imin(S, d->B);
+        const size_t bytes = (size_t)conv_head_smem(h, bwd).total * 4;
+        *out = h; *smem = bytes; *grid = tile_grid(di, d->B, h.S, bytes);
+        return MMX_OK;
     }
     return fail(MMX_E_UNSUPPORTED, "ConvMixer head tile does not fit shared memory (C=%d E=%d D=%d To=%d)", d->C, d->E, d->D, d->To);
 }
@@ -121,7 +117,7 @@ extern "C" int mmx_pose_encoder_bwd(const MmxEncoderDesc* d, const MmxEncoderPar
     }
     if (Hn == 0) return mmx_linear_bwd(rows, d->D, d->E, x, w->w, dm_ws, grads->w, grads->b, dx, stream);
     EncBwd2Args a;
-    a.d.B = d->B; a.d.T = d->T; a.d.D = d->D; a.d.E = d->E; a.d.Hn = Hn; a.d.R = env_int("MMX_ENC_BWD_R", 128); a.d.need_dx = dx != nullptr;
+    a.d.B = d->B; a.d.T = d->T; a.d.D = d->D; a.d.E = d->E; a.d.Hn = Hn; a.d.R = kEncBwdRows; a.d.need_dx = dx != nullptr;
     int HC = 32;
     while (HC > 2 && (HC > Hn || ((d->E + 3) / 4) * (2 * HC / 4) > kThreads)) HC /= 2;
     if (((d->E + 3) / 4) * (2 * HC / 4) > kThreads) return fail(MMX_E_UNSUPPORTED, "mmx_pose_encoder_bwd: dimPosEmb %d too large", d->E);

@@ -432,15 +432,15 @@ int plan_large(const MmxConvHalfDesc* d, bool wgrad, ConvL* out, size_t* smem, i
     ConvL m;
     m.B = d->B; m.C = d->C; m.T = d->T; m.E = d->E; m.kt = d->kt; m.kp = d->kp; m.pt = d->pad_t; m.pp = d->pad_p; m.transposed = 0;
     m.TP = d->T + d->kt - 1;
-    const size_t budget = smem_budget(di, 2);
-    for (int pass = 0; pass < 2; ++pass) {
-        const size_t lim = pass == 0 ? budget : (size_t)di.max_smem;
-        for (int EW = round_up(d->E, 4); EW >= 4; EW -= 4) {
-            m.EW = EW; m.EWP = EW + d->kp + 3; m.netile = (d->E + EW - 1) / EW;
-            const size_t slab = (size_t)m.C * m.TP * m.EWP;
-            const size_t fl = wgrad ? (size_t)m.C * m.T * EW + slab : (size_t)m.C * m.kt * m.kp * CO + slab;
-            if (fl * 4 + 64 <= lim) { *out = m; *smem = fl * 4 + 64; *co = CO; return MMX_OK; }
-        }
+    auto bytes_of = [&](int EW) {
+        const size_t slab = (size_t)m.C * m.TP * (EW + d->kp + 3);
+        return (wgrad ? (size_t)m.C * m.T * EW + slab : (size_t)m.C * m.kt * m.kp * CO + slab) * 4 + 64;
+    };
+    const int EW = fit_tile(di, round_up(d->E, 4), 4, 4, true, bytes_of);
+    if (EW) {
+        m.EW = EW; m.EWP = EW + d->kp + 3; m.netile = (d->E + EW - 1) / EW;
+        *out = m; *smem = bytes_of(EW); *co = CO;
+        return MMX_OK;
     }
     return fail(MMX_E_UNSUPPORTED, "large ConvMixerBlock path: kernel %dx%dx(%d,%d) does not fit shared memory", d->C, d->C, d->kt, d->kp);
 }

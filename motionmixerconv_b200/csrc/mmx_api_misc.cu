@@ -37,22 +37,13 @@ int plan_linear(int rows, int K, int N, bool bwd, LinearDims* out, size_t* smem,
     if (rows <= 0 || K <= 0 || N <= 0) return fail(MMX_E_INVALID, "non-positive dimension");
     const DevInfo di = dev_info();
     LinearDims d; d.rows = rows; d.K = K; d.N = N;
-    const int two_cta_budget = smem_budget(di, 2);
-    for (int pass = 0; pass < 2; ++pass) {
-        const int budget = pass == 0 ? two_cta_budget : di.max_smem;
-        for (int R = 128; R >= 8; R -= 8) {
-            d.R = R;
-            const size_t bytes = (size_t)linear_smem(d, bwd).total * 4;
-            if (bytes <= (size_t)budget) {
-                d.R = imin(R, round_up(rows, 4));
-                if (d.R == R && R >= 16) d.R = balanced_tile(rows, R, R / 2, 8, di.sms);
-                const size_t b2 = (size_t)linear_smem(d, bwd).total * 4;
-                *out = d; *smem = b2; *grid = balanced_grid((rows + d.R - 1) / d.R, di.sms * ctas_per_sm(di, b2, 8));
-                return MMX_OK;
-            }
-        }
-    }
-    return fail(MMX_E_UNSUPPORTED, "linear layer K=%d N=%d does not fit shared memory", K, N);
+    const int R = fit_tile(di, 128, 8, 8, true, [&](int r) { d.R = r; return (size_t)linear_smem(d, bwd).total * 4; });
+    if (!R) return fail(MMX_E_UNSUPPORTED, "linear layer K=%d N=%d does not fit shared memory", K, N);
+    d.R = imin(R, round_up(rows, 4));
+    if (d.R == R && R >= 16) d.R = balanced_tile(rows, R, R / 2, 8, di.sms);
+    const size_t bytes = (size_t)linear_smem(d, bwd).total * 4;
+    *out = d; *smem = bytes; *grid = tile_grid(di, rows, d.R, bytes);
+    return MMX_OK;
 }
 
 int check_head_desc(const MmxMlpHeadDesc* d) {
@@ -67,29 +58,18 @@ int plan_head(const MmxMlpHeadDesc* d, bool bwd, MlpHeadDims* out, size_t* smem,
     if (((d->To + 3) / 4) * ((d->T + 3) / 4) > kThreads) return fail(MMX_E_UNSUPPORTED, "pred_len %d too large", d->To);
     const DevInfo di = dev_info();
     MlpHeadDims h; h.B = d->B; h.T = d->T; h.To = d->To; h.H = d->H; h.D = d->D;
-    const int two_cta_budget = smem_budget(di, 2);
-    const int forced = env_int(bwd ? "MMX_HEAD_S_BWD" : "MMX_HEAD_S_FWD", 0);
-    // wide rows: one CTA per SM with a larger tile beats two CTAs with S = 2 (the forced-S sweep below ran in the full budget)
-    for (int pass = (d->H >= 64 && forced <= 0) ? 1 : 0; pass < 2; ++pass) {
-        const int budget = pass == 0 ? two_cta_budget : di.max_smem;
-        // sequences per tile: ~96 output rows per tile for narrow models; wide rows (H >= 64: K4, H = 128) amortise the fc_out weight
-        // reads over more rows -- measured at B = 4096, T = 10, To = 25, H = 128, D = 54 (us, fwd / bwd): S = 2: 122 / 400, 4: 98 / 302,
-        // 6: 120 / 285 (tools/head_sweep.py)
-        const int rows0 = d->H >= 64 ? (bwd ? 160 : 100) : 96;
-        for (int S = forced > 0 ? forced : imax(1, rows0 / imax(d->T, d->To)); S >= 1; --S) {
-            h.S = S;
-            const size_t bytes = (size_t)mlp_head_smem(h, bwd).total * 4;
-            if (bytes <= (size_t)budget) {
-                h.S = imin(S, d->B);
-                if (forced <= 0 && h.S == S && S >= 2) h.S = balanced_tile(d->B, S, (S + 1) / 2, 1, di.sms);
-                const size_t b2 = (size_t)mlp_head_smem(h, bwd).total * 4;
-                *out = h; *smem = b2; *grid = balanced_grid((d->B + h.S - 1) / h.S, di.sms * ctas_per_sm(di, b2, 8));
-                return MMX_OK;
-            }
-            if (forced > 0) break;
-        }
-    }
-    return fail(MMX_E_UNSUPPORTED, "MlpMixer head tile does not fit shared memory (H=%d D=%d To=%d)", d->H, d->D, d->To);
+    // sequences per tile: ~96 output rows per tile for narrow models.  Wide rows (H >= 64: K4, H = 128) amortise the fc_out weight
+    // reads over more rows, and one CTA per SM with a larger tile beats two CTAs with S = 2 -- measured in the one-CTA budget at
+    // B = 4096, T = 10, To = 25, H = 128, D = 54 (us, fwd / bwd): S = 2: 122 / 400, 4: 98 / 302, 6: 120 / 285
+    const int rows0 = d->H >= 64 ? (bwd ? 160 : 100) : 96;
+    const int S = fit_tile(di, imax(1, rows0 / imax(d->T, d->To)), 1, 1, d->H < 64,
+                           [&](int s) { h.S = s; return (size_t)mlp_head_smem(h, bwd).total * 4; });
+    if (!S) return fail(MMX_E_UNSUPPORTED, "MlpMixer head tile does not fit shared memory (H=%d D=%d To=%d)", d->H, d->D, d->To);
+    h.S = imin(S, d->B);
+    if (h.S == S && S >= 2) h.S = balanced_tile(d->B, S, (S + 1) / 2, 1, di.sms);
+    const size_t bytes = (size_t)mlp_head_smem(h, bwd).total * 4;
+    *out = h; *smem = bytes; *grid = tile_grid(di, d->B, h.S, bytes);
+    return MMX_OK;
 }
 
 

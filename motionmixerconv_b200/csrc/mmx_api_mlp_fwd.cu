@@ -35,12 +35,9 @@ extern "C" int mmx_mlp_block_fwd(const MmxMlpBlockDesc* d, const MmxMlpBlockPara
     a.w = to_w(w); a.x = x; a.y = y;
     if (warp_variant) {
         const int thr = nwarp * 32;
-        const int occ = env_int("MMX_MLP_FWD_OCC", 2);   // 2: the 128-register build, two CTAs per SM (measured 8 % faster than 1 x 254 registers)
-        if (occ >= 2)
-            return d->act == MMX_ACT_GELU ? launch<MlpFwdWarpBody<ACT_GELU, 10, 20>, MlpBlockFwdArgs, 2>(a, grid, thr, smem, stream)
-                                          : launch<MlpFwdWarpBody<ACT_MISH, 10, 20>, MlpBlockFwdArgs, 2>(a, grid, thr, smem, stream);
-        return d->act == MMX_ACT_GELU ? launch<MlpFwdWarpBody<ACT_GELU, 10, 20>>(a, grid, thr, smem, stream)
-                                      : launch<MlpFwdWarpBody<ACT_MISH, 10, 20>>(a, grid, thr, smem, stream);
+        // the 128-register build, two CTAs per SM (measured 8 % faster than 1 x 254 registers)
+        return d->act == MMX_ACT_GELU ? launch<MlpFwdWarpBody<ACT_GELU, 10, 20>, MlpBlockFwdArgs, 2>(a, grid, thr, smem, stream)
+                                      : launch<MlpFwdWarpBody<ACT_MISH, 10, 20>, MlpBlockFwdArgs, 2>(a, grid, thr, smem, stream);
     }
     return d->act == MMX_ACT_GELU ? dispatch_mlp_fwd<ACT_GELU>(a, grid, smem, stream) : dispatch_mlp_fwd<ACT_MISH>(a, grid, smem, stream);
 }

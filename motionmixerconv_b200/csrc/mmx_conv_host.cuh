@@ -37,28 +37,20 @@ static inline int plan_conv_half(const MmxConvHalfDesc* d, bool bwd, ConvDims* o
     m.B = d->B; m.C = d->C; m.T = d->T; m.E = d->E; m.kT = d->kt; m.kP = d->kp; m.pT = d->pad_t; m.pP = d->pad_p;
     m.rr = d->use_se ? d->se_hidden : 0; m.use_se = d->use_se; m.use_max = d->use_max_pooling; m.training = d->training;
     m.site = d->site; m.bn_mode = 0;
-    const int two_cta_budget = smem_budget(di, 2);
-    const int forced = env_int(bwd ? "MMX_CONV_S_BWD" : "MMX_CONV_S_FWD", 0);
+    const int forced = env_int(bwd ? "MMX_CONV_S_BWD" : "MMX_CONV_S_FWD", 0);   // tests: force the tile
     // about kConvTileElems activations per tile, but never fewer tiles than ~2 per SM when the batch is small
     int S0 = imax(1, kConvTileElems / (d->C * d->T * d->E));
     S0 = imax(1, imin(S0, (d->B + 2 * di.sms - 1) / (2 * di.sms)));
     if (forced > 0) S0 = forced;
-    for (int in_smem = 1; in_smem >= 0; --in_smem) {
-        m.x_in_smem = in_smem;
-        if (!bwd && !in_smem) break;
+    for (int in_smem = 1; in_smem >= (bwd ? 0 : 1); --in_smem) {
         if (bwd && in_smem && env_int("MMX_CONV_X_GLOBAL", 0)) continue;   // tests: force the streamed-input variant
-        for (int pass = 0; pass < 2; ++pass) {
-            const int budget = pass == 0 ? two_cta_budget : di.max_smem;
-            for (int S = S0; S >= 1; --S) {
-                m.S = S;
-                if ((size_t)conv_smem(m, bwd).total * 4 <= (size_t)budget) {
-                    m.S = imin(S, d->B);
-                    const size_t bytes = (size_t)conv_smem(m, bwd).total * 4;
-                    *out = m; *smem = bytes; *grid = balanced_grid((d->B + m.S - 1) / m.S, di.sms * ctas_per_sm(di, bytes, 8));
-                    return MMX_OK;
-                }
-                if (forced > 0) break;
-            }
+        m.x_in_smem = in_smem;
+        const int S = fit_tile(di, S0, forced > 0 ? forced : 1, 1, true, [&](int s) { m.S = s; return (size_t)conv_smem(m, bwd).total * 4; });
+        if (S) {
+            m.S = imin(S, d->B);
+            const size_t bytes = (size_t)conv_smem(m, bwd).total * 4;
+            *out = m; *smem = bytes; *grid = tile_grid(di, d->B, m.S, bytes);
+            return MMX_OK;
         }
     }
     return fail(MMX_E_UNSUPPORTED, "ConvMixerBlock tile does not fit shared memory (C=%d T=%d E=%d kernel %dx%d)", d->C, d->T, d->E, d->kt, d->kp);

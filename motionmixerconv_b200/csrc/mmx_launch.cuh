@@ -23,6 +23,10 @@ int* mmx_tc5_abort_ptr();
 
 namespace mmx {
 
+// The library's only environment inputs are test hooks, read through env_int; each forces a plan so that a test can check it:
+// MMX_MLP_V1 (generic MixerBlock kernels instead of the warp variant), MMX_CONV_S_FWD / MMX_CONV_S_BWD and
+// MMX_CHEAD_S_FWD / MMX_CHEAD_S_BWD (ConvMixer half / head tile), MMX_CONV_X_GLOBAL (streamed-input ConvMixer backward),
+// MMX_CHAN_STREAMED (tcgen05 channel-half plan) and MMX_IO_NO_TC5 (fp32 embedding and output head kernels under tf32).
 static inline int env_int(const char* name, int dflt) {
     const char* s = getenv(name);
     return s && *s ? atoi(s) : dflt;
@@ -126,7 +130,8 @@ static __global__ void __launch_bounds__(256, 2) mmx_kernel_occ2(const Args a) {
 
 template <class Body, class Args, int OCC = 1>
 static int launch(const Args& a, int grid, int block, size_t smem_bytes, void* stream) {
-    return launch_kernel(OCC >= 2 ? mmx_kernel_occ2<Body, Args> : mmx_kernel<Body, Args>, grid, block, smem_bytes, stream, kNoPdl, a);
+    if constexpr (OCC >= 2) return launch_kernel(mmx_kernel_occ2<Body, Args>, grid, block, smem_bytes, stream, kNoPdl, a);
+    else return launch_kernel(mmx_kernel<Body, Args>, grid, block, smem_bytes, stream, kNoPdl, a);
 }
 #endif
 
@@ -138,6 +143,17 @@ static inline int ctas_per_sm(const DevInfo& di, size_t smem, int cap) {
 }
 // dynamic shared memory per CTA that leaves room for n CTAs per SM (and 1 KB of slack)
 static inline int smem_budget(const DevInfo& di, int n) { return (di.max_smem + 1024) / n - 2048; }
+// Tile search of the fp32 planners: the largest tile S in hi, hi - step, ... >= lo whose shared memory bytes_of(S) leaves room
+// for two CTAs per SM, else the largest that fits one CTA; 0 if none fits.  two_cta_first = false: the one-CTA budget only.
+template <class F>
+static inline int fit_tile(const DevInfo& di, int hi, int lo, int step, bool two_cta_first, F bytes_of) {
+    for (int pass = two_cta_first ? 0 : 1; pass < 2; ++pass) {
+        const size_t budget = pass == 0 ? (size_t)smem_budget(di, 2) : (size_t)di.max_smem;
+        for (int S = hi; S >= lo; S -= step)
+            if ((size_t)bytes_of(S) <= budget) return S;
+    }
+    return 0;
+}
 // grid of ceil(work / per_cta) CTAs, in [1, k x SMs]
 static inline int capped_grid(const DevInfo& di, long long work, long long per_cta, int k) {
     const long long want = (work + per_cta - 1) / per_cta, cap = (long long)di.sms * k;
@@ -151,12 +167,15 @@ static inline int balanced_grid(int ntiles, int max_ctas) {
     const int waves = (ntiles + max_ctas - 1) / max_ctas;
     return (ntiles + waves - 1) / waves;
 }
+// grid for a persistent loop over n rows / sequences in tiles of S, each tile `bytes` of dynamic shared memory
+static inline int tile_grid(const DevInfo& di, int n, int S, size_t bytes) {
+    return balanced_grid((n + S - 1) / S, di.sms * ctas_per_sm(di, bytes, 8));
+}
 
 // Tile size in [lo, hi] (multiples of `step`) for a loop over n rows / sequences: CTAs are dealt round-robin to the SMs, so
 // the makespan is (tiles on the busiest SM) x (tile size) -- e.g. 4096 sequences in tiles of 9 give 456 tiles = 4 rounds of
 // 148 SMs at 9 sequences, tiles of 7 give 586 tiles = 4 rounds at 7.  Ties go to the larger tile (better weight reuse).
 static inline int balanced_tile(int n, int hi, int lo, int step, int sms) {
-    if (env_int("MMX_NO_BALANCED_TILE", 0)) return hi;
     int best = hi;
     long long best_cost = -1;
     for (int S = hi; S >= imax(lo, 1); S -= step) {

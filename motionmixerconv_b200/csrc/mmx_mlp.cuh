@@ -71,7 +71,6 @@ struct MlpDims {
     int training;
     int site_base;             // dropout site id of this block's first Dropout (block_index*4)
     int w_in_smem;             // 1: channel-MLP weights staged in shared memory, 0: read from global (needs H%4==0, ch%4==0)
-    int align_mask;            // warp-variant backward: enabled CTA re-alignment points (bit i = point i)
 };
 
 struct MlpBlockW {            // parameter (or gradient) pointers of one MixerBlock, reference layouts

@@ -34,9 +34,6 @@ static inline int plan_mlp_block(const MmxMlpBlockDesc* d, bool bwd, MlpDims* ou
     MlpDims m;
     m.B = d->B; m.T = d->T; m.H = d->H; m.tok = d->tok; m.ch = d->ch; m.rr = d->use_se ? d->se_hidden : 0;
     m.use_se = d->use_se; m.use_max = d->use_max_pooling; m.training = d->training; m.site_base = d->block_index * 4;
-    m.align_mask = 0;
-    const int forced = env_int(bwd ? "MMX_MLP_S_BWD" : "MMX_MLP_S_FWD", 0);
-    const int two_cta_budget = smem_budget(di, 2);
     const int row_target = bwd ? 96 : 128;
     // Two candidates: channel-MLP weights staged in shared memory, or read from global (L1/L2; needs H, ch % 4 == 0).  Large H:
     // the staged weights leave room for a single sequence per tile (10 rows: GEMM phases with a handful of busy threads),
@@ -45,25 +42,16 @@ static inline int plan_mlp_block(const MmxMlpBlockDesc* d, bool bwd, MlpDims* ou
     for (int in_smem = 1; in_smem >= 0; --in_smem) {
         if (!in_smem && ((d->H & 3) || (d->ch & 3))) continue;
         m.w_in_smem = in_smem;
-        for (int budget_pass = 0; budget_pass < 2 && !bestS[in_smem]; ++budget_pass) {
-            const int budget = budget_pass == 0 ? two_cta_budget : di.max_smem;
-            for (int S = imax(1, row_target / d->T); S >= 1; --S) {
-                m.S = S;
-                if ((size_t)mlp_block_smem(m, bwd).total * 4 <= (size_t)budget) { bestS[in_smem] = S; break; }
-            }
-        }
-        if (forced > 0) { m.S = forced; bestS[in_smem] = (size_t)mlp_block_smem(m, bwd).total * 4 <= (size_t)di.max_smem ? forced : 0; }
+        bestS[in_smem] = fit_tile(di, imax(1, row_target / d->T), 1, 1, true, [&](int S) { m.S = S; return (size_t)mlp_block_smem(m, bwd).total * 4; });
     }
     int pick = bestS[1] ? 1 : 0;
     if (bestS[0] >= 2 * imax(bestS[1], 1) && bestS[1] * d->T < 32) pick = 0;
-    if (env_int("MMX_MLP_W_SMEM", -1) >= 0 && bestS[env_int("MMX_MLP_W_SMEM", -1) & 1]) pick = env_int("MMX_MLP_W_SMEM", -1) & 1;
     if (bestS[pick]) {
         m.w_in_smem = pick;
         m.S = imin(bestS[pick], d->B);
-        if (forced <= 0 && m.S == bestS[pick] && m.S >= 2) m.S = balanced_tile(d->B, m.S, (m.S + 1) / 2, 1, di.sms);
+        if (m.S == bestS[pick] && m.S >= 2) m.S = balanced_tile(d->B, m.S, (m.S + 1) / 2, 1, di.sms);
         const size_t bytes = (size_t)mlp_block_smem(m, bwd).total * 4;
-        const int ntiles = (d->B + m.S - 1) / m.S;
-        *out = m; *smem = bytes; *grid = balanced_grid(ntiles, di.sms * ctas_per_sm(di, bytes, 8));
+        *out = m; *smem = bytes; *grid = tile_grid(di, d->B, m.S, bytes);
         return MMX_OK;
     }
     return fail(MMX_E_UNSUPPORTED, "MixerBlock tile does not fit shared memory (H=%d ch=%d)", d->H, d->ch);
@@ -84,8 +72,8 @@ static inline int plan_mlp_block_warp(const MmxMlpBlockDesc* d, bool bwd, MlpDim
     MlpDims m;
     m.B = d->B; m.T = d->T; m.H = d->H; m.tok = d->tok; m.ch = d->ch; m.rr = d->use_se ? d->se_hidden : 0;
     m.use_se = d->use_se; m.use_max = 0; m.training = d->training; m.site_base = d->block_index * 4;
-    m.S = kSPW; m.w_in_smem = 1; m.align_mask = env_int("MMX_MLP_ALIGN_MASK", 64) | (env_int("MMX_MLP_ALIGN_MASK_FWD", 2) << 16);   // bwd: bits 0-15, fwd: bits 16+
-    int nwarp = env_int("MMX_MLP_WARPS", kWarpVariantWarps);
+    m.S = kSPW; m.w_in_smem = 1;
+    int nwarp = kWarpVariantWarps;
     size_t bytes = 0;
     for (; nwarp >= 2; --nwarp) {      // as many warps per CTA as the shared-memory scratch allows
         bytes = (size_t)mlp_warp_smem(m, bwd, nwarp).total * 4;
@@ -101,7 +89,7 @@ static inline int plan_mlp_block_warp(const MmxMlpBlockDesc* d, bool bwd, MlpDim
     // faster with fewer co-resident warps and the makespan is waves x the per-pair latency either way
     const int slots = di.sms * per_sm;
     const int spread = imax(2, imin(nwarp, (warps_needed + slots - 1) / slots));
-    if (spread < nwarp && !env_int("MMX_MLP_NO_SPREAD", 0)) {
+    if (spread < nwarp) {
         nwarp = spread;
         bytes = (size_t)mlp_warp_smem(m, bwd, nwarp).total * 4;
     }

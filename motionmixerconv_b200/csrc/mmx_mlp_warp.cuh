@@ -358,7 +358,6 @@ MMX_D void mlp_block_fwd_warp_body(Exec& ex, const MlpBlockFwdArgs& a) {
     const bool drop = d.training && dr.thresh != 0u;
     typedef WLane<TC> ST;
     PerThread<ST> regs(ex);
-    const int amask_f = d.align_mask >> 16;     // forward: enabled CTA re-alignment points
 
     ex.phase([&](int tid) { mlp_warp_stage(tid, nthr, sm, L, d, a.w); });
 
@@ -368,15 +367,12 @@ MMX_D void mlp_block_fwd_warp_body(Exec& ex, const MlpBlockFwdArgs& a) {
         float* red = ws + L.red;
         float* tot = ws + L.tot;
         // every warp of the CTA runs the same number of iterations (a warp without a pair runs a dead one: nothing is stored
-        // or accumulated) and the CTA can re-align at the points marked wx.align(): the loop body is several times the size
-        // of the instruction caches, and warps that walk it together share each fetched line.  Which points are on is a
-        // measured choice (tools/gpu_align_sweep.sh): ONE re-alignment per iteration, placed after the lock-protected
-        // weight-gradient phases, is best (backward 316 -> 233 us at B=4096); aligning right in front of those phases
-        // makes every warp hit the locks at once and costs more than it saves
+        // or accumulated) and the CTA re-aligns once per iteration at wx.align(): the loop body is several times the size of
+        // the instruction caches, and warps that walk it together share each fetched line.  The forward time is the same for
+        // every choice of re-alignment points (profiles/r1zc_alignment_sweeps.txt); this one sits in front of the X1 phase
         const int per_iter = ex.nblk * nwarp, n_iter = (groups + per_iter - 1) / per_iter;
         for (int it = 0; it < n_iter; ++it) {
             const int grp = it * per_iter + ex.bid * nwarp + wx.warp;
-            if (amask_f >> 0 & 1) wx.align();
             // lane geometry (recomputed inside each sub-phase from `lane`)
 #define MMX_LANE_GEOM                                                                                     \
     ST& st = regs[wx.warp * 32 + lane];                                                                   \
@@ -431,7 +427,7 @@ MMX_D void mlp_block_fwd_warp_body(Exec& ex, const MlpBlockFwdArgs& a) {
             });
             if (d.use_se) wx.phase([&](int lane) { red_sum<TC>(red, tot, lane); });
             // X1 = X + gate1 * Yt ; LN2 statistics
-            if (amask_f >> 1 & 1) wx.align();
+            wx.align();
             wx.phase([&](int lane) {
                 MMX_LANE_GEOM
                 float gate[TC];
@@ -485,7 +481,6 @@ MMX_D void mlp_block_fwd_warp_body(Exec& ex, const MlpBlockFwdArgs& a) {
                 }
             });
             // G2 = drop(act(N2 V1^T + c1)) -> tile1
-            if (amask_f >> 2 & 1) wx.align();
             wx.phase([&](int lane) {
                 MMX_LANE_GEOM
                 MMX_UNROLL
@@ -506,7 +501,6 @@ MMX_D void mlp_block_fwd_warp_body(Exec& ex, const MlpBlockFwdArgs& a) {
                 }
             });
             // Y2 = drop(G2 V2^T + c2) ; SE2 squeeze
-            if (amask_f >> 3 & 1) wx.align();
             wx.phase([&](int lane) {
                 MMX_LANE_GEOM
                 MMX_UNROLL
@@ -570,7 +564,6 @@ MMX_D void mlp_block_bwd_warp_body(Exec& ex, const MlpBlockBwdArgs& a) {
     const Dropout dr = resolve_dropout(a.dr);
     const bool drop = d.training && dr.thresh != 0u;
     constexpr int NTR = 2 * TC + 1;      // per-k transpose-reduce values: dW2[:,k] (TC), dW1[k,:] (TC), db1[k]
-    const int amask = d.align_mask;      // which CTA re-alignment points are on (tuning knob, MMX_MLP_ALIGN_MASK)
     typedef WLane<TC> ST;
     PerThread<ST> regs(ex);
 
@@ -587,15 +580,14 @@ MMX_D void mlp_block_bwd_warp_body(Exec& ex, const MlpBlockBwdArgs& a) {
         float* trb = ws + L.tile[1];     // token phase: 2 transpose buffers [NTR][kTrP] (tiles 1..2 are free by then)
         unsigned int* locks = reinterpret_cast<unsigned int*>(sm + L.lock);
         // every warp of the CTA runs the same number of iterations (a warp without a pair runs a dead one: nothing is stored
-        // or accumulated) and the CTA can re-align at the points marked wx.align(): the loop body is several times the size
-        // of the instruction caches, and warps that walk it together share each fetched line.  Which points are on is a
-        // measured choice (tools/gpu_align_sweep.sh): ONE re-alignment per iteration, placed after the lock-protected
-        // weight-gradient phases, is best (backward 316 -> 233 us at B=4096); aligning right in front of those phases
-        // makes every warp hit the locks at once and costs more than it saves
+        // or accumulated) and the CTA re-aligns once per iteration at wx.align(): the loop body is several times the size of
+        // the instruction caches, and warps that walk it together share each fetched line.  Where is a measured choice
+        // (profiles/r1zc_alignment_sweeps.txt): after the lock-protected weight-gradient phases is best (backward
+        // 316 -> 233 us at B=4096); aligning right in front of those phases makes every warp hit the locks at once and costs
+        // more than it saves
         const int per_iter = ex.nblk * nwarp, n_iter = (groups + per_iter - 1) / per_iter;
         for (int it = 0; it < n_iter; ++it) {
             const int grp = it * per_iter + ex.bid * nwarp + wx.warp;
-            if (amask >> 0 & 1) wx.align();
             // ---------------- recompute: LN1, token MLP, SE1, X1, LN2, channel MLP ----------------
             wx.phase([&](int lane) {
                 MMX_LANE_GEOM
@@ -698,7 +690,6 @@ MMX_D void mlp_block_bwd_warp_body(Exec& ex, const MlpBlockBwdArgs& a) {
                     if (4 * q < P) st4(t0 + t * P, make_f4(v[0], v[1], v[2], v[3]));
                 }
             });
-            if (amask >> 1 & 1) wx.align();
             wx.phase([&](int lane) {      // U2 -> e (registers), G2 -> tile1
                 MMX_LANE_GEOM
                 MMX_UNROLL
@@ -723,7 +714,6 @@ MMX_D void mlp_block_bwd_warp_body(Exec& ex, const MlpBlockBwdArgs& a) {
                     if (4 * q < P) st4(t1 + t * P, make_f4(v[0], v[1], v[2], v[3]));
                 }
             });
-            if (amask >> 2 & 1) wx.align();
             // Y2 ; dOut ; SE2 squeeze + dgate2 partials
             wx.phase([&](int lane) {
                 MMX_LANE_GEOM
@@ -786,7 +776,6 @@ MMX_D void mlp_block_bwd_warp_body(Exec& ex, const MlpBlockBwdArgs& a) {
                         if (j < nvh) ws[L.wv + (s * 6 + 5) * 64 + 4 * q + j] += cs[j];
                 }
             });
-            if (amask >> 3 & 1) wx.align();
             // dV2[h][c] += dY2^T G2 ; dG2 = dY2 V2
             wx.phase([&](int lane) {
                 MMX_LANE_GEOM
@@ -798,7 +787,6 @@ MMX_D void mlp_block_bwd_warp_body(Exec& ex, const MlpBlockBwdArgs& a) {
                     for (int j = 0; j < 4; ++j) st.b[t][j] = 0.0f;
                 warp_gemm_nn<TC>(st.b, ws + L.tile[2] + s * TC * P, P, sm + L.v2, L.PC, H, q);
             });
-            if (amask >> 4 & 1) wx.align();
             // dU2 = dG2 * mask2 * act'(U2) -> tile1 ; dc1
             wx.phase([&](int lane) {
                 MMX_LANE_GEOM
@@ -826,7 +814,6 @@ MMX_D void mlp_block_bwd_warp_body(Exec& ex, const MlpBlockBwdArgs& a) {
                         if (j < nvc) ws[L.wv + (s * 6 + 4) * 64 + 4 * q + j] += cs[j];
                 }
             });
-            if (amask >> 5 & 1) wx.align();
             // dV1[c][h] += dU2^T N2 ; dN2 = dU2 V1 ; LN2 backward partials
             wx.phase([&](int lane) {
                 MMX_LANE_GEOM
@@ -861,7 +848,7 @@ MMX_D void mlp_block_bwd_warp_body(Exec& ex, const MlpBlockBwdArgs& a) {
                 red_write<2 * TC>(red, lane, st.rv);
             });
             wx.phase([&](int lane) { red_sum<2 * TC>(red, tot, lane); });
-            if (amask >> 6 & 1) wx.align();
+            wx.align();
             // dX1 = dOut + LN2'(dN2) -> e ; token half: reload X, LN1, token forward, dgate1 partials
             wx.phase([&](int lane) {
                 MMX_LANE_GEOM
@@ -900,7 +887,6 @@ MMX_D void mlp_block_bwd_warp_body(Exec& ex, const MlpBlockBwdArgs& a) {
                 }
             });
             if (d.use_se) wx.phase([&](int lane) { red_sum<TC>(red, tot, lane); });
-            if (amask >> 7 & 1) wx.align();
             // dYt = (dX1*gate1 + ds1/H) * mask1 -> c ; db2 partials ; dX1 stashed in tile0 ; dN1 accumulator (a) zeroed
             wx.phase([&](int lane) {
                 MMX_LANE_GEOM
@@ -941,7 +927,6 @@ MMX_D void mlp_block_bwd_warp_body(Exec& ex, const MlpBlockBwdArgs& a) {
             // hidden columns) are transposed through shared memory: lane v then owns value v of unit k-1
             MMX_NOUNROLL
             for (int k = 0; k <= TOKC; ++k) {
-                if ((k & 3) == 0 && (amask >> 12 & 1)) wx.align();
                 wx.phase([&](int lane) {
                     MMX_LANE_GEOM
                     if (k == 0 && q == 0 && live) {      // db2[t] (token fc2 bias): totals of the dYt row sums
@@ -1001,7 +986,6 @@ MMX_D void mlp_block_bwd_warp_body(Exec& ex, const MlpBlockBwdArgs& a) {
                     }
                 });
             }
-            if (amask >> 8 & 1) wx.align();
             // LN1 backward: dX = dX1 + LN1'(dN1)
             wx.phase([&](int lane) {
                 MMX_LANE_GEOM
