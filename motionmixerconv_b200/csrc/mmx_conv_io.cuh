@@ -269,7 +269,8 @@ struct EncDims {
     int B, T, D, E, C, Hn;
     int K;        // embedding width: Hn > 0 ? 2*Hn*D : D
     int KC;       // embedding columns per chunk (multiple of 4)
-    int DC;       // harmonic embedding: input dimensions per chunk (a chunk = their sin AND cos columns, KC >= 2*DC*Hn)
+    int DC;       // harmonic embedding: input dimensions per chunk (a chunk = their sin AND cos columns, KC >= 2*DC*HC)
+    int HC;       // harmonic embedding: harmonics per chunk; HC < Hn (then DC = 1) splits one input dimension over several chunks
     int R;        // frames (rows of x) per CTA tile
 };
 struct EncW { float *freq, *w, *b, *wc, *bc; };   // frequencies[Hn], embed_mlp.{weight[E,K],bias[E]}, channelUpscaling.{weight[C,1],bias[C]}
@@ -305,8 +306,9 @@ MMX_D void enc_fwd_body(Exec& ex, const EncFwdArgs& a) {
     float* sm = ex.smem;
     const int nthr = ex.nthr, D = d.D, E = d.E, C = d.C, T = d.T, K = d.K, KC = d.KC, R = d.R, PKC = L.PKC, PE = L.PE;
     const int rows = d.B * T;
-    const int Hn = d.Hn, DC = d.DC;
-    const int nchunks = Hn > 0 ? (D + DC - 1) / DC : (K + KC - 1) / KC;
+    const int Hn = d.Hn, DC = d.DC, HC = d.HC;
+    const int nseg = Hn > 0 ? (Hn + HC - 1) / HC : 1;     // harmonic segments per group of DC input dimensions
+    const int nchunks = Hn > 0 ? ((D + DC - 1) / DC) * nseg : (K + KC - 1) / KC;
     PerThread<EncFwdRegs> regs(ex);
     ex.phase([&](int tid) {
         copy_vec(tid, nthr, sm + L.b, a.w.b, E);
@@ -333,20 +335,21 @@ MMX_D void enc_fwd_body(Exec& ex, const EncFwdArgs& a) {
                 for (int j = 0; j < 4; ++j) rg.acc[i][j] = 0.0f;
         });
         for (int ch = 0; ch < nchunks; ++ch) {
-            // chunk geometry.  Plain input: columns [k0, k0+kc) of x.  Harmonic: dims [d0, d0+dcv): their dcv*Hn sin columns
-            // (global column dd*Hn+h) followed by their dcv*Hn cos columns (global column Hn*D + dd*Hn+h)
-            const int d0 = ch * DC, dcv = Hn > 0 ? imin(DC, D - d0) : 0, half = dcv * Hn;
+            // chunk geometry.  Plain input: columns [k0, k0+kc) of x.  Harmonic: dims [d0, d0+dcv) and harmonics [hs0, hs0+hc):
+            // their dcv*hc sin columns (global column dd*Hn+h) followed by their dcv*hc cos columns (global column Hn*D + dd*Hn+h)
+            const int dg = ch / nseg, hs0 = (ch - dg * nseg) * HC, hc = Hn > 0 ? imin(HC, Hn - hs0) : 0;
+            const int d0 = dg * DC, dcv = Hn > 0 ? imin(DC, D - d0) : 0, half = dcv * hc;
             const int k0 = ch * KC, kc = Hn > 0 ? 2 * half : imin(KC, K - k0), kc4 = (kc + 3) >> 2;
             ex.phase([&](int tid) {
                 if (Hn > 0) {
                     const bool pow2 = sm[L.flag] != 0.0f;
-                    const int nseg = (Hn + 7) >> 3;
-                    for (int i = tid; i < nr * dcv * nseg; i += nthr) {
-                        const int hs = i % nseg, rd = i / nseg, dd = rd % dcv, r = rd / dcv;
-                        const int h0 = 8 * hs, n = imin(8, Hn - h0);
+                    const int n8 = (hc + 7) >> 3;
+                    for (int i = tid; i < nr * dcv * n8; i += nthr) {
+                        const int hs = i % n8, rd = i / n8, dd = rd % dcv, r = rd / dcv;
+                        const int h0 = 8 * hs, n = imin(8, hc - h0);
                         float sv[8], cv[8];
-                        harmonics(sm[L.x + r * L.PD + d0 + dd], sm + L.freq, pow2, h0, n, sv, cv);
-                        float* es = sm + L.emb + r * PKC + dd * Hn + h0;
+                        harmonics(sm[L.x + r * L.PD + d0 + dd], sm + L.freq, pow2, hs0 + h0, n, sv, cv);
+                        float* es = sm + L.emb + r * PKC + dd * hc + h0;
                         for (int j = 0; j < n; ++j) { es[j] = sv[j]; es[half + j] = cv[j]; }
                     }
                     for (int i = tid; i < nr * (4 * kc4 - kc); i += nthr) {
@@ -355,7 +358,8 @@ MMX_D void enc_fwd_body(Exec& ex, const EncFwdArgs& a) {
                     }
                     for (int i = tid; i < E * 4 * kc4; i += nthr) {
                         const int e = i / (4 * kc4), c = i - e * 4 * kc4;
-                        const int col = c < half ? d0 * Hn + c : Hn * D + d0 * Hn + (c - half);
+                        const int cs = c < half ? c : c - half;
+                        const int col = (c < half ? 0 : Hn * D) + d0 * Hn + (hc == Hn ? cs : (cs / hc) * Hn + hs0 + cs % hc);
                         sm[L.w + e * PKC + c] = c < kc ? a.w.w[(size_t)e * K + col] : 0.0f;
                     }
                 } else {
@@ -615,7 +619,10 @@ MMX_D void enc_bwd2_body(Exec& ex, const EncBwd2Args& a) {
 // (project_channels and conv_out are both linear, so the channel mix is applied first: one time-mix
 //  instead of C.)
 // ==========================================================================================
-struct ConvHeadDims { int B, C, T, To, E, D, S; };
+struct ConvHeadDims {
+    int B, C, T, To, E, D, S;
+    int EC;       // chunked plan (conv_head_*_chunked_body): embedding columns per chunk, a multiple of 4; 0 for the resident plan
+};
 struct ConvHeadW { float *ln_g, *ln_b, *wt, *bt, *wp, *bp, *wf, *bf; };
 struct ConvHeadSmem {
     int PE, PD, R, ln_g, ln_b, wt, bt, wp, wf, bf, part, part2, mean, rstd, bY, bQ, bR, bG, bO;
@@ -642,7 +649,9 @@ MMX_HD ConvHeadSmem conv_head_smem(const ConvHeadDims& d, bool bwd) {
     return L;
 }
 
-MMX_D void conv_head_stage(int tid, int nthr, float* sm, const ConvHeadSmem& L, const ConvHeadDims& d, const ConvHeadW& w) {
+// small parameters of the head, and (resident plan) all of Wf; the chunked plan stages Wf one chunk at a time
+template <class Layout>
+MMX_D void conv_head_stage(int tid, int nthr, float* sm, const Layout& L, const ConvHeadDims& d, const ConvHeadW& w) {
     copy_vec(tid, nthr, sm + L.ln_g, w.ln_g, d.E); copy_vec(tid, nthr, sm + L.ln_b, w.ln_b, d.E);
     copy_vec(tid, nthr, sm + L.wt, w.wt, d.To * d.T); copy_vec(tid, nthr, sm + L.bt, w.bt, d.To);
     for (int i = tid; i < 8; i += nthr) sm[L.wp + i] = i < d.C ? w.wp[i] : 0.0f;
@@ -652,7 +661,7 @@ MMX_D void conv_head_stage(int tid, int nthr, float* sm, const ConvHeadSmem& L, 
         sm[L.wp + 8] = sw;          // sum_c wp[c]
         sm[L.wp + 9] = w.bp[0];
     }
-    stage_matrix(tid, nthr, sm + L.wf, w.wf, d.D, d.E, L.PE);
+    if (d.EC == 0) stage_matrix(tid, nthr, sm + L.wf, w.wf, d.D, d.E, L.PE);
     copy_vec(tid, nthr, sm + L.bf, w.bf, d.D);
 }
 
@@ -891,6 +900,279 @@ MMX_D void conv_head_bwd_body(Exec& ex, const ConvHeadBwdArgs& a) {
         }
         const int slice = tid / t_tiles, otile = tid - slice * t_tiles;
         if (slice < n_slices) smem_add_acc4x4(rg.dWt, otile, t_nt, sm + L.a_wt, T, To, T);    // combine the CTA's K-split slices
+        for (int e = tid; e < E; e += nthr) { red_add(a.g.ln_g + e, sm[L.a_lng + e]); red_add(a.g.ln_b + e, sm[L.a_lnb + e]); }
+        for (int n = tid; n < D; n += nthr) red_add(a.g.bf + n, sm[L.a_bf + n]);
+        for (int o = tid; o < To; o += nthr) red_add(a.g.bt + o, sm[L.a_bt + o]);
+        for (int c = tid; c < C; c += nthr) red_add(a.g.wp + c, sm[L.a_wp + c] + sm[L.a_bp + 1]);
+        if (tid == 0) red_add(a.g.bp, sm[L.a_bp]);
+    });
+    ex.phase([&](int tid) {
+        for (int i = tid; i < To * T; i += nthr) red_add(a.g.wt + i, sm[L.a_wt + i]);
+    });
+}
+
+// ------------------------------------------------------------------------------------------
+// Chunked head plan, for the shapes whose resident tile (all of Wf [D][E] plus the tile's Y, q, r, g rows) does not fit
+// shared memory.  Only the LayerNorm statistics and the fc_out contraction span E; everything else is elementwise in e.
+// A tile takes its row statistics from Y in global memory, then walks the embedding in chunks of EC columns: it stages
+// Wf[:, chunk], forms q, r and g of the chunk (reading Y from global memory) and accumulates out over the chunks.
+// The backward makes the same sweep and accumulates every parameter gradient and the two per-row LayerNorm sums m1, m2
+// that dy needs; it keeps the tile's dq [S*T][E] so that dy is one elementwise pass after the sweep.  The CTA's partial
+// dWf [D][E] stays in shared memory for the whole persistent loop and is flushed once, as the resident plan does with
+// registers.
+// ------------------------------------------------------------------------------------------
+struct ConvHeadChunkSmem {
+    int PC, PE, PD, R, ln_g, ln_b, wt, bt, wp, bf, wf, part, part2, mean, rstd, bQ, bG, bO;
+    int bR, dq, pm1, pm2, a_wf, a_lng, a_lnb, a_bf, a_bt, a_wp, a_bp, a_wt, total;
+};
+MMX_HD ConvHeadChunkSmem conv_head_chunk_smem(const ConvHeadDims& d, bool bwd) {
+    ConvHeadChunkSmem L; L.PC = pitch_of(d.EC); L.PE = pitch_of(d.E); L.PD = pitch_of(d.D); L.R = d.S * d.C * d.T;
+    const int no = d.S * d.To;
+    int o = 0;
+    auto take = [&](int n) { int r = o; o += round_up(n, 4); return r; };
+    L.ln_g = take(d.E); L.ln_b = take(d.E); L.wt = take(d.To * d.T); L.bt = take(d.To); L.wp = take(8 + 4); L.bf = take(d.D);
+    L.wf = take(d.D * L.PC);
+    const int nred = imax(L.R, no) * kParts;
+    L.part = take(nred); L.part2 = take(nred); L.mean = take(L.R); L.rstd = take(L.R);
+    L.bQ = take(d.S * d.T * L.PC); L.bG = take(no * L.PC); L.bO = take(no * L.PD);   // bO: out accumulator (fwd), dout (bwd)
+    if (bwd) {
+        L.bR = take(no * L.PC); L.dq = take(d.S * d.T * L.PE); L.pm1 = take(L.R * kParts); L.pm2 = take(L.R * kParts);
+        L.a_wf = take(d.D * d.E); L.a_lng = take(d.E); L.a_lnb = take(d.E); L.a_bf = take(d.D); L.a_bt = take(d.To);
+        L.a_wp = take(8); L.a_bp = take(4); L.a_wt = take(d.To * d.T);
+    } else { L.bR = L.dq = L.pm1 = L.pm2 = L.a_wf = L.a_lng = L.a_lnb = L.a_bf = L.a_bt = L.a_wp = L.a_bp = L.a_wt = -1; }
+    L.total = o;
+    return L;
+}
+
+// Wf[:, e0:e0+ec) -> wf [D][PC] and q of the chunk -> bQ [ns*T][PC] (Y from global); pad columns zeroed
+MMX_D void conv_head_chunk_stage_q(int tid, int nthr, float* sm, const ConvHeadChunkSmem& L, const ConvHeadDims& d,
+                                   const ConvHeadW& w, const float* yg, int ns, int e0, int ec) {
+    const int C = d.C, T = d.T, E = d.E, PC = L.PC;
+    for (int i = tid; i < d.D * PC; i += nthr) {
+        const int n = i / PC, j = i - n * PC;
+        sm[L.wf + i] = j < ec ? w.wf[(size_t)n * E + e0 + j] : 0.0f;
+    }
+    for (int i = tid; i < ns * T * PC; i += nthr) {
+        const int st = i / PC, j = i - st * PC, s = st / T, t = st - s * T, e = e0 + j;
+        float acc = 0.0f;
+        if (j < ec)
+            for (int c = 0; c < C; ++c) {
+                const int r = (s * C + c) * T + t;
+                const float qv = (yg[(size_t)r * E + e] - sm[L.mean + r]) * sm[L.rstd + r] * sm[L.ln_g + e] + sm[L.ln_b + e];
+                acc = fmaf(sm[L.wp + c], qv, acc);
+            }
+        sm[L.bQ + i] = acc;
+    }
+}
+
+// r (pre-GELU, bwd only -> bR) and g = GELU(r) -> bG of the chunk; pad columns zeroed
+MMX_D void conv_head_chunk_rg(int tid, int nthr, float* sm, const ConvHeadChunkSmem& L, const ConvHeadDims& d, int ns, int ec, bool keep_r) {
+    const int T = d.T, To = d.To, PC = L.PC;
+    for (int i = tid; i < ns * To * PC; i += nthr) {
+        const int so = i / PC, j = i - so * PC, s = so / To, o = so - s * To;
+        float acc = 0.0f, g = 0.0f;
+        if (j < ec) {
+            acc = fmaf(sm[L.bt + o], sm[L.wp + 8], sm[L.wp + 9]);
+            for (int t = 0; t < T; ++t) acc = fmaf(sm[L.wt + o * T + t], sm[L.bQ + (s * T + t) * PC + j], acc);
+            g = act_fwd<ACT_GELU>(acc);
+        }
+        if (keep_r) sm[L.bR + i] = acc;
+        sm[L.bG + i] = g;
+    }
+}
+
+MMX_D void conv_head_fwd_chunked_body(Exec& ex, const ConvHeadFwdArgs& a) {
+    const ConvHeadDims& d = a.d;
+    const ConvHeadChunkSmem L = conv_head_chunk_smem(d, false);
+    float* sm = ex.smem;
+    const int nthr = ex.nthr, C = d.C, T = d.T, To = d.To, E = d.E, D = d.D, S = d.S, PC = L.PC, PD = L.PD;
+    ex.phase([&](int tid) { conv_head_stage(tid, nthr, sm, L, d, a.w); });
+    const int ntiles = (d.B + S - 1) / S;
+    for (int tile = ex.bid; tile < ntiles; tile += ex.nblk) {
+        const long long seq0 = (long long)tile * S;
+        const int ns = imin(S, d.B - (int)seq0), nr = ns * C * T, no = ns * To;
+        const float* yg = a.y + (size_t)seq0 * C * T * E;
+        ln_stats_phases(ex, sm, L.part, L.part2, L.mean, L.rstd, yg, E, nr, E);
+        for (int e0 = 0; e0 < E; e0 += d.EC) {
+            const int ec = imin(d.EC, E - e0);
+            ex.phase([&](int tid) {
+                if (e0 == 0) zero_vec(tid, nthr, sm + L.bO, no * PD);
+                conv_head_chunk_stage_q(tid, nthr, sm, L, d, a.w, yg, ns, e0, ec);
+            });
+            ex.phase([&](int tid) { conv_head_chunk_rg(tid, nthr, sm, L, d, ns, ec, false); });
+            ex.phase([&](int tid) {
+                gemm_nt<4, 4>(tid, nthr, sm + L.bG, PC, sm + L.wf, PC, no, D, ec, [&](int m, int n, float v) { sm[L.bO + m * PD + n] += v; });
+            });
+        }
+        ex.phase([&](int tid) {
+            float* og = a.out + (size_t)seq0 * To * D;
+            for (int i = tid; i < no * D; i += nthr) {
+                const int m = i / D, n = i - m * D;
+                og[i] = sm[L.bO + m * PD + n] + sm[L.bf + n];
+            }
+        });
+    }
+}
+
+struct ConvHeadChunkBwdRegs { float dWt[4][4]; };
+
+MMX_D void conv_head_bwd_chunked_body(Exec& ex, const ConvHeadBwdArgs& a) {
+    const ConvHeadDims& d = a.d;
+    const ConvHeadChunkSmem L = conv_head_chunk_smem(d, true);
+    float* sm = ex.smem;
+    const int nthr = ex.nthr, C = d.C, T = d.T, To = d.To, E = d.E, D = d.D, S = d.S, PC = L.PC, PE = L.PE, PD = L.PD;
+    const float invE = 1.0f / (float)E;
+    const int t_nt = (T + 3) >> 2, t_tiles = ((To + 3) >> 2) * t_nt;      // dWt [To][T]
+    const int n_slices = imax(1, nthr / t_tiles);
+    PerThread<ConvHeadChunkBwdRegs> regs(ex);
+    ex.phase([&](int tid) {
+        conv_head_stage(tid, nthr, sm, L, d, a.w);
+        zero_vec(tid, nthr, sm + L.a_wf, D * E);
+        zero_vec(tid, nthr, sm + L.a_lng, E); zero_vec(tid, nthr, sm + L.a_lnb, E);
+        zero_vec(tid, nthr, sm + L.a_bf, D); zero_vec(tid, nthr, sm + L.a_bt, To);
+        zero_vec(tid, nthr, sm + L.a_wp, 8); zero_vec(tid, nthr, sm + L.a_bp, 4); zero_vec(tid, nthr, sm + L.a_wt, To * T);
+        ConvHeadChunkBwdRegs& rg = regs[tid];
+        MMX_UNROLL
+        for (int i = 0; i < 4; ++i)
+            MMX_UNROLL
+            for (int j = 0; j < 4; ++j) rg.dWt[i][j] = 0.0f;
+    });
+    const int ntiles = (d.B + S - 1) / S;
+    for (int tile = ex.bid; tile < ntiles; tile += ex.nblk) {
+        const long long seq0 = (long long)tile * S;
+        const int ns = imin(S, d.B - (int)seq0), nr = ns * C * T, no = ns * To;
+        const float* yg = a.y + (size_t)seq0 * C * T * E;
+        ex.phase([&](int tid) {
+            load_tile(tid, nthr, sm + L.bO, a.dout + (size_t)seq0 * To * D, no, D, PD);
+            zero_vec(tid, nthr, sm + L.pm1, nr * kParts); zero_vec(tid, nthr, sm + L.pm2, nr * kParts);
+        });
+        ln_stats_phases(ex, sm, L.part, L.part2, L.mean, L.rstd, yg, E, nr, E);
+        for (int e0 = 0; e0 < E; e0 += d.EC) {
+            const int ec = imin(d.EC, E - e0);
+            ex.phase([&](int tid) {
+                if (e0 == 0)
+                    for (int n = tid; n < D; n += nthr) {
+                        float s = 0.0f;
+                        for (int r = 0; r < no; ++r) s += sm[L.bO + r * PD + n];
+                        sm[L.a_bf + n] += s;
+                    }
+                conv_head_chunk_stage_q(tid, nthr, sm, L, d, a.w, yg, ns, e0, ec);
+            });
+            ex.phase([&](int tid) { conv_head_chunk_rg(tid, nthr, sm, L, d, ns, ec, true); });
+            // dWf[n][e0+j] += sum_rows dout[row][n] g[row][j];  dr = (dout Wf) * gelu'(r) -> bR in place
+            ex.phase([&](int tid) {
+                const int f_nt = (ec + 3) >> 2, f_tiles = ((D + 3) >> 2) * f_nt;
+                for (int t = tid; t < f_tiles; t += nthr) {
+                    float acc[4][4] = {};
+                    gemm_tn_acc4x4(acc, t, f_nt, sm + L.bO, PD, sm + L.bG, PC, no);
+                    const int mt = t / f_nt, nt = t - mt * f_nt;
+                    MMX_UNROLL
+                    for (int i = 0; i < 4; ++i)
+                        MMX_UNROLL
+                        for (int j = 0; j < 4; ++j)
+                            if (4 * mt + i < D && 4 * nt + j < ec) sm[L.a_wf + (4 * mt + i) * E + e0 + 4 * nt + j] += acc[i][j];
+                }
+                gemm_nn<4>(tid, nthr, sm + L.bO, PD, sm + L.wf, PC, no, ec, D, [&](int m, int n, float v) {
+                    float ga;
+                    sm[L.bR + m * PC + n] = v * act_fwd_grad<ACT_GELU>(sm[L.bR + m * PC + n], &ga);
+                });
+            });
+            // row sums of dr (-> dbp, dbt, the bias part of dwp);  dWt[o][t] += sum_{s,e} dr[s,o,e] q[s,t,e]
+            ex.phase([&](int tid) {
+                for (int i = tid; i < no * kParts; i += nthr) sm[L.part + i] = row_part_sum(sm + L.bR + (i / kParts) * PC, ec, i % kParts);
+                ConvHeadChunkBwdRegs& rg = regs[tid];
+                const int slice = tid / t_tiles, otile = tid - slice * t_tiles;
+                if (slice < n_slices) {
+                    const int E4 = (ec + 3) >> 2;
+                    const int mt = otile / t_nt, nt = otile - mt * t_nt;
+                    for (int s = slice; s < ns; s += n_slices) {
+                        const float* A = sm + L.bR + (s * To) * PC;
+                        const float* Bm = sm + L.bQ + (s * T) * PC;
+                        for (int q = 0; q < E4; ++q) {
+                            f4 av[4], bv[4];
+                            MMX_UNROLL
+                            for (int i = 0; i < 4; ++i) av[i] = ld4(A + imin(4 * mt + i, To - 1) * PC + 4 * q);
+                            MMX_UNROLL
+                            for (int j = 0; j < 4; ++j) bv[j] = ld4(Bm + imin(4 * nt + j, T - 1) * PC + 4 * q);
+                            MMX_UNROLL
+                            for (int i = 0; i < 4; ++i)
+                                MMX_UNROLL
+                                for (int j = 0; j < 4; ++j)
+                                    rg.dWt[i][j] += (av[i].x * bv[j].x + av[i].y * bv[j].y) + (av[i].z * bv[j].z + av[i].w * bv[j].w);
+                        }
+                    }
+                }
+            });
+            // drsum[o] over the tile's sequences -> dbt, dbp, bias part of dwp;  dq[s][t][e0+j] = sum_o Wt[o][t] dr[s][o][j]
+            ex.phase([&](int tid) {
+                for (int o = tid; o < To; o += nthr) {
+                    float s_ = 0.0f;
+                    for (int s = 0; s < ns; ++s) s_ += sum_parts(sm + L.part + (s * To + o) * kParts);
+                    sm[L.a_bt + o] += s_ * sm[L.wp + 8];
+                    smem_add(sm + L.a_bp, s_);
+                    smem_add(sm + L.a_bp + 1, s_ * sm[L.bt + o]);
+                }
+                for (int i = tid; i < ns * T * ec; i += nthr) {
+                    const int st = i / ec, j = i - st * ec, s = st / T, t = st - s * T;
+                    float acc = 0.0f;
+                    for (int o = 0; o < To; ++o) acc = fmaf(sm[L.wt + o * T + t], sm[L.bR + (s * To + o) * PC + j], acc);
+                    sm[L.dq + st * PE + e0 + j] = acc;
+                }
+            });
+            // dgamma, dbeta of the chunk's columns; dwp[c] += sum Q dq; the chunk's share of the LN sums m1, m2 of every row
+            ex.phase([&](int tid) {
+                const int nsl = imax(1, nthr / ec);
+                for (int it = tid; it < ec * nsl; it += nthr) {
+                    const int sl = it / ec, e = e0 + (it - sl * ec);
+                    float sg = 0.0f, sb = 0.0f;
+                    for (int r = sl; r < nr; r += nsl) {
+                        const int sc = r / T, t = r - sc * T, s = sc / C, c = sc - s * C;
+                        const float dn = sm[L.wp + c] * sm[L.dq + (s * T + t) * PE + e];
+                        const float xh = (yg[(size_t)r * E + e] - sm[L.mean + r]) * sm[L.rstd + r];
+                        sg = fmaf(dn, xh, sg); sb += dn;
+                    }
+                    smem_add(sm + L.a_lng + e, sg); smem_add(sm + L.a_lnb + e, sb);
+                }
+                for (int i = tid; i < nr * kParts; i += nthr) {
+                    const int r = i / kParts, p = i - r * kParts;
+                    const int sc = r / T, t = r - sc * T, s = sc / C, c = sc - s * C;
+                    const float mu = sm[L.mean + r], rs = sm[L.rstd + r], wpc = sm[L.wp + c];
+                    const float* dq = sm + L.dq + (s * T + t) * PE + e0;
+                    const float* yr = yg + (size_t)r * E + e0;
+                    const float* lg = sm + L.ln_g + e0;
+                    const float* lb = sm + L.ln_b + e0;
+                    float m1 = 0.0f, m2 = 0.0f, qd = 0.0f;
+                    for (int h = 4 * p; h < ec; h += 4 * kParts) {
+                        const int n = imin(4, ec - h);
+                        for (int k = 0; k < n; ++k) {
+                            const float xh = (yr[h + k] - mu) * rs;
+                            const float dxh = wpc * dq[h + k] * lg[h + k];
+                            m1 += dxh; m2 = fmaf(dxh, xh, m2);
+                            qd = fmaf(fmaf(xh, lg[h + k], lb[h + k]), dq[h + k], qd);
+                        }
+                    }
+                    sm[L.pm1 + i] += m1; sm[L.pm2 + i] += m2;
+                    smem_add(sm + L.a_wp + c, qd);
+                }
+            });
+        }
+        ex.phase([&](int tid) {
+            float* dyg = a.dy + (size_t)seq0 * C * T * E;
+            for (int i = tid; i < nr * E; i += nthr) {
+                const int r = i / E, e = i - r * E;
+                const int sc = r / T, t = r - sc * T, s = sc / C, c = sc - s * C;
+                const float mu = sm[L.mean + r], rs = sm[L.rstd + r];
+                const float m1 = sum_parts(sm + L.pm1 + r * kParts) * invE, m2 = sum_parts(sm + L.pm2 + r * kParts) * invE;
+                const float dxh = sm[L.wp + c] * sm[L.dq + (s * T + t) * PE + e] * sm[L.ln_g + e];
+                const float xh = (yg[i] - mu) * rs;
+                dyg[i] = rs * (dxh - m1 - xh * m2);
+            }
+        });
+    }
+    ex.phase([&](int tid) {
+        for (int i = tid; i < D * E; i += nthr) red_add(a.g.wf + i, sm[L.a_wf + i]);
+        const int slice = tid / t_tiles, otile = tid - slice * t_tiles;
+        if (slice < n_slices) smem_add_acc4x4(regs[tid].dWt, otile, t_nt, sm + L.a_wt, T, To, T);    // combine the CTA's K-split slices
         for (int e = tid; e < E; e += nthr) { red_add(a.g.ln_g + e, sm[L.a_lng + e]); red_add(a.g.ln_b + e, sm[L.a_lnb + e]); }
         for (int n = tid; n < D; n += nthr) red_add(a.g.bf + n, sm[L.a_bf + n]);
         for (int o = tid; o < To; o += nthr) red_add(a.g.bt + o, sm[L.a_bt + o]);

@@ -26,7 +26,9 @@ namespace mmx {
 // The library's only environment inputs are test hooks, read through env_int; each forces a plan so that a test can check it:
 // MMX_MLP_V1 (generic MixerBlock kernels instead of the warp variant), MMX_CONV_S_FWD / MMX_CONV_S_BWD and
 // MMX_CHEAD_S_FWD / MMX_CHEAD_S_BWD (ConvMixer half / head tile), MMX_CONV_X_GLOBAL (streamed-input ConvMixer backward),
-// MMX_CHAN_STREAMED (tcgen05 channel-half plan) and MMX_IO_NO_TC5 (fp32 embedding and output head kernels under tf32).
+// MMX_CHAN_STREAMED (tcgen05 channel-half plan), MMX_IO_NO_TC5 (fp32 embedding and output head kernels under tf32),
+// MMX_CHEAD_EC (chunked ConvMixer head and its chunk width), MMX_ENC_HC (harmonic PoseEncoder forward: harmonics per chunk)
+// and MMX_ENC_BWD_ROWS (harmonic PoseEncoder backward: staged frames).
 static inline int env_int(const char* name, int dflt) {
     const char* s = getenv(name);
     return s && *s ? atoi(s) : dflt;
