@@ -191,9 +191,10 @@ def _replicate(a, B):
 
 def _check_replicated(model, oracles, xb, gtb, B, tol, floor_k, dx_atol_k=0.0, grad_atol=None):
     """Full batch x[i] = xb[i % P] through autograd + mean MPJPE against the replicated-batch oracle.  ``oracles``: fresh
-    oracles, the first is compared with (the second, if any, is the fp64 truth of the noise clause)."""
+    oracles, or their replicated_oracle results (Rep) at this B; the first is compared with (the second, if any, is the fp64
+    truth of the noise clause)."""
     from motionmixerconv_b200.functional import mpjpe_error
-    reps = [replicated_oracle(o, xb, gtb, B) for o in oracles]
+    reps = [o if isinstance(o, Rep) else replicated_oracle(o, xb, gtb, B) for o in oracles]
     want, truth = reps[0], (reps[1] if len(reps) > 1 else None)
     model.zero_grad()
     x = _replicate(xb, B).requires_grad_(True)
